@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- throughput of the .lfm compress + decompress hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3s|c4s|c5s]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3s|c4s|c5s] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): synthetic 2048x2048 uint16 light-field frames, Nnum=15, predictor way "space", fixed
 predictor 4 + bzip2, 96x96x1 KLB blocks (484 per frame).  One STEP = ONE stack of N frames (N = number of GPUs; at N = 1 this is
@@ -28,6 +28,18 @@ sharded file is compared (md5) with the file ONE GPU writes for the same stack b
   cpu_baseline / --impl reference: the UNMODIFIED reference (oracle/_ref, its CUDA predictor + threaded CPU bzip2, all host
             cores) on the same N-frame stack, file on /dev/shm; falls back to the oracle port if oracle/_ref is absent.
 Inputs rotate through a pool larger than L2 (24 frame sets = 201 MB per GPU > 126 MB), so no step finds its input in L2.
+
+--steps K sets the number of timed steps of every leg: value, e2e, e2e_memory and auto_select, the round trips of cpu_baseline
+(the oracle port, when it stands in, times one quarter frame) and the launches predictor_roofline averages per kernel.
+--dump-outputs DIR writes what the last timed step of `value` handed its caller (rank 0's shard on several GPUs) to DIR as .npy:
+  decoded.npy                lfmDecompressDevice's output, float32 of the uint16 pixels
+  payload.npy                lfmCompressDevice's block streams, float32 of the bytes
+  block_offset.npy           its blockOffset[], float64
+  stored_header_version.npy  its stored headerVersion, float64
+decoded.npy and payload.npy longer than their caps (4M / 8M elements) keep, of their flattened form, the elements at the sorted
+indices np.random.default_rng(0).integers(0, n, cap); blockOffset[] (at most 3698 blocks per workload) is kept whole: at most
+48 MiB and 30 kB in all.  The inputs are seeded, so two builds run with the same
+arguments can be compared file for file.
 """
 import argparse
 import ctypes as C
@@ -113,6 +125,34 @@ class ClockSampler:
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": reasons}
 
 
+class DeviceBytes:
+    """a device buffer the engine owns, seen by torch through the CUDA array interface (no copy)"""
+
+    def __init__(self, ptr, nbytes):
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 2}
+
+
+def dump_outputs(dirname, decoded, d_payload, payload_bytes, block_offset, stored_hv):
+    """--dump-outputs (module docstring): the caller-visible results of one device round trip as float .npy files"""
+    import torch
+
+    def sample(t, cap):
+        """t (device tensor) flattened, or the elements at `cap` seeded sorted indices of it, as a host array"""
+        t = t.reshape(-1)
+        if t.numel() > cap:
+            t = t[torch.from_numpy(np.sort(np.random.default_rng(0).integers(0, t.numel(), cap))).to(t.device)]
+        return t.cpu().numpy()
+
+    payload = torch.as_tensor(DeviceBytes(d_payload, payload_bytes), device="cuda")
+    out = {"decoded": sample(decoded, 1 << 22).view(np.uint16).astype(np.float32),
+           "payload": sample(payload, 1 << 23).astype(np.float32),
+           "block_offset": block_offset.astype(np.float64),
+           "stored_header_version": np.array([stored_hv], np.float64)}
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ reference arm
 def load_reference(way):
     """the real reference (GPU build: its CUDA predictor + threaded CPU bzip2); else its CPU-shim build; else None"""
@@ -188,7 +228,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     nfr, H, W, nnum, way, hv, bdepth, desc = WORKLOADS[args.workload]
@@ -309,6 +352,8 @@ def main():
         step_device(args.warmup + i, True)
     barrier(); t_all = time.perf_counter() - t_start
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:                   # before the next engine call releases the payload
+        dump_outputs(args.dump_outputs, dout, dp.value, pb.value, off, shv.value)
 
     # ---- e2e: the reference-facing API, PAGEABLE host buffers, ONE file on /dev/shm (what the reference arm does)
     fname = shm_path("lfm_bench_%s_%d.lfm" % (os.environ.get("MASTER_PORT", "single"), os.getppid() if world > 1 else os.getpid()))
@@ -415,7 +460,7 @@ def main():
     auto_leg = None
     if world == 1 and not auto:
         ta = dict(tc=0.0, td=0.0, sel=0.0, k=-1)
-        nst = max(3, min(args.steps, 10))
+        nst = args.steps
         for i in range(2 + nst):
             d = dpool[i % POOL]
             torch.cuda.synchronize(); t0 = time.perf_counter()
@@ -451,7 +496,7 @@ def main():
                 L.set_way(wy)
                 for inv, src, dst in ((0, big, symb), (1, symb, back)):
                     assert L.lib.lfmDebugPredictDevice(src.data_ptr(), dst.data_ptr(), xyz_b, nnum, kk, 0, inv, 2, C.byref(ms)) == 0
-                    assert L.lib.lfmDebugPredictDevice(src.data_ptr(), dst.data_ptr(), xyz_b, nnum, kk, 0, inv, 5, C.byref(ms)) == 0
+                    assert L.lib.lfmDebugPredictDevice(src.data_ptr(), dst.data_ptr(), xyz_b, nnum, kk, 0, inv, args.steps, C.byref(ms)) == 0
                     gbs = 4.0 * big.numel() / (ms.value * 1e-3) / 1e9
                     pred_roof["runs"]["way%d_k%d_%s" % (wy, kk, "inverse" if inv else "forward")] = {"ms": ms.value, "achieved_gbs": gbs}
                 assert torch.equal(back, big), "predictor round trip mismatch"
@@ -492,7 +537,7 @@ def main():
         cpu = None
         if world == 1:
             try:
-                rb = reference_round_trip(pool[:4], nnum, way, hv, bdepth, 3, 2, settle=False)
+                rb = reference_round_trip(pool[:4], nnum, way, hv, bdepth, args.steps, 2, settle=False)
                 cpu = {"value": rb["raw"] / (rb["tc"] + rb["td"]) / 1e9, "unit": "GB/s", "cores": rb["cores"], "kind": rb["kind"], "sample": rb["sample"],
                        "compress_gbs": rb["raw"] / rb["tc"] / 1e9, "decompress_gbs": rb["raw"] / rb["td"] / 1e9}
             except Exception as ex:            # the baseline must never take the bench line down

@@ -47,7 +47,8 @@ int lfmCompressToBuffer(const void* im, const uint32_t xyzct[KLB_DATA_DIMS], con
 int lfmDecompressFromMemory(const void* file_bytes, uint64_t file_size, void* im);
 
 /* device-resident entry points (one GPU, the current lfmSetDevices first device). d_im / d_out are CUDA device pointers.
-   lfmCompressDevice leaves the compacted block streams on the device; *d_payload stays valid until the next call.
+   lfmCompressDevice leaves the compacted block streams on the device; *d_payload stays valid until the next call other than
+   lfmDecompressDevice, which only reads the payload it is given.
    blockOffset[Nb] (host) receives the inclusive prefix sum of the stream sizes = header.blockOffset[]. */
 int lfmCompressDevice(const void* d_im, const uint32_t xyzct[KLB_DATA_DIMS], const uint32_t blockSize[KLB_DATA_DIMS],
                       uint8_t headerVersion, uint8_t Nnum, uint8_t* storedHeaderVersion, uint64_t* blockOffset,
