@@ -83,6 +83,26 @@ int lfmWriteHeader(const char* filename, const uint32_t xyzct[KLB_DATA_DIMS], co
 /* number of KLB blocks for a stack (klb_imageHeader.cpp:77-85, after clamping blockSize to xyzct; NULL = default) */
 uint64_t lfmNumBlocks(const uint32_t xyzct[KLB_DATA_DIMS], const uint32_t blockSize[KLB_DATA_DIMS]);
 
+/* ---- standalone bzip2 streams of arbitrary bytes (no KLB framing), on the first device of lfmSetDevices.
+   lfmBz2Compress writes one bzip2 stream byte-identical to BZ2_bzBuffToBuffCompress(dst, &len, src, n, level, 0, 30), level 1..9,
+   any number of bzip2 blocks; n == 0 gives the 14-byte empty stream.  *dst_size receives the stream size; when `capacity` is
+   smaller, nothing is written and the call returns 5.  lfmBz2CompressDevice takes a device pointer and leaves the stream in an
+   engine-owned device buffer (*d_out, *out_size) that stays valid until the next call, as with lfmCompressDevice.
+   Return codes: 0 ok, 2 codec failure, 3 bad arguments (level outside 1..9, NULL with n > 0), 5 dst too small, 6 CUDA error,
+   7 input or stream of 2^32 bytes or more (the unsigned int limit of libbz2's buffer API).  lfmGetLastStats: ms_rle (run-length
+   structure, block boundaries and per-block run-length coding), ms_bwt, ms_mtf, ms_huff (Huffman coding and stream assembly),
+   payload_bytes = stream size, gpu_launches. */
+int lfmBz2Compress(const void* src, uint64_t n, int level, void* dst, uint64_t capacity, uint64_t* dst_size);
+int lfmBz2CompressDevice(const void* d_src, uint64_t n, int level, const void** d_out, uint64_t* out_size);
+/* any .bz2 data: one or more concatenated streams (bzip2, pbzip2, lbzip2 output), each with its own level, randomised blocks
+   included; block and stream CRCs checked.  *dst_size receives the decompressed size, known before any byte is written: when
+   `capacity` is smaller the call returns 5 and writes nothing.  Code 2: corrupt data (bad magic, CRC mismatch, truncated stream, a
+   block over 100000 * level bytes, bytes after the last stream that do not start another one, n == 0 as in
+   BZ2_bzBuffToBuffDecompress).  lfmGetLastStats: ms_decode (magic scan, speculative Huffman decode of every candidate block, chain
+   walk), ms_unrle (the real blocks: decode, inverse BWT, un-RLE1, CRCs), gpu_launches. */
+int lfmBz2Decompress(const void* src, uint64_t n, void* dst, uint64_t capacity, uint64_t* dst_size);
+int lfmBz2DecompressDevice(const void* d_src, uint64_t n, void* d_dst, uint64_t capacity, uint64_t* dst_size);
+
 /* statistics of the last compress / decompress call made by the calling thread */
 typedef struct {
 	int    predictor;         /* stored predictor 0..7 */

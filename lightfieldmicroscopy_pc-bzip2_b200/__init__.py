@@ -89,6 +89,14 @@ lib.lfmDebugEncodeBlock.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void
 lib.lfmDebugEncodeBlock.restype = C.c_int
 lib.lfmDebugPredictDevice.argtypes = [C.c_void_p, C.c_void_p, _u32x5, C.c_uint8, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float)]
 lib.lfmDebugPredictDevice.restype = C.c_int
+lib.lfmBz2Compress.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+lib.lfmBz2Compress.restype = C.c_int
+lib.lfmBz2CompressDevice.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
+lib.lfmBz2CompressDevice.restype = C.c_int
+lib.lfmBz2Decompress.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+lib.lfmBz2Decompress.restype = C.c_int
+lib.lfmBz2DecompressDevice.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+lib.lfmBz2DecompressDevice.restype = C.c_int
 
 _libc = C.CDLL(None)
 _libc.free.argtypes = [C.c_void_p]
@@ -97,7 +105,8 @@ EXPORTS = ["writeKLBstack", "writeKLBstackSlices", "readKLBheader", "readKLBstac
            "lfmSetPredictorWay", "lfmGetPredictorWay", "lfmSetDevices", "writeLFMstackEx", "readLFMheaderEx",
            "lfmCompressToMemory", "lfmCompressToBuffer", "lfmDecompressFromMemory", "lfmCompressDevice", "lfmDecompressDevice", "lfmNumBlocks",
            "lfmGetLastStats", "lfmLastError", "lfmDebugEncodeBlock", "lfmDebugPredictDevice", "lfmDebugParMemcpy",
-           "lfmShardCompress", "lfmShardWritePayload", "lfmShardFetchPayload", "lfmWriteHeader", "lfmSelectDevice"]
+           "lfmShardCompress", "lfmShardWritePayload", "lfmShardFetchPayload", "lfmWriteHeader", "lfmSelectDevice",
+           "lfmBz2Compress", "lfmBz2CompressDevice", "lfmBz2Decompress", "lfmBz2DecompressDevice"]
 
 
 class LfmError(RuntimeError):
@@ -282,3 +291,78 @@ def debug_encode_block(data):
     nblock, crc, orig, n_in_use, n_mtf, n_groups, n_sel, sbytes = list(info)
     return dict(nblock=nblock, crc=crc, orig_ptr=orig, n_in_use=n_in_use, n_mtf=n_mtf, n_groups=n_groups, n_sel=n_sel,
                 rle1=rle1[:nblock].copy(), bwt=bwt[:nblock].copy(), mtfv=mtfv[:n_mtf].copy(), stream=stream[:sbytes].tobytes())
+
+
+class _DeviceBytes:
+    """an engine-owned device buffer seen by torch through the CUDA array interface (no copy)"""
+
+    def __init__(self, ptr, nbytes):
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 2}
+
+
+def _is_cuda_tensor(data):
+    return type(data).__module__.startswith("torch") and getattr(data, "is_cuda", False)
+
+
+def bz2_compress(data, level=9):
+    """One bzip2 stream of `data`, byte-identical to BZ2_bzBuffToBuffCompress(.., level, 0, 30) (include/lfm_b200.h).
+    A bytes-like object or numpy array gives `bytes`; a CUDA torch.uint8 tensor (on the first device of set_devices) gives a
+    CUDA torch.uint8 tensor."""
+    if _is_cuda_tensor(data):
+        import torch
+        if data.dtype != torch.uint8:
+            raise TypeError("bz2_compress takes a torch.uint8 tensor")
+        src = data.contiguous().reshape(-1)
+        with torch.cuda.device(src.device):
+            torch.cuda.current_stream().synchronize()           # the engine runs on its own stream
+            p = C.c_void_p(); n = C.c_uint64()
+            rc = lib.lfmBz2CompressDevice(src.data_ptr() if src.numel() else None, src.numel(), int(level), C.byref(p), C.byref(n))
+            if rc:
+                raise LfmError(rc, "lfmBz2CompressDevice")
+            return torch.as_tensor(_DeviceBytes(p.value, n.value), device=src.device).clone()
+    src = np.ascontiguousarray(np.frombuffer(memoryview(data).cast("B"), np.uint8) if not isinstance(data, np.ndarray)
+                               else data.reshape(-1).view(np.uint8))
+    n = src.nbytes
+    cap = n + n // 64 + 1024 * (n // 99981 + 2) + 4096
+    out = np.empty(cap, np.uint8)
+    size = C.c_uint64()
+    rc = lib.lfmBz2Compress(src.ctypes.data if n else None, n, int(level), out.ctypes.data, cap, C.byref(size))
+    if rc == 5:                                                  # cannot happen with the bound above; retry with the size needed
+        out = np.empty(size.value, np.uint8)
+        rc = lib.lfmBz2Compress(src.ctypes.data if n else None, n, int(level), out.ctypes.data, size.value, C.byref(size))
+    if rc:
+        raise LfmError(rc, "lfmBz2Compress")
+    return out[:size.value].tobytes()
+
+
+def bz2_decompress(data):
+    """Any .bz2 data (one or more concatenated streams, any level) -> the original bytes, CRCs checked (include/lfm_b200.h).
+    A bytes-like object or numpy array gives `bytes`; a CUDA torch.uint8 tensor (on the first device of set_devices) gives a CUDA
+    torch.uint8 tensor.  The output is sized by one retry when the first guess is too small."""
+    size = C.c_uint64()
+    if _is_cuda_tensor(data):
+        import torch
+        if data.dtype != torch.uint8:
+            raise TypeError("bz2_decompress takes a torch.uint8 tensor")
+        src = data.contiguous().reshape(-1)
+        with torch.cuda.device(src.device):
+            torch.cuda.current_stream().synchronize()
+            out = torch.empty(4 * src.numel() + 4096, dtype=torch.uint8, device=src.device)
+            rc = lib.lfmBz2DecompressDevice(src.data_ptr() if src.numel() else None, src.numel(), out.data_ptr(), out.numel(), C.byref(size))
+            if rc == 5:
+                out = torch.empty(max(1, size.value), dtype=torch.uint8, device=src.device)
+                rc = lib.lfmBz2DecompressDevice(src.data_ptr(), src.numel(), out.data_ptr(), out.numel(), C.byref(size))
+            if rc:
+                raise LfmError(rc, "lfmBz2DecompressDevice")
+            return out[:size.value].clone()
+    src = np.ascontiguousarray(np.frombuffer(memoryview(data).cast("B"), np.uint8) if not isinstance(data, np.ndarray)
+                               else data.reshape(-1).view(np.uint8))
+    n = src.nbytes
+    out = np.empty(4 * n + 4096, np.uint8)
+    rc = lib.lfmBz2Decompress(src.ctypes.data if n else None, n, out.ctypes.data, out.nbytes, C.byref(size))
+    if rc == 5:
+        out = np.empty(max(1, size.value), np.uint8)
+        rc = lib.lfmBz2Decompress(src.ctypes.data, n, out.ctypes.data, out.nbytes, C.byref(size))
+    if rc:
+        raise LfmError(rc, "lfmBz2Decompress")
+    return out[:size.value].tobytes()

@@ -11,6 +11,7 @@
 //                 of the block into the symbol image
 #include "lfm_radix.cuh"
 #include "bz_randtable.h"
+#include "bz_rle1.cuh"
 #include <algorithm>
 #include <cstdlib>
 
@@ -50,11 +51,15 @@ __host__ __device__ inline size_t dec_sel_bytes(uint32_t selcap) { return (((siz
 
 extern __shared__ __align__(16) uint8_t dec_smem[];
 
-template <int DEC_LB>
+// SINGLE (standalone streams, bz_stream.cu): job = ONE bzip2 block that starts at bit begin[job] of the payload (its block magic),
+// no stream header; the level bound comes from job_level[job] (9 when NULL); end[0] = payload bytes.  The bit after the block's
+// last symbol goes to endbit[job] (~0 when the block does not decode), its stored CRC to crc_out[job].
+template <int DEC_LB, bool SINGLE>
 __global__ void __launch_bounds__(256)
 k_huff_decode(const uint8_t* __restrict__ payload, const uint64_t* __restrict__ begin, const uint64_t* __restrict__ end,
               uint32_t njobs, DecJob* __restrict__ jobs, uint16_t* __restrict__ mtfv_all, uint32_t mcap, uint32_t cap,
-              uint32_t selcap, uint32_t nsub)
+              uint32_t selcap, uint32_t nsub, uint64_t* __restrict__ endbit, uint32_t* __restrict__ crc_out,
+              const uint32_t* __restrict__ job_level)
 {
 	const uint32_t lane = lane_id(), w = warp_id(), nw = blockDim.x >> 5;
 	const uint32_t job = blockIdx.x * nw + w;
@@ -68,9 +73,10 @@ k_huff_decode(const uint8_t* __restrict__ payload, const uint64_t* __restrict__ 
 	uint16_t* so = reinterpret_cast<uint16_t*>(sw + DEC_RING);           // decoded symbols, flushed 32 at a time
 	// the stream's bzip2 blocks go to records job * nsub + kb (kb = 0, 1, ...); errors are reported in record 0
 	DecJob& J0 = jobs[(size_t)job * nsub];
-	const uint8_t* src = payload + begin[job];
-	const uint64_t nbytes = end[job] - begin[job];
-	#define FAIL(code) do { if (lane == 0) { J0.status = (code); J0.n = 0; J0.n_mtf = 0; } return; } while (0)
+	const uint64_t beg = SINGLE ? (begin[job] >> 3) : begin[job];
+	const uint8_t* src = payload + beg;
+	const uint64_t nbytes = end[SINGLE ? 0 : job] - beg;
+	#define FAIL(code) do { if (lane == 0) { J0.status = (code); J0.n = 0; J0.n_mtf = 0; if (SINGLE) endbit[job] = ~0ull; } return; } while (0)
 	for (uint32_t k = lane; k < nsub; k += 32) {
 		DecJob& Jk = jobs[(size_t)job * nsub + k];
 		Jk.n = 0; Jk.n_mtf = 0; Jk.out_bytes = 0; Jk.orig_ptr = 0; Jk.stored_crc = 0; Jk.status = 0; Jk.flags = kSubUnused; Jk.level = 0; Jk.max_block = 0;
@@ -115,13 +121,20 @@ k_huff_decode(const uint8_t* __restrict__ payload, const uint64_t* __restrict__ 
 	auto peek = [&](uint32_t nb) -> uint32_t { return (uint32_t)(bb >> (64 - nb)); };
 	auto get = [&](uint32_t nb) -> uint32_t { uint32_t v = peek(nb); drop(nb); return v; };
 
-	if (get(8) != 'B' || get(8) != 'Z' || get(8) != 'h') FAIL(1);
-	const int level = (int)get(8) - '0';
-	if (level < 1 || level > 9) FAIL(1);
+	int level;
+	if (SINGLE) {
+		drop((uint32_t)(begin[job] & 7u));
+		level = job_level ? (int)job_level[job] : 9;
+	} else {
+		if (get(8) != 'B' || get(8) != 'Z' || get(8) != 'h') FAIL(1);
+		level = (int)get(8) - '0';
+		if (level < 1 || level > 9) FAIL(1);
+	}
 	const uint32_t max_block = min((uint32_t)(100000 * level), cap);
 	uint32_t m1 = get(24), m2 = get(24);
 	uint32_t combined = 0, kb = 0;
 	for (;; kb++) {                                        // one bzip2 block per iteration (decompress.c:196-487)
+	if (SINGLE && (m1 != 0x314159 || m2 != 0x265359)) FAIL(1);
 	if (m1 == 0x177245 && m2 == 0x385090) break;           // end of stream
 	if (m1 != 0x314159 || m2 != 0x265359) FAIL(2);
 	if (kb >= nsub) FAIL(4);                               // more blocks than this block geometry can produce
@@ -370,6 +383,10 @@ k_huff_decode(const uint8_t* __restrict__ payload, const uint64_t* __restrict__ 
 		J.n_mtf = nsym; J.n_in_use = n_in_use; J.orig_ptr = orig_ptr; J.stored_crc = stored_crc; J.level = (uint32_t)level; J.status = 0;
 		J.max_block = max_block; J.flags = (kb == 0 ? kSubFirst : 0u) | (randomised ? kSubRand : 0u);
 		for (int k = 0; k < 8; k++) J.in_use[k] = iu[k];
+	}
+	if (SINGLE) {                                          // the block ends here: what follows is the chain walk's business
+		if (lane == 0) { J.flags |= kSubLast; endbit[job] = beg * 8 + (uint64_t)wi * 32 - bc; crc_out[job] = stored_crc; }
+		return;
 	}
 	combined = ((combined << 1) | (combined >> 31)) ^ stored_crc;         // bzlib.c / decompress.c: calculatedCombinedCRC
 	m1 = get(24); m2 = get(24);                            // next block header or end-of-stream magic
@@ -761,28 +778,122 @@ k_inv_bwt(const uint8_t* __restrict__ bwt_all, uint32_t cap, DecJob* __restrict_
 // =====================================================================================================
 constexpr int UR_NT = 256;
 
-__device__ __forceinline__ uint32_t ur_mulmod(uint32_t a, uint32_t b)
-{
-	uint32_t r = 0;
-	#pragma unroll 8
-	for (int i = 31; i >= 0; i--) {
-		r = (r << 1) ^ ((r & 0x80000000u) ? 0x04C11DB7u : 0u);
-		if ((b >> i) & 1u) r ^= a;
-	}
-	return r;
-}
-__device__ __forceinline__ uint32_t ur_xpow8(uint32_t nbytes)
-{
-	uint32_t e = nbytes * 8u, r = 1u;
-	for (int i = 31 - __clz(e | 1u); i >= 0; i--) {
-		r = ur_mulmod(r, r);
-		if ((e >> i) & 1u) r = (r << 1) ^ ((r & 0x80000000u) ? 0x04C11DB7u : 0u);
-	}
-	return r;
-}
-
 extern __shared__ __align__(16) uint8_t ur_smem[];
 
+// shared state of the run-length machine of one block (phases 1-2)
+template <int NT>
+struct UrShared {
+	uint32_t fn[NT];          // packed transition map of each chunk: 5 x 3 bits (then the CRC level multipliers)
+	uint32_t cnt[NT][5];      // bytes produced by each chunk for each entry state
+	uint32_t in[NT], off[NT];
+	uint32_t crc[NT];
+	uint32_t total;
+	uint32_t red[64];
+};
+
+// ---- 1 + 2. chunk maps, entry state and output offset of every chunk; returns the block's output length (all threads)
+template <int NT>
+__device__ __forceinline__ uint32_t ur_lengths(const uint8_t* txt, uint32_t n, uint32_t a0, uint32_t a1, UrShared<NT>& U)
+{
+	const uint32_t tid = threadIdx.x, lane = lane_id(), wid = warp_id();
+	{
+		// all five entry states in one pass over the chunk (each byte is loaded once)
+		uint32_t st[5] = { 0, 1, 2, 3, 4 }, cn[5] = { 0, 0, 0, 0, 0 };
+		uint32_t prev = a0 > 0 ? txt[a0 - 1] : 0x100u;
+		ByteReader rd;
+		if (a0 < a1) rd.init(txt, a0, a1);
+		// the five machines fall into step at the first run break that none of them reads as a count byte (a handful of
+		// bytes into the chunk): from there on ONE machine is simulated and its byte count added to all five
+		uint32_t i = a0;
+		bool same = false;
+		for (; i < a1 && !same; i++) {
+			const uint32_t ch = rd.get(i);
+			const bool eq = (ch == prev);
+			#pragma unroll
+			for (int m = 0; m < 5; m++) {
+				if (st[m] == 4) { cn[m] += ch; st[m] = 0; }
+				else { st[m] = (st[m] >= 1 && eq) ? st[m] + 1 : 1; cn[m]++; }
+			}
+			prev = ch;
+			same = (st[0] == st[1]) & (st[1] == st[2]) & (st[2] == st[3]) & (st[3] == st[4]);
+		}
+		if (same) {
+			uint32_t s1 = st[0], c1 = 0;
+			for (; i < a1; i++) {
+				const uint32_t ch = rd.get(i);
+				if (s1 == 4) { c1 += ch; s1 = 0; }
+				else { s1 = (s1 >= 1 && ch == prev) ? s1 + 1 : 1; c1++; }
+				prev = ch;
+			}
+			#pragma unroll
+			for (int m = 0; m < 5; m++) { st[m] = s1; cn[m] += c1; }
+		}
+		uint32_t fn = 0;
+		#pragma unroll
+		for (int m = 0; m < 5; m++) { fn |= st[m] << (3 * m); U.cnt[tid][m] = cn[m]; }
+		U.fn[tid] = fn;
+	}
+	__syncthreads();
+	// entry state / output offset of every chunk: inclusive scan of the composed transition maps (composition is associative),
+	// applied to the start state 0; then a block scan of the byte counts for those entry states
+	{
+		auto compose = [](uint32_t f, uint32_t g2) -> uint32_t {                      // first f, then g2
+			uint32_t h = 0;
+			#pragma unroll
+			for (int m = 0; m < 5; m++) { const uint32_t mid = (f >> (3 * m)) & 7u; h |= ((g2 >> (3 * mid)) & 7u) << (3 * m); }
+			return h;
+		};
+		const uint32_t ident = 0u | (1u << 3) | (2u << 6) | (3u << 9) | (4u << 12);
+		uint32_t f = U.fn[tid];
+		#pragma unroll
+		for (int o = 1; o < 32; o <<= 1) { const uint32_t pf = __shfl_up_sync(0xffffffffu, f, o); if (lane >= (uint32_t)o) f = compose(pf, f); }
+		if (lane == 31) U.in[wid] = f;                                                // U.in doubles as the warp totals for a moment
+		__syncthreads();
+		uint32_t before = ident;
+		for (uint32_t ww = 0; ww < wid; ww++) before = compose(before, U.in[ww]);
+		uint32_t ef = __shfl_up_sync(0xffffffffu, f, 1);
+		if (lane == 0) ef = ident;
+		const uint32_t excl = compose(before, ef);                                    // map of everything before my chunk
+		const uint32_t st_in = excl & 7u;                                              // applied to state 0
+		__syncthreads();
+		U.in[tid] = st_in;
+		uint32_t tot; const uint32_t incs = block_scan_add<NT>(U.cnt[tid][st_in], U.red, &tot);
+		U.off[tid] = incs - U.cnt[tid][st_in];
+		if (tid == 0) U.total = tot;
+	}
+	__syncthreads();
+	return U.total;
+}
+
+// ---- 3. replay my chunk from its entry state into out[obase + my offset ..]
+template <int NT>
+__device__ __forceinline__ void ur_replay(const uint8_t* txt, uint32_t a0, uint32_t a1, const UrShared<NT>& U, uint8_t* out, uint64_t obase)
+{
+	uint32_t st = U.in[threadIdx.x];
+	uint8_t* o = out + obase + U.off[threadIdx.x];
+	uint32_t pv = a0 > 0 ? txt[a0 - 1] : 0x100u;             // the byte before (never equal to a byte at the block start)
+	ByteReader rd;
+	if (a0 < a1) rd.init(txt, a0, a1);
+	for (uint32_t i = a0; i < a1; i++) {
+		const uint32_t ch = rd.get(i);
+		if (st == 4) { for (uint32_t k = 0; k < ch; k++) o[k] = (uint8_t)pv; o += ch; st = 0; }
+		else { st = (st >= 1 && ch == pv) ? st + 1 : 1; *o++ = (uint8_t)ch; }
+		pv = ch;
+	}
+}
+
+// =====================================================================================================
+// k_unrle : one CTA per block -- inverse of bzip2's initial run-length coding, CRC check, scatter into the image.
+// The decoder is a 5-state machine (state = equal bytes seen in a row, 4 = "next byte is a repeat count",
+// 0 = fresh start; bzlib.c:561-728).  Parallel form:
+//   1. thread t runs the machine over its chunk of the text for all 5 possible entry states -> (exit state, bytes out);
+//   2. the entry state and output offset of every chunk follow from composing those maps in chunk order;
+//   3. thread t replays its chunk from the now known entry state, writing into a staging copy of the block
+//      (shared memory; the block's dead BWT slot when it does not fit);
+//   4. CRC-32 of the staged block: per-chunk table CRC + binary tree of carry-less multiplications (rle1_crc, bz_rle1.cuh);
+//   5. rows are copied to the symbol image, one warp per row.
+// k_unrle_len / k_unrle_flat (standalone streams) run phases 1-2, and 1-4 into a flat output at the block's global offset.
+// =====================================================================================================
 template <int NT>
 __global__ void __launch_bounds__(NT)
 k_unrle(const uint8_t* __restrict__ txt_all, uint8_t* __restrict__ stage_all /* = BWT slots, dead by now */, uint32_t cap /* sub-slot */,
@@ -790,12 +901,7 @@ k_unrle(const uint8_t* __restrict__ txt_all, uint8_t* __restrict__ stage_all /* 
         int stage_in_smem)
 {
 	__shared__ uint32_t crc_tab[256];
-	__shared__ uint32_t s_fn[NT];          // packed transition map of each chunk: 5 x 3 bits
-	__shared__ uint32_t s_cnt[NT][5];      // bytes produced by each chunk for each entry state
-	__shared__ uint32_t s_in[NT], s_off[NT];
-	__shared__ uint32_t s_crc[NT];
-	__shared__ uint32_t s_total;
-	__shared__ uint32_t red[64];
+	__shared__ UrShared<NT> U;
 	const uint32_t tid = threadIdx.x, lane = lane_id(), wid = warp_id();
 	const uint32_t job = blockIdx.x;                                    // KLB block; its bzip2 blocks are records job * nsub + k
 	if (job >= njobs) return;
@@ -815,116 +921,13 @@ k_unrle(const uint8_t* __restrict__ txt_all, uint8_t* __restrict__ stage_all /* 
 		const uint8_t* txt = txt_all + ((size_t)job * nsub + kb) * cap;
 		const uint32_t n = J.n;
 		__syncthreads();
-		// ---- 1. chunk maps
 		const uint32_t CH = (n + NT - 1) / NT;
 		const uint32_t a0 = min(n, tid * CH), a1 = min(n, a0 + CH);
-		{
-			// all five entry states in one pass over the chunk (each byte is loaded once)
-			uint32_t st[5] = { 0, 1, 2, 3, 4 }, cn[5] = { 0, 0, 0, 0, 0 };
-			uint32_t prev = a0 > 0 ? txt[a0 - 1] : 0x100u;
-			ByteReader rd;
-			if (a0 < a1) rd.init(txt, a0, a1);
-			// the five machines fall into step at the first run break that none of them reads as a count byte (a handful of
-			// bytes into the chunk): from there on ONE machine is simulated and its byte count added to all five
-			uint32_t i = a0;
-			bool same = false;
-			for (; i < a1 && !same; i++) {
-				const uint32_t ch = rd.get(i);
-				const bool eq = (ch == prev);
-				#pragma unroll
-				for (int m = 0; m < 5; m++) {
-					if (st[m] == 4) { cn[m] += ch; st[m] = 0; }
-					else { st[m] = (st[m] >= 1 && eq) ? st[m] + 1 : 1; cn[m]++; }
-				}
-				prev = ch;
-				same = (st[0] == st[1]) & (st[1] == st[2]) & (st[2] == st[3]) & (st[3] == st[4]);
-			}
-			if (same) {
-				uint32_t s1 = st[0], c1 = 0;
-				for (; i < a1; i++) {
-					const uint32_t ch = rd.get(i);
-					if (s1 == 4) { c1 += ch; s1 = 0; }
-					else { s1 = (s1 >= 1 && ch == prev) ? s1 + 1 : 1; c1++; }
-					prev = ch;
-				}
-				#pragma unroll
-				for (int m = 0; m < 5; m++) { st[m] = s1; cn[m] += c1; }
-			}
-			uint32_t fn = 0;
-			#pragma unroll
-			for (int m = 0; m < 5; m++) { fn |= st[m] << (3 * m); s_cnt[tid][m] = cn[m]; }
-			s_fn[tid] = fn;
-		}
-		__syncthreads();
-		// ---- 2. entry state / output offset of every chunk: inclusive scan of the composed transition maps (composition
-		// is associative), applied to the start state 0; then a block scan of the byte counts for those entry states
-		{
-			auto compose = [](uint32_t f, uint32_t g2) -> uint32_t {                      // first f, then g2
-				uint32_t h = 0;
-				#pragma unroll
-				for (int m = 0; m < 5; m++) { const uint32_t mid = (f >> (3 * m)) & 7u; h |= ((g2 >> (3 * mid)) & 7u) << (3 * m); }
-				return h;
-			};
-			const uint32_t ident = 0u | (1u << 3) | (2u << 6) | (3u << 9) | (4u << 12);
-			uint32_t f = s_fn[tid];
-			#pragma unroll
-			for (int o = 1; o < 32; o <<= 1) { const uint32_t pf = __shfl_up_sync(0xffffffffu, f, o); if (lane >= (uint32_t)o) f = compose(pf, f); }
-			if (lane == 31) s_in[wid] = f;                                                // s_in doubles as the warp totals for a moment
-			__syncthreads();
-			uint32_t before = ident;
-			for (uint32_t ww = 0; ww < wid; ww++) before = compose(before, s_in[ww]);
-			uint32_t ef = __shfl_up_sync(0xffffffffu, f, 1);
-			if (lane == 0) ef = ident;
-			const uint32_t excl = compose(before, ef);                                    // map of everything before my chunk
-			const uint32_t st_in = excl & 7u;                                              // applied to state 0
-			__syncthreads();
-			s_in[tid] = st_in;
-			uint32_t tot; const uint32_t incs = block_scan_add<NT>(s_cnt[tid][st_in], red, &tot);
-			s_off[tid] = incs - s_cnt[tid][st_in];
-			if (tid == 0) s_total = tot;
-		}
-		__syncthreads();
-		const uint32_t len = s_total;
+		const uint32_t len = ur_lengths<NT>(txt, n, a0, a1, U);
 		if (len > gcount - obase) { if (tid == 0) { J0.status = 2; J0.out_bytes = obase + len; } return; }     // more than the KLB block holds
-		// ---- 3. replay into the staging copy
-		{
-			uint32_t st = s_in[tid], o = obase + s_off[tid];
-			uint32_t pv = a0 > 0 ? txt[a0 - 1] : 0x100u;             // the byte before (never equal to a byte at the block start)
-			ByteReader rd;
-			if (a0 < a1) rd.init(txt, a0, a1);
-			for (uint32_t i = a0; i < a1; i++) {
-				const uint32_t ch = rd.get(i);
-				if (st == 4) { for (uint32_t k = 0; k < ch; k++) stage[o + k] = (uint8_t)pv; o += ch; st = 0; }
-				else { st = (st >= 1 && ch == pv) ? st + 1 : 1; stage[o++] = (uint8_t)ch; }
-				pv = ch;
-			}
-		}
+		ur_replay<NT>(txt, a0, a1, U, stage, obase);
 		__syncthreads();
-		// ---- 4. CRC of this block's bytes (chunks right aligned: only the first non-empty one is short)
-		{
-			uint32_t CC = ((len + NT - 1) / NT + 3) & ~3u;
-			if (((CC >> 2) & 1u) == 0) CC += 4;
-			const uint32_t after = (NT - 1 - tid) * CC;
-			const uint32_t e1 = len > after ? len - after : 0;
-			const uint32_t e0 = e1 > CC ? e1 - CC : 0;
-			uint32_t crc = 0;
-			if (e1 > e0) {
-				crc = (e0 == 0) ? 0xFFFFFFFFu : 0u;
-				for (uint32_t j = obase + e0; j < obase + e1; j++) crc = (crc << 8) ^ crc_tab[(crc >> 24) ^ stage[j]];
-			}
-			s_crc[tid] = crc;
-			// x^(8 CC 2^k) mod P for the k-th tree level: thread k squares k times (s_fn is free by now)
-			if (tid < 12) { uint32_t M = ur_xpow8(CC); for (uint32_t q = 0; q < tid; q++) M = ur_mulmod(M, M); s_fn[tid] = M; }
-			__syncthreads();
-			{
-				uint32_t lvl = 0;
-				for (uint32_t stride = 1; stride < NT; stride <<= 1, lvl++) {
-					if ((tid & (2 * stride - 1)) == 0) s_crc[tid] = ur_mulmod(s_crc[tid], s_fn[lvl]) ^ s_crc[tid + stride];
-					__syncthreads();
-				}
-			}
-		}
-		if (~s_crc[0] != J.stored_crc) { if (tid == 0) J0.status = 3; return; }
+		if (rle1_crc<NT>(stage, obase, len, crc_tab, U.crc, U.fn) != J.stored_crc) { if (tid == 0) J0.status = 3; return; }
 		if (tid == 0) J.out_bytes = len;
 		obase += len;
 	}
@@ -940,12 +943,47 @@ k_unrle(const uint8_t* __restrict__ txt_all, uint8_t* __restrict__ stage_all /* 
 		const uint16_t* srcrow = reinterpret_cast<const uint16_t*>(stage) + (size_t)r * rowpx;
 		for (uint32_t x = lane; x < rowpx; x += 32) row[x] = srcrow[x];
 	}
+	(void)lane;
+}
+
+// lens[j] = output bytes of block j (0 when it failed an earlier stage: its status says why)
+__global__ void __launch_bounds__(UR_NT)
+k_unrle_len(const uint8_t* __restrict__ txt_all, uint32_t cap, const DecJob* __restrict__ jobs, uint32_t* __restrict__ lens)
+{
+	__shared__ UrShared<UR_NT> U;
+	const DecJob& J = jobs[blockIdx.x];
+	if (J.status != 0) { if (threadIdx.x == 0) lens[blockIdx.x] = 0; return; }
+	const uint8_t* txt = txt_all + (size_t)blockIdx.x * cap;
+	const uint32_t n = J.n, CH = (n + UR_NT - 1) / UR_NT;
+	const uint32_t a0 = min(n, threadIdx.x * CH), a1 = min(n, a0 + CH);
+	const uint32_t len = ur_lengths<UR_NT>(txt, n, a0, a1, U);
+	if (threadIdx.x == 0) lens[blockIdx.x] = len;
+}
+
+// block j replayed into out[boff[j] ..], CRC checked against the stored one (status 3)
+__global__ void __launch_bounds__(UR_NT)
+k_unrle_flat(const uint8_t* __restrict__ txt_all, uint32_t cap, DecJob* __restrict__ jobs, const uint64_t* __restrict__ boff, uint8_t* __restrict__ out)
+{
+	__shared__ uint32_t crc_tab[256];
+	__shared__ UrShared<UR_NT> U;
+	DecJob& J = jobs[blockIdx.x];
+	if (J.status != 0) return;
+	if (threadIdx.x < 256) crc_tab[threadIdx.x] = crc_table_entry(threadIdx.x);
+	const uint8_t* txt = txt_all + (size_t)blockIdx.x * cap;
+	const uint32_t n = J.n, CH = (n + UR_NT - 1) / UR_NT;
+	const uint32_t a0 = min(n, threadIdx.x * CH), a1 = min(n, a0 + CH);
+	const uint32_t len = ur_lengths<UR_NT>(txt, n, a0, a1, U);
+	if ((uint64_t)len != boff[blockIdx.x + 1] - boff[blockIdx.x]) { if (threadIdx.x == 0) J.status = 2; return; }
+	uint8_t* o = out + boff[blockIdx.x];
+	ur_replay<UR_NT>(txt, a0, a1, U, o, 0);
+	__syncthreads();
+	if (rle1_crc<UR_NT>(o, 0, len, crc_tab, U.crc, U.fn) != J.stored_crc && threadIdx.x == 0) J.status = 3;
 }
 
 // ------------------------------------------------------------------------------------------------ launchers
 int launch_decode(const uint8_t* payload, const uint64_t* begin, const uint64_t* end, uint32_t njobs, uint32_t nsub, DecJob* jobs,
                   uint16_t* mtfv, uint32_t mcap, uint8_t* q_scratch, uint8_t* bwt, uint32_t cap, uint32_t selcap, cudaStream_t st,
-                  cudaEvent_t between)
+                  cudaEvent_t between, uint64_t* endbit, uint32_t* crc_out, const uint32_t* job_level, bool imtf)
 {
 	static const int lb_forced = getenv("LFM_B200_DEC_LB") ? atoi(getenv("LFM_B200_DEC_LB")) : 0;
 	int dev = 0, sms = 148; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -966,14 +1004,14 @@ int launch_decode(const uint8_t* payload, const uint64_t* begin, const uint64_t*
 	if (nine) plan(sizeof(DecWarpSmemT<9>), nw, per_warp);
 	if (nw < 1) return 1;
 	const size_t smem = per_warp * nw;
-	if (nine) {
-		cudaFuncSetAttribute(k_huff_decode<9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-		k_huff_decode<9><<<(njobs + nw - 1) / nw, nw * 32, smem, st>>>(payload, begin, end, njobs, jobs, mtfv, mcap, cap, selcap, nsub);
-	} else {
-		cudaFuncSetAttribute(k_huff_decode<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-		k_huff_decode<10><<<(njobs + nw - 1) / nw, nw * 32, smem, st>>>(payload, begin, end, njobs, jobs, mtfv, mcap, cap, selcap, nsub);
-	}
+	auto go = [&](auto kern) {
+		cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+		kern<<<(njobs + nw - 1) / nw, nw * 32, smem, st>>>(payload, begin, end, njobs, jobs, mtfv, mcap, cap, selcap, nsub, endbit, crc_out, job_level);
+	};
+	if (endbit) { if (nine) go(k_huff_decode<9, true>); else go(k_huff_decode<10, true>); }
+	else { if (nine) go(k_huff_decode<9, false>); else go(k_huff_decode<10, false>); }
 	if (between) cudaEventRecord(between, st);               // stage timing: Huffman decode | inverse MTF
+	if (!imtf) return 0;
 	const size_t smem2 = imtf_smem_bytes();
 	cudaFuncSetAttribute(k_imtf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
 	k_imtf<<<njobs * nsub, IM_NT, smem2, st>>>(mtfv, mcap, jobs, njobs * nsub, q_scratch, bwt, cap);
@@ -1000,6 +1038,14 @@ void launch_inv_bwt(const uint8_t* bwt, uint32_t cap, DecJob* jobs, uint32_t njo
 	const size_t smem = (size_t)2 * (IB_MAXS + 2) * (4 + 2);
 	cudaFuncSetAttribute(k_inv_bwt<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 	k_inv_bwt<1024><<<grid, 1024, smem, st>>>(bwt, cap, jobs, njobs, tt_scratch, txt, (uint32_t)IB_MAXS);
+}
+void launch_unrle_len(const uint8_t* txt, uint32_t cap, const DecJob* jobs, uint32_t njobs, uint32_t* lens, cudaStream_t st)
+{
+	k_unrle_len<<<njobs, UR_NT, 0, st>>>(txt, cap, jobs, lens);
+}
+void launch_unrle_flat(const uint8_t* txt, uint32_t cap, DecJob* jobs, uint32_t njobs, const uint64_t* boff, uint8_t* out, cudaStream_t st)
+{
+	k_unrle_flat<<<njobs, UR_NT, 0, st>>>(txt, cap, jobs, boff, out);
 }
 void launch_unrle(const uint8_t* txt, uint8_t* stage_scratch, uint32_t cap, uint32_t nsub, uint32_t max_raw_bytes, DecJob* jobs, uint32_t njobs,
                   uint16_t* sym, const Geom& g, const uint64_t* block_ids, cudaStream_t st)

@@ -9,7 +9,7 @@
 //               MSB-first bit packing and stream framing     (compress.c:240-600 sendMTFValues, huffman.c:63-166,
 //               compress.c:603-676 BZ2_compressBlock header/trailer)
 #include <cstdio>
-#include "lfm_device.cuh"
+#include "bz_rle1.cuh"
 
 #include <cstdlib>
 namespace lfm {
@@ -28,32 +28,6 @@ namespace lfm {
 // (bzlib.c:216-354 ADD_CHAR_TO_BLOCK / add_pair_to_block / flush_RL; bzlib_private.h:157-171)
 // =====================================================================================================
 constexpr int RLE_NT = 256;                 // small blocks; blocks above 48 KB run with 1024 threads (one CTA per SM: occupancy)
-constexpr uint32_t kCrcPoly = 0x04C11DB7u;
-
-__device__ __forceinline__ uint32_t crc_mulmod(uint32_t a, uint32_t b)      // a * b in GF(2)[x] / P, bit k <-> x^k
-{
-	uint32_t r = 0;
-	#pragma unroll 8
-	for (int i = 31; i >= 0; i--) {
-		r = (r << 1) ^ ((r & 0x80000000u) ? kCrcPoly : 0u);
-		if ((b >> i) & 1u) r ^= a;
-	}
-	return r;
-}
-__device__ __forceinline__ uint32_t crc_xpow8(uint32_t nbytes)              // x^(8 nbytes) mod P
-{
-	uint32_t e = nbytes * 8u, r = 1u;
-	for (int i = 31 - __clz(e | 1u); i >= 0; i--) {
-		r = crc_mulmod(r, r);
-		if ((e >> i) & 1u) r = (r << 1) ^ ((r & 0x80000000u) ? kCrcPoly : 0u);
-	}
-	return r;
-}
-__device__ __forceinline__ uint32_t rle_g(uint32_t x)                        // outputs produced by run positions [0, x)
-{
-	uint32_t m = x % 255u;
-	return (x / 255u) * 5u + min(m, 4u) + (m >= 4u ? 1u : 0u);
-}
 
 extern __shared__ __align__(16) uint8_t rle_smem[];
 
@@ -93,77 +67,15 @@ k_rle1(const uint16_t* __restrict__ sym, Geom g, uint64_t first_block, uint32_t 
 	__syncthreads();
 	const uint8_t* b = stage;
 
-	// ---- B. chunks (right aligned) and run boundaries
-	uint32_t CH = ((gcount + NT - 1) / NT + 3) & ~3u;              // whole words, and an odd number of them:
-	if (((CH >> 2) & 1u) == 0) CH += 4;                                 // threads then hit distinct shared-memory banks
-	const uint32_t after = (NT - 1 - tid) * CH;                     // bytes owned by later threads
-	const uint32_t e1 = gcount > after ? gcount - after : 0;
-	const uint32_t e0 = e1 > CH ? e1 - CH : 0;
+	// ---- B. chunks (right aligned) and run boundaries (bz_rle1.cuh)
 	const uint32_t NONE = 0xFFFFFFFFu;
-	uint32_t first_head = NONE, last_head = NONE;
-	for (uint32_t i = e0; i < e1; i++) {
-		if (i == 0 || b[i] != b[i - 1]) { if (first_head == NONE) first_head = i; last_head = i; }
-	}
-	// start of the run that is open at my chunk start = last head before e0 (max-scan; heads ascend with the thread)
-	const uint32_t incl = block_scan_max<NT>(last_head == NONE ? 0u : last_head + 1u, red);     // +1 so that 0 = none
-	uint32_t prev_incl = __shfl_up_sync(0xffffffffu, incl, 1);
-	if (lane == 0) prev_incl = wid ? red[wid - 1] : 0;
-	const uint32_t open_start = prev_incl ? prev_incl - 1u : 0u;
-	// first head after my chunk (gcount if none): reverse min-scan done through shared memory
-	s_a[tid] = first_head;
-	__syncthreads();
-	{
-		// thread r looks at chunk NT-1-r: an inclusive max-scan of ~first_head over r is a suffix min-scan over the chunks
-		const uint32_t rv = s_a[NT - 1 - tid];
-		const uint32_t rincl = block_scan_max<NT>(~rv, red);                           // NONE -> 0
-		uint32_t rprev = __shfl_up_sync(0xffffffffu, rincl, 1);
-		if (lane == 0) rprev = wid ? red[wid - 1] : 0;
-		s_b[NT - 1 - tid] = rprev ? ~rprev : gcount;                                      // heads strictly after the chunk
-	}
-	__syncthreads();
-	const uint32_t next_head = s_b[tid];
+	const Rle1Chunk ck = rle1_chunk<NT>(b, 0, gcount, true, 0, gcount, red, s_a, s_b);
 
-	// ---- C. count, scan, [block boundaries], write. Walk the chunk run segment by run segment.
-	uint32_t outc = 0;
-	{
-		uint32_t i = e0, rs = open_start;
-		while (i < e1) {
-			if (i == 0 || b[i] != b[i - 1]) rs = i;
-			uint32_t e = i + 1;
-			while (e < e1 && b[e] == b[e - 1]) e++;
-			outc += rle_g(e - rs) - rle_g(i - rs);
-			i = e;
-		}
-	}
+	// ---- C. count, scan, [block boundaries], write
+	const uint32_t outc = rle1_count(b, ck);
 	uint32_t total; const uint32_t incs = block_scan_add<NT>(outc, red, &total);
 	const uint32_t n = total;
-
-	// One walk of the chunk in output order.  A RECORD is (a part of) a run of at most 255 equal bytes: up to 4 literals and,
-	// from 4 on, a count byte.  emit(o, byte) is called for every output byte, rec_end(o, in_end) after the last byte of
-	// every record that ends in this chunk's output (o = output offset after it, in_end = input offset after it).
-	auto walk = [&](auto emit, auto rec_end) {
-		uint32_t o = incs - outc, i = e0, rs = open_start;
-		while (i < e1) {
-			if (i == 0 || b[i] != b[i - 1]) rs = i;
-			const uint32_t ch = b[i];
-			uint32_t e = i + 1;
-			while (e < e1 && b[e] == b[e - 1]) e++;
-			const uint32_t run_end = (e < e1) ? e : next_head;       // where the whole run stops
-			const uint32_t run_len = run_end - rs;
-			uint32_t p = i;
-			while (p < e) {
-				const uint32_t r = p - rs, q = r % 255u;
-				if (q < 4) {
-					const uint32_t reclen = min(255u, run_len - (r - q));
-					emit(o++, (uint8_t)ch);
-					if (q == 3) { emit(o++, (uint8_t)(reclen - 4)); rec_end(o, rs + (r - 3) + reclen); }
-					else if (q + 1 == reclen) rec_end(o, rs + r + 1);
-					p++;
-				} else p += 255u - q;                                   // the rest of this 255-record emits nothing
-			}
-			i = e;
-		}
-	};
+	auto walk = [&](auto emit, auto rec_end) { rle1_walk(b, ck, incs - outc, emit, rec_end); };
 
 	// bzip2 closes a block after the record that brings it to nblockMAX bytes or more -- records are flushed when the first
 	// byte of the NEXT record is consumed (ADD_CHAR_TO_BLOCK, bzlib.c:216-258), the test sits before every input byte
@@ -218,43 +130,14 @@ k_rle1(const uint16_t* __restrict__ sym, Geom g, uint64_t first_block, uint32_t 
 	__syncthreads();
 	// 8 wrap-around bytes after every block (the sort reads text[i + 0..7]) and zero padding to a multiple of 4
 	for (uint32_t k = tid / 12; k < nb; k += NT / 12) {
-		const uint32_t t = tid % 12, nk = s_bout[k + 1] - s_bout[k];
-		uint8_t* ok = out0 + (size_t)k * cap;
-		const uint32_t pos = nk + t;
-		if (t < 8) ok[pos] = ok[t % nk];
-		else if (pos < ((nk + 8 + 3) & ~3u)) ok[pos] = 0;
+		rle1_wrap(out0 + (size_t)k * cap, s_bout[k + 1] - s_bout[k], tid % 12);
 	}
-	// ---- D. CRC-32 of every block's input bytes: per-chunk table CRC (chunks right aligned inside the block's input range: only
-	// the first non-empty one is short and carries the 0xFFFFFFFF start value), combined in a binary tree
+	// ---- D. CRC-32 of every block's input bytes (bz_rle1.cuh)
 	uint32_t combined = 0;
 	for (uint32_t k = 0; k < nb; k++) {
-		const uint32_t lo = s_bin[k], len = s_bin[k + 1] - lo;
-		uint32_t CC = ((len + NT - 1) / NT + 3) & ~3u;
-		if (((CC >> 2) & 1u) == 0) CC += 4;
-		const uint32_t aft = (NT - 1 - tid) * CC;
-		const uint32_t x1 = len > aft ? len - aft : 0;
-		const uint32_t x0 = x1 > CC ? x1 - CC : 0;
-		uint32_t crc = 0;
-		if (x1 > x0) {
-			crc = (x0 == 0) ? 0xFFFFFFFFu : 0u;
-			for (uint32_t j = lo + x0; j < lo + x1; j++) crc = (crc << 8) ^ crc_tab[(crc >> 24) ^ b[j]];
-		}
-		__syncthreads();
-		s_a[tid] = crc;
-		__syncthreads();
-		// x^(8 CC 2^k) mod P for the k-th tree level: thread k squares k times (instead of every thread squaring at every level)
-		if (tid < 12) { uint32_t M = crc_xpow8(CC); for (uint32_t q = 0; q < tid; q++) M = crc_mulmod(M, M); s_b[tid] = M; }
-		__syncthreads();
-		{
-			uint32_t lvl = 0;
-			for (uint32_t stride = 1; stride < NT; stride <<= 1, lvl++) {
-				if ((tid & (2 * stride - 1)) == 0) s_a[tid] = crc_mulmod(s_a[tid], s_b[lvl]) ^ s_a[tid + stride];
-				__syncthreads();
-			}
-		}
+		const uint32_t bc = rle1_crc<NT>(b, s_bin[k], s_bin[k + 1] - s_bin[k], crc_tab, s_a, s_b);
 		if (tid == 0) {
 			EncJob& J = jobs[(size_t)job * nsub + k];
-			const uint32_t bc = ~s_a[0];
 			combined = ((combined << 1) | (combined >> 31)) ^ bc;       // bzlib.c:  combinedCRC = (combinedCRC << 1 | >> 31) ^ blockCRC
 			J.raw_bytes = gcount; J.n = s_bout[k + 1] - s_bout[k]; J.crc = bc; J.status = 0; J.periodic = 0; J.orig_ptr = 0;
 			// the inUse map (bzlib.c:226, :243-258) is exactly "byte values with a non-zero count in the block": k_bwt derives

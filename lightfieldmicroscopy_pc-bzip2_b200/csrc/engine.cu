@@ -257,6 +257,14 @@ static Geom make_geom(const StackDesc& s)
 // nblockMAX .. nblockMAX + 4 run-length coded bytes (bzlib.c: nblockMAX = 100000 * level - 19, a block is closed by the
 // record that reaches it), so nsub = floor(maxn / nblockMAX) + 1 and a sub-slot holds nblockMAX + 10 bytes.
 struct EncSizes { uint32_t cap, mcap, selcap, ocap, nsub, nblock_max; int level; int text_in_smem; };
+static void slot_sizes(uint64_t subn, EncSizes& z)         // subn: most run-length coded bytes one block can hold
+{
+	z.cap = round16(subn + 8) + 16;
+	z.mcap = round16((uint64_t)z.cap + 2);
+	z.selcap = round16((uint64_t)z.mcap / kGSize + 2);
+	z.ocap = round16(subn + subn / 8 + subn / 16 + 8192);
+	z.text_in_smem = bwt_smem_bytes(z.cap, 1) <= 227 * 1024;
+}
 static int enc_sizes(const StackDesc& s, EncSizes& z)
 {
 	uint64_t blockBytes = 2;
@@ -267,13 +275,15 @@ static int enc_sizes(const StackDesc& s, EncSizes& z)
 	const uint64_t nsub = maxn / z.nblock_max + 1;
 	if (nsub > (uint64_t)kMaxSub || blockBytes > 0x7fffffffull / 2) return LFM_ERR_UNSUPPORTED;
 	z.nsub = (uint32_t)nsub;
-	const uint64_t subn = std::min<uint64_t>(maxn, (uint64_t)z.nblock_max + 10);
-	z.cap = round16(subn + 8) + 16;
-	z.mcap = round16((uint64_t)z.cap + 2);
-	z.selcap = round16((uint64_t)z.mcap / kGSize + 2);
-	z.ocap = round16(subn + subn / 8 + subn / 16 + 8192);
-	z.text_in_smem = bwt_smem_bytes(z.cap, 1) <= 227 * 1024;
+	slot_sizes(std::min<uint64_t>(maxn, (uint64_t)z.nblock_max + 10), z);
 	return LFM_OK;
+}
+// a standalone stream (bz2_compress): any number of blocks at the caller's level, one record per block
+static void stream_sizes(int level, EncSizes& z)
+{
+	z.level = level; z.nsub = 1;
+	z.nblock_max = (uint32_t)(100000 * level - 19);
+	slot_sizes((uint64_t)z.nblock_max + 10, z);
 }
 
 // ------------------------------------------------------------------------------------------------ selection
@@ -521,6 +531,236 @@ int Engine::fetch_encode_trace(EncodeTrace& t)
 	cudaMemcpyAsync(t.mtfv.data(), mtfv_.p, t.mtfv.size() * 2, cudaMemcpyDeviceToHost, st);
 	cudaStreamSynchronize(st);
 	return check("fetch_encode_trace");
+}
+
+// ------------------------------------------------------------------------------------------------ standalone bzip2 stream
+uint8_t* Engine::bz2_staging(size_t bytes)
+{
+	cudaSetDevice(device_);
+	return reserve(sz_in_, bytes + 16) ? nullptr : (uint8_t*)sz_in_.p;
+}
+
+// One stream of any number of bzip2 blocks (bz_stream.cu): the RLE1 structure of the whole input and the block boundaries first,
+// then the blocks in batches through the stages of the KLB path, each batch's bits assembled into the stream before the next one
+// reuses the slots.  Workspace beyond the input and the stream: the slots of one batch (as compress_blocks), a record per tile of
+// kSzTile input bytes, a record per block and the record-end bitmap (one bit per run-length coded byte).
+int Engine::bz2_compress(const uint8_t* d_src, uint64_t n, int level, const uint8_t** d_out, uint64_t* out_size, CompressStats* stt)
+{
+	cudaSetDevice(device_);
+	cudaStream_t st = (cudaStream_t)stream_;
+	if (level < 1 || level > 9) { err_ = "level must be 1..9"; return LFM_ERR_OPEN; }
+	if (n >= (1ull << 32)) { err_ = "input of 2^32 bytes or more"; return LFM_ERR_UNSUPPORTED; }
+	EncSizes z; stream_sizes(level, z);
+	const uint32_t n32 = (uint32_t)n, nt = sz_tiles(n);
+	const uint64_t max_rle = n + n / 4 + 1;                                    // RLE1 worst case: 4 -> 5 bytes
+	const uint32_t max_blocks = (uint32_t)(max_rle / z.nblock_max + 2);
+	const uint64_t bitmap_words = (max_rle + 31) / 32 + 2;
+	const uint64_t out_cap = (n + n / 64 + 1024ull * max_blocks + 4096) & ~3ull;
+	const size_t per_job = (size_t)z.cap * 3 + (size_t)z.mcap * 2 + (size_t)z.selcap * 2 + z.ocap + sizeof(EncJob);
+	uint32_t B = (uint32_t)std::min<uint64_t>(max_blocks, std::max<uint64_t>(1, ((size_t)6 << 30) / per_job));
+	B = std::min<uint32_t>(B, 16384);
+	const int grid = (int)std::min<uint64_t>(B, (uint64_t)sm_count_ * bwt_ctas_per_sm(z.cap, z.text_in_smem));
+	int rc;
+	if ((rc = reserve(sz_tiles_, (size_t)nt * 5 * 4 + ((size_t)nt + 1) * 8 + 64))) return rc;
+	if ((rc = reserve(sz_bits_, bitmap_words * 4))) return rc;
+	if ((rc = reserve(sz_blocks_, ((size_t)max_blocks + 1) * 12 + ((size_t)B + 1) * 8 + 64))) return rc;
+	if ((rc = reserve(sz_out_, out_cap + 16))) return rc;
+	if ((rc = reserve(jobs_, (size_t)B * sizeof(EncJob)))) return rc;
+	if ((rc = reserve(txt_, (size_t)B * z.cap))) return rc;
+	if ((rc = reserve(bwt_, (size_t)B * z.cap))) return rc;
+	if ((rc = reserve(rank_, (size_t)B * z.cap))) return rc;
+	if ((rc = reserve(mtfv_, (size_t)B * z.mcap * 2))) return rc;
+	if ((rc = reserve(sel_, (size_t)B * z.selcap * 2))) return rc;
+	if ((rc = reserve(out_, (size_t)B * z.ocap + 16))) return rc;
+	if ((rc = reserve(scratch_, (size_t)grid * bwt_scratch_elems_per_cta(z.cap) * 4))) return rc;
+	uint64_t* tobase = (uint64_t*)sz_tiles_.p;                                 // [nt + 1]
+	uint32_t* t32 = (uint32_t*)(tobase + nt + 1);
+	uint32_t *tfirst = t32, *tlast = t32 + nt, *topen = t32 + 2 * (size_t)nt, *tnext = t32 + 3 * (size_t)nt, *tcount = t32 + 4 * (size_t)nt;
+	uint64_t* bout = (uint64_t*)sz_blocks_.p;                                  // [max_blocks + 1]
+	uint64_t* bitoff = bout + max_blocks + 1;                                  // [B + 1]
+	SzRun* run = (SzRun*)(bitoff + B + 1);
+	uint32_t* nbp = (uint32_t*)(run + 1);
+	uint32_t* combined = nbp + 1;
+	uint32_t* bin = combined + 1;                                              // [max_blocks + 1]
+	cudaMemsetAsync(run, 0, sizeof(SzRun) + 8 + ((size_t)max_blocks + 1) * 4, st);
+	cudaMemsetAsync(sz_out_.p, 0, out_cap, st);
+
+	std::vector<cudaEvent_t> evs;
+	auto mark = [&]() { if (stt) { cudaEvent_t e = (cudaEvent_t)pooled_event(evs.size()); cudaEventRecord(e, st); evs.push_back(e); } };
+	uint64_t launches = 0;
+	mark();
+	uint32_t nb = 1;
+	if (n > 0) {
+		launch_sz_runs(d_src, n32, tfirst, tlast, topen, tnext, st);
+		launch_sz_count(d_src, n32, topen, tnext, tcount, tobase, st);
+		launch_sz_chain(d_src, n32, topen, tnext, tobase, (uint32_t*)sz_bits_.p, bitmap_words, z.nblock_max, max_blocks, bout, nbp, st);
+		launches += 6;
+		cudaMemcpyAsync(&nb, nbp, 4, cudaMemcpyDeviceToHost, st);
+		cudaStreamSynchronize(st);
+		if ((rc = check("bz2_compress structure"))) return rc;
+		cudaMemcpyAsync(bin + nb, &n32, 4, cudaMemcpyHostToDevice, st);          // bin[0] = 0 from the memset
+		launch_sz_locate(d_src, n32, topen, tnext, tobase, bout, bin, nb, st);
+		launches += nb > 1 ? 1 : 0;
+	} else {
+		cudaMemsetAsync(bout, 0, 16, st);                                      // one empty block: header and trailer only
+	}
+	mark();
+	for (uint32_t k0 = 0; k0 < nb; k0 += B) {
+		const uint32_t nj = std::min<uint32_t>(B, nb - k0);
+		EncJob* jobs = (EncJob*)jobs_.p;
+		mark();
+		launch_sz_emit(d_src, bin, bout, k0, nj, nb, (uint8_t*)txt_.p, z.cap, jobs, combined, st);
+		mark();
+		launch_bwt((uint8_t*)txt_.p, z.cap, jobs, nj, (uint8_t*)bwt_.p, (uint32_t*)scratch_.p, (int)std::min<uint32_t>(nj, (uint32_t)grid), z.text_in_smem, st);
+		mark();
+		launch_mtf((uint8_t*)bwt_.p, (uint8_t*)rank_.p, z.cap, jobs, nj, (uint16_t*)mtfv_.p, z.mcap, st);
+		mark();
+		launch_huff_pack((uint16_t*)mtfv_.p, z.mcap, jobs, nj, (uint8_t*)sel_.p, z.selcap, (uint8_t*)out_.p, z.ocap, level, st);
+		launch_sz_assemble(jobs, nj, (uint8_t*)out_.p, z.ocap, bitoff, run, (uint8_t*)sz_out_.p, out_cap, sm_count_, st);
+		mark();
+		launches += 6 + (k0 + nj == nb ? 1 : 0);
+	}
+	SzRun h;
+	cudaMemcpyAsync(&h, run, sizeof(h), cudaMemcpyDeviceToHost, st);
+	cudaStreamSynchronize(st);
+	if ((rc = check("bz2_compress"))) return rc;
+	if (stt) {
+		stt->ms_rle += elapsed_or_zero(evs[0], evs[1]);
+		for (size_t i = 2; i + 4 < evs.size(); i += 5) {
+			stt->ms_rle += elapsed_or_zero(evs[i], evs[i + 1]);
+			stt->ms_bwt += elapsed_or_zero(evs[i + 1], evs[i + 2]);
+			stt->ms_mtf += elapsed_or_zero(evs[i + 2], evs[i + 3]);
+			stt->ms_huff += elapsed_or_zero(evs[i + 3], evs[i + 4]);          // Huffman coding + stream assembly
+		}
+		stt->launches += launches;
+	}
+	if (h.err) { err_ = "block encoder reported an error"; return LFM_ERR_BZIP; }
+	const uint64_t bytes = (h.bits + 7) / 8;
+	if (bytes > out_cap) { err_ = "stream buffer overflow"; return LFM_ERR_BZIP; }
+	if (bytes >= (1ull << 32)) { err_ = "compressed stream of 2^32 bytes or more"; return LFM_ERR_UNSUPPORTED; }
+	*d_out = (const uint8_t*)sz_out_.p;
+	*out_size = bytes;
+	return LFM_OK;
+}
+
+// Any .bz2 data (bz_stream.cu): candidate magics at every bit, every candidate decoded speculatively as a block (Huffman stage
+// only, in batches) to learn where it ends, the chain walk keeps the real blocks; then the real blocks in batches through
+// k_huff_decode / k_imtf / k_inv_bwt and the un-RLE1 length pass, a prefix sum of the lengths, the capacity check, and the replay
+// into the flat output (the batches are decoded again when there is more than one).
+int Engine::bz2_decompress(const void* src, uint64_t n, bool src_on_host, uint8_t* d_dst, uint64_t capacity, const uint8_t** d_out,
+                           uint64_t* out_size, DecompressStats* stt)
+{
+	cudaSetDevice(device_);
+	cudaStream_t st = (cudaStream_t)stream_;
+	if (n == 0) { err_ = "empty input"; return LFM_ERR_BZIP; }
+	if (n >= (1ull << 32)) { err_ = "input of 2^32 bytes or more"; return LFM_ERR_UNSUPPORTED; }
+	EncSizes z; stream_sizes(9, z);                                            // slots for the largest block
+	const uint32_t nt = sz_tiles(n);
+	const size_t per_job = (size_t)z.cap * 2 + (size_t)z.mcap * 2 + sizeof(DecJob) + 24;
+	const uint32_t B = (uint32_t)std::min<uint64_t>(16384, std::max<uint64_t>(1, ((size_t)6 << 30) / per_job));
+	int rc;
+	if ((rc = reserve(dz_in_, n + 64))) return rc;
+	if ((rc = reserve(sz_tiles_, (size_t)nt * 4 + ((size_t)nt + 1) * 8 + 64))) return rc;
+	uint8_t* in = (uint8_t*)dz_in_.p;
+	cudaMemcpyAsync(in, src, n, src_on_host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st);
+	cudaMemsetAsync(in + n, 0, 64, st);
+	uint64_t* tbase = (uint64_t*)sz_tiles_.p;
+	uint32_t* tcount = (uint32_t*)(tbase + nt + 1);
+	std::vector<cudaEvent_t> evs;
+	auto mark = [&]() { if (stt) { cudaEvent_t e = (cudaEvent_t)pooled_event(evs.size()); cudaEventRecord(e, st); evs.push_back(e); } };
+	mark();
+	launch_bz_magic(in, n, 0, tcount, tbase, nullptr, nullptr, st);
+	uint64_t nc64 = 0;
+	cudaMemcpyAsync(&nc64, tbase + nt, 8, cudaMemcpyDeviceToHost, st);
+	cudaStreamSynchronize(st);
+	if ((rc = check("bz2_decompress magic scan"))) return rc;
+	if (nc64 == 0) { err_ = "no bzip2 block or end-of-stream magic"; return LFM_ERR_BZIP; }
+	const uint32_t nc = (uint32_t)nc64;
+	// candidate records: cbit, cend, bbit (u64); ccrc, succ, blev, blen (u32); ceos (u8); boff (u64, nc + 1); dn, res
+	if ((rc = reserve(dz_cand_, (size_t)nc * (3 * 8 + 4 * 4 + 1) + ((size_t)nc + 1) * 8 + 256))) return rc;
+	uint64_t* cbit = (uint64_t*)dz_cand_.p; uint64_t* cend = cbit + nc; uint64_t* bbit = cend + nc; uint64_t* boff = bbit + nc;
+	uint64_t* dn = boff + nc + 1;
+	uint32_t* res = (uint32_t*)(dn + 1);
+	uint32_t* ccrc = res + 4; uint32_t* succ = ccrc + nc; uint32_t* blev = succ + nc; uint32_t* blen = blev + nc;
+	uint8_t* ceos = (uint8_t*)(blen + nc);
+	cudaMemcpyAsync(dn, &n, 8, cudaMemcpyHostToDevice, st);
+	launch_bz_magic(in, n, 1, tcount, tbase, cbit, ceos, st);
+	const uint32_t grid = (uint32_t)std::min<uint64_t>(B, (uint64_t)sm_count_ * inv_bwt_ctas_per_sm(z.cap));
+	if ((rc = reserve(djobs_, (size_t)B * sizeof(DecJob) + 16))) return rc;
+	if ((rc = reserve(bwt_, (size_t)B * z.cap))) return rc;
+	if ((rc = reserve(txt_, (size_t)B * z.cap))) return rc;
+	if ((rc = reserve(mtfv_, (size_t)B * z.mcap * 2))) return rc;
+	if ((rc = reserve(tt_, inv_bwt_scratch_elems(grid, z.cap) * 4))) return rc;
+	DecJob* jobs = (DecJob*)djobs_.p;
+	uint32_t* flag = (uint32_t*)(jobs + B);
+	cudaMemsetAsync(flag, 0, 4, st);
+	uint64_t launches = 2;
+	mark();
+	// ---- speculative pass: where does every candidate block end
+	for (uint32_t c0 = 0; c0 < nc; c0 += B) {
+		const uint32_t nj = std::min(B, nc - c0);
+		if (launch_decode(in, cbit + c0, dn, nj, 1, jobs, (uint16_t*)mtfv_.p, z.mcap, (uint8_t*)txt_.p, (uint8_t*)bwt_.p, z.cap, z.selcap, st,
+		                  nullptr, cend + c0, ccrc + c0, nullptr, false)) { err_ = "decoder launch failed"; return LFM_ERR_UNSUPPORTED; }
+		launches++;
+	}
+	launch_bz_chain(in, n, cbit, ceos, nc, cend, ccrc, succ, bbit, blev, res, st);
+	launches += 2;
+	uint32_t hres[2] = { 0, 0 };
+	cudaMemcpyAsync(hres, res, 8, cudaMemcpyDeviceToHost, st);
+	cudaStreamSynchronize(st);
+	if ((rc = check("bz2_decompress chain"))) return rc;
+	mark();
+	if (hres[1]) { err_ = "corrupt bzip2 data: the blocks do not chain from the stream header to the end of the input"; return LFM_ERR_BZIP; }
+	const uint32_t nb = hres[0];
+	const uint32_t nbatch = (nb + B - 1) / B;
+	auto decode_batch = [&](uint32_t k0, uint32_t nj) -> int {
+		if (launch_decode(in, bbit + k0, dn, nj, 1, jobs, (uint16_t*)mtfv_.p, z.mcap, (uint8_t*)txt_.p, (uint8_t*)bwt_.p, z.cap, z.selcap, st,
+		                  nullptr, cend + k0, ccrc + k0, blev + k0, true)) { err_ = "decoder launch failed"; return LFM_ERR_UNSUPPORTED; }
+		launch_inv_bwt((uint8_t*)bwt_.p, z.cap, jobs, nj, (uint32_t*)tt_.p, (uint8_t*)txt_.p, (int)std::min(nj, grid), st);
+		launches += 3;
+		return LFM_OK;
+	};
+	// ---- blocks: decode, lengths
+	for (uint32_t k0 = 0; k0 < nb; k0 += B) {
+		const uint32_t nj = std::min(B, nb - k0);
+		if ((rc = decode_batch(k0, nj))) return rc;
+		launch_unrle_len((uint8_t*)txt_.p, z.cap, jobs, nj, blen + k0, st);
+		k_dec_status<<<(nj + 255) / 256, 256, 0, st>>>(jobs, nj, flag);
+		launches += 2;
+	}
+	launch_scan_u32(nb, blen, boff, st);
+	launches++;
+	uint64_t total = 0; uint32_t hflag = 0;
+	cudaMemcpyAsync(&total, boff + nb, 8, cudaMemcpyDeviceToHost, st);
+	cudaMemcpyAsync(&hflag, flag, 4, cudaMemcpyDeviceToHost, st);
+	cudaStreamSynchronize(st);
+	if ((rc = check("bz2_decompress blocks"))) return rc;
+	if (hflag) { char m[96]; snprintf(m, sizeof(m), "corrupt bzip2 block (decoder status mask 0x%x)", hflag); err_ = m; return LFM_ERR_BZIP; }
+	*out_size = total;
+	if (total >= (1ull << 32)) { err_ = "decompressed data of 2^32 bytes or more"; return LFM_ERR_UNSUPPORTED; }
+	if (total > capacity) { err_ = "destination buffer too small"; return LFM_ERR_CREATE; }
+	uint8_t* out = d_dst;
+	if (!out) { if ((rc = reserve(dz_out_, total + 16))) return rc; out = (uint8_t*)dz_out_.p; }
+	// ---- replay into the flat output, block CRCs checked
+	for (uint32_t k0 = 0; k0 < nb; k0 += B) {
+		const uint32_t nj = std::min(B, nb - k0);
+		if (nbatch > 1 && (rc = decode_batch(k0, nj))) return rc;
+		launch_unrle_flat((uint8_t*)txt_.p, z.cap, jobs, nj, boff + k0, out, st);
+		k_dec_status<<<(nj + 255) / 256, 256, 0, st>>>(jobs, nj, flag);
+		launches += 2;
+	}
+	mark();
+	cudaMemcpyAsync(&hflag, flag, 4, cudaMemcpyDeviceToHost, st);
+	cudaStreamSynchronize(st);
+	if ((rc = check("bz2_decompress"))) return rc;
+	if (stt) {
+		stt->ms_decode += elapsed_or_zero(evs[0], evs[2]);                    // magic scan, speculative decode, chain walk
+		stt->ms_unrle += elapsed_or_zero(evs[2], evs[3]);                     // blocks: decode, inverse BWT, un-RLE1, CRCs
+		stt->launches += launches;
+	}
+	if (hflag) { char m[96]; snprintf(m, sizeof(m), "block CRC mismatch (decoder status mask 0x%x)", hflag); err_ = m; return LFM_ERR_BZIP; }
+	*d_out = out;
+	return LFM_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ decompress

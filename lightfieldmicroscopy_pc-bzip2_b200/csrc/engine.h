@@ -64,6 +64,18 @@ public:
 	int decompress_blocks(const uint8_t* d_payload, const uint64_t* begin, const uint64_t* end, const uint64_t* block_ids,
 	                      uint64_t count, uint16_t* d_sym, const StackDesc& s, DecompressStats* st);
 
+	// One bzip2 stream of the device-resident bytes d_src[0, n), byte-identical to BZ2_bzBuffToBuffCompress(.., level, 0, 30);
+	// n < 2^32, level 1..9.  The stream is left in an engine-owned device buffer (*d_out, *out_size) valid until the next call.
+	int bz2_compress(const uint8_t* d_src, uint64_t n, int level, const uint8_t** d_out, uint64_t* out_size, CompressStats* st);
+	// Any .bz2 data (src: n bytes, host or device memory) -> its decompressed bytes: one or more concatenated streams, block
+	// and stream CRCs checked.  Output into d_dst (device, `capacity` bytes) or, when d_dst is NULL, an engine-owned device
+	// buffer (*d_out) valid until the next call.  *out_size = decompressed size; LFM_ERR_CREATE (5) when it exceeds capacity
+	// (nothing written).
+	int bz2_decompress(const void* src, uint64_t n, bool src_on_host, uint8_t* d_dst, uint64_t capacity, const uint8_t** d_out,
+	                   uint64_t* out_size, DecompressStats* st);
+	// device buffer of at least `bytes` for a caller's input that has to be staged on this GPU first
+	uint8_t* bz2_staging(size_t bytes);
+
 	// Inverse predictor (unsymbolize fused) over frames [z0, z0+nz); in place is NOT allowed (d_sym != d_out).
 	int unpredict(const uint16_t* d_sym, uint16_t* d_out, const StackDesc& s, int predictor, int video, uint32_t z0, uint32_t nz);
 
@@ -116,6 +128,8 @@ private:
 	int pay_sel_ = 0;
 	Buf djobs_, dbegin_, dend_, dids_, tt_;
 	Buf sel_sorted_, sel_hist_, sel_e_, sel_cand_;
+	Buf sz_tiles_, sz_bits_, sz_blocks_, sz_out_, sz_in_;      // bz2_compress: tile records, record-end bitmap, block records, stream, staging
+	Buf dz_in_, dz_cand_, dz_out_;                              // bz2_decompress: padded input, candidate / block records, output
 	uint32_t last_cap_ = 0, last_mcap_ = 0, last_njobs_ = 0;
 	void* pin_[2] = { nullptr, nullptr }; size_t pin_cap_[2] = { 0, 0 };
 	static constexpr int kMaxGroups = 4;   // forked streams a small batch is spread over

@@ -1326,6 +1326,128 @@ try {
 /* test hook (no GPU needed): the threaded host copy the staging paths use (pageable <-> pinned memory, mapped file ranges) */
 int lfmDebugParMemcpy(void* dst, const void* src, uint64_t n) { if (!dst || !src) return 1; par_memcpy(dst, src, (size_t)n); return 0; }
 
+// ---- standalone bzip2 streams (bz_stream.cu): one stream per call, on the first device of lfmSetDevices
+namespace {
+int bz2_compress_core(Engine& e, const uint8_t* d_src, uint64_t n, int level, const void** d_out, uint64_t* out_size)
+{
+	CompressStats st;
+	const uint8_t* p = nullptr; uint64_t bytes = 0;
+	const int rc = e.bz2_compress(d_src, n, level, &p, &bytes, &st);
+	if (rc) { g_err = e.last_error(); return rc; }
+	g_stats.ms_rle = st.ms_rle; g_stats.ms_bwt = st.ms_bwt; g_stats.ms_mtf = st.ms_mtf; g_stats.ms_huff = st.ms_huff;
+	g_stats.gpu_launches += st.launches; g_stats.payload_bytes = bytes;
+	*d_out = p; *out_size = bytes;
+	return LFM_OK;
+}
+}
+
+int lfmBz2CompressDevice(const void* d_src, uint64_t n, int level, const void** d_out, uint64_t* out_size)
+try {
+	LFM_API_LOCK();
+	memset(&g_stats, 0, sizeof(g_stats));
+	if ((!d_src && n > 0) || !d_out || !out_size || level < 1 || level > 9) return LFM_ERR_OPEN;
+	if (n >= (1ull << 32)) { g_err = "input of 2^32 bytes or more"; return LFM_ERR_UNSUPPORTED; }
+	if (current_ndev() <= 0) return LFM_ERR_CUDA;
+	Engine& e = Engine::for_device(g_set.first_device);
+	cudaSetDevice(e.device());
+	if (n > 0) {
+		cudaPointerAttributes a;
+		if (cudaPointerGetAttributes(&a, d_src) != cudaSuccess) { cudaGetLastError(); return LFM_ERR_OPEN; }
+		if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) { g_err = "d_src is not device memory"; return LFM_ERR_OPEN; }
+		if (a.device != e.device()) { g_err = "d_src is not on the first device of lfmSetDevices"; return LFM_ERR_OPEN; }
+	}
+	const double t0 = now_ms();
+	const int rc = bz2_compress_core(e, (const uint8_t*)d_src, n, level, d_out, out_size);
+	g_stats.ms_total = now_ms() - t0;
+	return rc;
+} LFM_CATCH
+
+int lfmBz2Compress(const void* src, uint64_t n, int level, void* dst, uint64_t capacity, uint64_t* dst_size)
+try {
+	LFM_API_LOCK();
+	memset(&g_stats, 0, sizeof(g_stats));
+	if ((!src && n > 0) || !dst_size || level < 1 || level > 9) return LFM_ERR_OPEN;
+	if (n >= (1ull << 32)) { g_err = "input of 2^32 bytes or more"; return LFM_ERR_UNSUPPORTED; }
+	if (current_ndev() <= 0) return LFM_ERR_CUDA;
+	Engine& e = Engine::for_device(g_set.first_device);
+	cudaSetDevice(e.device());
+	cudaStream_t st = (cudaStream_t)e.stream();
+	const double t0 = now_ms();
+	uint8_t* d_in = e.bz2_staging(n);
+	if (!d_in) { g_err = e.last_error(); return LFM_ERR_CUDA; }
+	if (n) cudaMemcpyAsync(d_in, src, n, cudaMemcpyHostToDevice, st);
+	cudaStreamSynchronize(st);
+	const double t1 = now_ms();
+	const void* d_out = nullptr; uint64_t bytes = 0;
+	int rc = bz2_compress_core(e, d_in, n, level, &d_out, &bytes);
+	g_stats.ms_h2d = t1 - t0;
+	if (rc) return rc;
+	*dst_size = bytes;
+	if (!dst || capacity < bytes) { g_err = "destination buffer too small"; g_stats.ms_total = now_ms() - t0; return LFM_ERR_CREATE; }
+	const double t2 = now_ms();
+	cudaMemcpyAsync(dst, d_out, bytes, cudaMemcpyDeviceToHost, st);
+	cudaStreamSynchronize(st);
+	if (cudaGetLastError() != cudaSuccess) { g_err = "copy of the stream to the host failed"; return LFM_ERR_CUDA; }
+	g_stats.ms_d2h = now_ms() - t2;
+	g_stats.ms_total = now_ms() - t0;
+	return LFM_OK;
+} LFM_CATCH
+
+namespace {
+int bz2_decompress_core(const void* src, uint64_t n, bool on_host, uint8_t* d_dst, uint64_t capacity, const void** d_out, uint64_t* out_size)
+{
+	if (current_ndev() <= 0) return LFM_ERR_CUDA;
+	Engine& e = Engine::for_device(g_set.first_device);
+	cudaSetDevice(e.device());
+	DecompressStats st;
+	const uint8_t* p = nullptr; uint64_t bytes = 0;
+	const int rc = e.bz2_decompress(src, n, on_host, d_dst, capacity, &p, &bytes, &st);
+	*out_size = bytes;
+	if (rc) { g_err = e.last_error(); return rc; }
+	g_stats.ms_decode = st.ms_decode; g_stats.ms_unrle = st.ms_unrle;
+	g_stats.gpu_launches += st.launches; g_stats.payload_bytes = n;
+	*d_out = p;
+	return LFM_OK;
+}
+}
+
+int lfmBz2Decompress(const void* src, uint64_t n, void* dst, uint64_t capacity, uint64_t* dst_size)
+try {
+	LFM_API_LOCK();
+	memset(&g_stats, 0, sizeof(g_stats));
+	if ((!src && n > 0) || !dst_size || (!dst && capacity > 0)) return LFM_ERR_OPEN;
+	if (n == 0) { g_err = "empty input"; return LFM_ERR_BZIP; }
+	if (n >= (1ull << 32)) { g_err = "input of 2^32 bytes or more"; return LFM_ERR_UNSUPPORTED; }
+	const double t0 = now_ms();
+	const void* d_out = nullptr; uint64_t bytes = 0;
+	int rc = bz2_decompress_core(src, n, true, nullptr, capacity, &d_out, &bytes);
+	*dst_size = bytes;
+	if (rc) return rc;
+	Engine& e = Engine::for_device(g_set.first_device);
+	cudaStream_t st = (cudaStream_t)e.stream();
+	const double t2 = now_ms();
+	if (bytes) cudaMemcpyAsync(dst, d_out, bytes, cudaMemcpyDeviceToHost, st);
+	cudaStreamSynchronize(st);
+	if (cudaGetLastError() != cudaSuccess) { g_err = "copy of the data to the host failed"; return LFM_ERR_CUDA; }
+	g_stats.ms_d2h = now_ms() - t2;
+	g_stats.ms_total = now_ms() - t0;
+	return LFM_OK;
+} LFM_CATCH
+
+int lfmBz2DecompressDevice(const void* d_src, uint64_t n, void* d_dst, uint64_t capacity, uint64_t* dst_size)
+try {
+	LFM_API_LOCK();
+	memset(&g_stats, 0, sizeof(g_stats));
+	if ((!d_src && n > 0) || !dst_size || (!d_dst && capacity > 0)) return LFM_ERR_OPEN;
+	if (n == 0) { g_err = "empty input"; return LFM_ERR_BZIP; }
+	if (n >= (1ull << 32)) { g_err = "input of 2^32 bytes or more"; return LFM_ERR_UNSUPPORTED; }
+	const double t0 = now_ms();
+	const void* d_out = nullptr;
+	const int rc = bz2_decompress_core(d_src, n, false, (uint8_t*)d_dst, capacity, &d_out, dst_size);
+	g_stats.ms_total = now_ms() - t0;
+	return rc;
+} LFM_CATCH
+
 int lfmGetLastStats(lfm_stats* out) { if (!out) return 1; *out = g_stats; return 0; }
 const char* lfmLastError(void) { return g_err.c_str(); }
 
