@@ -32,6 +32,27 @@ int writeLFMstackEx(const void* im, const char* filename, const uint32_t xyzct[K
                     enum KLB_COMPRESSION_TYPE compressionType, const char metadata[KLB_METADATA_SIZE],
                     uint8_t headerVersion, uint8_t Nnum);
 
+/* ---- device-resident files: the pixels stay in GPU memory, only the compressed payload crosses PCIe.
+   Both calls run on the first device of lfmSetDevices only, also with lfmSetDevices(first, n > 1), and return with the engine
+   stream synchronised.  The caller's buffer must be device or managed memory on that device (code 3 otherwise); a caller
+   that writes it on another stream synchronises that stream first.
+
+   writeLFMstackEx with the stack in DEVICE memory (d_im: x fastest, frames = z*c*t).  Same arguments, same return codes, and a
+   file byte-identical to what writeLFMstackEx writes for the same pixels.  lfmGetLastStats: ms_h2d stays 0. */
+int writeLFMstackDevice(const void* d_im, const char* filename, const uint32_t xyzct[KLB_DATA_DIMS], enum KLB_DATA_TYPE dataType,
+                        int numThreads, const float32_t pixelSize[KLB_DATA_DIMS], const uint32_t blockSize[KLB_DATA_DIMS],
+                        enum KLB_COMPRESSION_TYPE compressionType, const char metadata[KLB_METADATA_SIZE],
+                        uint8_t headerVersion, uint8_t Nnum);
+/* decode a file, or the box lb..ub of it (inclusive x,y,z,c,t bounds; both NULL = whole stack), into DEVICE memory d_out:
+   dense [t][c][z][y][x] of the box, the same pixels readKLBstackInPlace / readKLBroiInPlace return.  *out_bytes (may be NULL)
+   receives the size of the box in bytes; when capacity is smaller the call returns 5 and writes nothing to d_out.  Any 2-byte
+   aligned d_out works; a whole-stack read decodes in place only into a 16-byte aligned d_out (cudaMalloc's are), into any
+   other one through the engine's frame buffers and one more device copy.
+   Return codes: 2 truncated or corrupt file, 3 a file that cannot be opened (readKLBstackInPlace gives 2 there), a box outside
+   the stack or a bad d_out, 6 no CUDA device, 7 ZLIB payloads or pixels that are not 16-bit.  lfmGetLastStats: ms_d2h stays 0. */
+int readLFMroiDevice(const char* filename, const uint32_t lb[KLB_DATA_DIMS], const uint32_t ub[KLB_DATA_DIMS],
+                     void* d_out, uint64_t capacity, uint64_t* out_bytes);
+
 /* header byte 0 / byte 1 of a file (stored predictor | video bit, Nnum); 0 ok */
 int readLFMheaderEx(const char* filename, uint8_t* headerVersion, uint8_t* Nnum);
 

@@ -63,6 +63,10 @@ lib.lfmGetPredictorWay.restype = C.c_int
 lib.lfmSetDevices.argtypes = [C.c_int, C.c_int]; lib.lfmSetDevices.restype = C.c_int
 lib.writeLFMstackEx.argtypes = [C.c_void_p, C.c_char_p, _u32x5, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_uint8, C.c_uint8]
 lib.writeLFMstackEx.restype = C.c_int
+lib.writeLFMstackDevice.argtypes = lib.writeLFMstackEx.argtypes
+lib.writeLFMstackDevice.restype = C.c_int
+lib.readLFMroiDevice.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+lib.readLFMroiDevice.restype = C.c_int
 lib.readLFMheaderEx.argtypes = [C.c_char_p, C.POINTER(C.c_uint8), C.POINTER(C.c_uint8)]
 lib.readLFMheaderEx.restype = C.c_int
 lib.lfmCompressToMemory.argtypes = [C.c_void_p, _u32x5, C.c_void_p, C.c_uint8, C.c_uint8, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
@@ -106,7 +110,8 @@ EXPORTS = ["writeKLBstack", "writeKLBstackSlices", "readKLBheader", "readKLBstac
            "lfmCompressToMemory", "lfmCompressToBuffer", "lfmDecompressFromMemory", "lfmCompressDevice", "lfmDecompressDevice", "lfmNumBlocks",
            "lfmGetLastStats", "lfmLastError", "lfmDebugEncodeBlock", "lfmDebugPredictDevice", "lfmDebugParMemcpy",
            "lfmShardCompress", "lfmShardWritePayload", "lfmShardFetchPayload", "lfmWriteHeader", "lfmSelectDevice",
-           "lfmBz2Compress", "lfmBz2CompressDevice", "lfmBz2Decompress", "lfmBz2DecompressDevice"]
+           "lfmBz2Compress", "lfmBz2CompressDevice", "lfmBz2Decompress", "lfmBz2DecompressDevice",
+           "writeLFMstackDevice", "readLFMroiDevice"]
 
 
 class LfmError(RuntimeError):
@@ -146,7 +151,11 @@ def stats():
 
 
 def write_stack(img, filename, header_version=0, nnum=13, block_size=None, way=None, codec=BZIP2):
-    """img: uint16 array [..., z, y, x]. Mirrors writeKLBstack + the header knobs (writeLFMstackEx)."""
+    """img: uint16 array [..., z, y, x]. Mirrors writeKLBstack + the header knobs (writeLFMstackEx).
+    img may also be a CUDA torch.uint16 or torch.int16 tensor (uint16 bits, as lf_synth_int makes them) on the first device of
+    set_devices: it is compressed where it is (writeLFMstackDevice), into the same file the numpy copy would give."""
+    if _is_cuda_tensor(img):
+        return _write_stack_device(img, filename, header_version, nnum, block_size, way, codec)
     img = np.ascontiguousarray(img, dtype=np.uint16)
     if way is not None:
         set_way(way)
@@ -169,11 +178,56 @@ def read_header(filename):
                 metadata=meta.raw, headerVersion=hv.value, Nnum=nn.value)
 
 
-def read_stack(filename, way=None):
+def _write_stack_device(img, filename, header_version, nnum, block_size, way, codec):
+    import torch
+    if img.dtype not in (torch.uint16, torch.int16):
+        raise TypeError("write_stack takes a torch.uint16 or torch.int16 tensor")
+    src = img.view(torch.int16).contiguous()
+    if way is not None:
+        set_way(way)
+    bs = _bs(block_size)
+    with torch.cuda.device(src.device):
+        torch.cuda.current_stream().synchronize()               # the engine runs on its own stream
+        rc = lib.writeLFMstackDevice(src.data_ptr(), os.fsencode(filename), _xyzct(src.shape), UINT16_TYPE, -1, None,
+                                     C.cast(bs, C.c_void_p) if bs is not None else None, codec, None, header_version, nnum)
+    if rc:
+        raise LfmError(rc, "writeLFMstackDevice")
+    return rc
+
+
+def _read_device(filename, lb, ub, shape, device, out):
+    """decode the box lb..ub (None, None: the whole stack) of a file into a CUDA tensor: `out`, or a new torch.uint16 tensor of
+    `shape` on `device`"""
+    import torch
+    nbytes = 2 * int(np.prod(shape))
+    if out is None:
+        out = torch.empty(shape, dtype=torch.uint16, device=device)
+    elif not _is_cuda_tensor(out) or not out.is_contiguous() or out.numel() * out.element_size() != nbytes:
+        raise ValueError("out= takes a contiguous CUDA tensor of %d bytes" % nbytes)
+    elif device is not None:
+        d = torch.device(device)
+        if d.type != "cuda" or (d.index if d.index is not None else torch.cuda.current_device()) != out.device.index:
+            raise ValueError("device=%s and out= on %s name different devices" % (device, out.device))
+    n = C.c_uint64()
+    with torch.cuda.device(out.device):
+        torch.cuda.current_stream().synchronize()               # the engine runs on its own stream
+        rc = lib.readLFMroiDevice(os.fsencode(filename), lb, ub, out.data_ptr(), nbytes, C.byref(n))
+    if rc:
+        raise LfmError(rc, "readLFMroiDevice")
+    return out
+
+
+def read_stack(filename, way=None, device=None, out=None):
+    """[z][y][x] (c == t == 1) or [t][c][z][y][x] uint16 array of the whole stack.  With `device` (a CUDA device) or `out` (a
+    contiguous CUDA tensor of the stack's size in bytes) the stack is decoded into GPU memory instead (readLFMroiDevice) and comes
+    back as a torch.uint16 tensor of that shape, or as `out` itself; only the compressed payload crosses PCIe.  Given both,
+    `device` must name the device `out` is on (ValueError otherwise)."""
     if way is not None:
         set_way(way)
     h = read_header(filename)
     x, y, z, c, t = h["xyzct"]
+    if device is not None or out is not None:
+        return _read_device(filename, None, None, (z, y, x) if (c == 1 and t == 1) else (t, c, z, y, x), device, out)
     out = np.empty((t, c, z, y, x), dtype=np.uint16)
     dt = C.c_int()
     rc = lib.readKLBstackInPlace(os.fsencode(filename), out.ctypes.data, C.byref(dt), -1)
@@ -182,11 +236,14 @@ def read_stack(filename, way=None):
     return out.reshape((z, y, x)) if (c == 1 and t == 1) else out
 
 
-def read_roi(filename, lb, ub, way=None):
-    """lb/ub: inclusive x,y,z,c,t bounds. Returns array [t][c][z][y][x] of the ROI."""
+def read_roi(filename, lb, ub, way=None, device=None, out=None):
+    """lb/ub: inclusive x,y,z,c,t bounds. Returns array [t][c][z][y][x] of the ROI.  With `device` or `out` as in read_stack, a
+    CUDA torch.uint16 tensor of that shape (or `out`)."""
     if way is not None:
         set_way(way)
     shape = [ub[i] - lb[i] + 1 for i in range(5)]
+    if device is not None or out is not None:
+        return _read_device(filename, _u32x5(*lb), _u32x5(*ub), tuple(shape[::-1]), device, out)
     out = np.empty(shape[::-1], dtype=np.uint16)
     rc = lib.readKLBroiInPlace(os.fsencode(filename), out.ctypes.data, _u32x5(*lb), _u32x5(*ub), -1)
     if rc:

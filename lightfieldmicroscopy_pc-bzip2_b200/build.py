@@ -6,7 +6,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "liblfm_b200.so")
-CU = ["bz_bwt.cu", "bz_encode.cu", "bz_decode.cu", "bz_stream.cu", "lfm_predict.cu", "lfm_select.cu", "engine.cu"]
+CU = ["bz_bwt.cu", "bz_encode.cu", "bz_decode.cu", "bz_stream.cu", "lfm_predict.cu", "lfm_select.cu", "lfm_roi.cu", "engine.cu"]
 CPP = ["klb_imageHeader.cpp", "klb_ROI.cpp", "klb_imageIO.cpp", "klb_Cwrapper.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

@@ -79,6 +79,10 @@ public:
 	// Inverse predictor (unsymbolize fused) over frames [z0, z0+nz); in place is NOT allowed (d_sym != d_out).
 	int unpredict(const uint16_t* d_sym, uint16_t* d_out, const StackDesc& s, int predictor, int video, uint32_t z0, uint32_t nz);
 
+	// The box lb..ub (inclusive x,y,z,c,t bounds) of the decoded frames d_frames (absolute frame indexing) -> dense
+	// [t][c][z][y][x] at d_out, one k_roi_gather launch on the engine stream (not synchronised).
+	int roi_gather(const uint16_t* d_frames, const StackDesc& s, const uint32_t lb[5], const uint32_t ub[5], uint16_t* d_out);
+
 	// device time of the last predict() / unpredict() call (valid once the stream has been synchronised)
 	double last_predict_ms();
 	double last_unpredict_ms();

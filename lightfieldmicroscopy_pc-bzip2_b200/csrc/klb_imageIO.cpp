@@ -71,7 +71,14 @@ double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::
 struct FrameSource {              // contiguous stack or one pointer per XY slice
 	const uint16_t* base = nullptr;
 	const uint16_t* const* slices = nullptr;
+	bool device = false;          // base is a contiguous stack in device memory of the first device: nothing is uploaded
 	const uint16_t* frame(uint64_t f, uint64_t fpx) const { return slices ? slices[f] : base + f * fpx; }
+};
+// Where decoded pixels go when they stay on the GPU: the caller's device buffer of `capacity` bytes (dense box of the read)
+struct DeviceSink {
+	void* d_out = nullptr;
+	uint64_t capacity = 0;
+	uint64_t* out_bytes = nullptr;
 };
 
 struct Layout {                   // derived block / frame geometry
@@ -142,6 +149,20 @@ int validate(const klb_image_header& h, bool writing)
 		return LFM_ERR_UNSUPPORTED;
 	}
 	for (int d = 0; d < 5; d++) if (h.xyzct[d] == 0 || h.blockSize[d] == 0) return LFM_ERR_BZIP;
+	return LFM_OK;
+}
+
+// a caller's buffer for the device-resident file calls: device or managed memory on the first device of lfmSetDevices, holding
+// whole 16-bit pixels (code 3 otherwise)
+int check_device_ptr(const void* p, const char* what)
+{
+	const int dev = Engine::for_device(g_set.first_device).device();
+	cudaPointerAttributes a;
+	if (!p || ((uintptr_t)p & 1) || cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+		cudaGetLastError(); g_err = std::string(what) + " is not a CUDA pointer to 16-bit pixels"; return LFM_ERR_OPEN;
+	}
+	if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) { g_err = std::string(what) + " is not device memory"; return LFM_ERR_OPEN; }
+	if (a.device != dev) { g_err = std::string(what) + " is not on the first device of lfmSetDevices"; return LFM_ERR_OPEN; }
 	return LFM_OK;
 }
 
@@ -398,13 +419,15 @@ static int compress_pipelined(const FrameSource& src, klb_image_header& h, const
 		max_nf = std::max(max_nf, B[b].nf);
 	}
 	const size_t img_bytes = (size_t)max_nf * L.fpx * 2;
-	if (e.reserve(e.user[UB_IMG], img_bytes) || e.reserve(e.user[UB_IMG2], img_bytes) || (k != 0 && e.reserve(e.user[UB_SYM], img_bytes))) return LFM_ERR_CUDA;
+	if ((!src.device && (e.reserve(e.user[UB_IMG], img_bytes) || e.reserve(e.user[UB_IMG2], img_bytes))) ||
+	    (k != 0 && e.reserve(e.user[UB_SYM], img_bytes))) return LFM_ERR_CUDA;
 	if (!e.pinned(kStageBufs * kStageChunk, 0) || !e.pinned(kStageBufs * kStageChunk, 1)) return LFM_ERR_CUDA;
 	uint16_t* dimg[2] = { (uint16_t*)e.user[UB_IMG].p, (uint16_t*)e.user[UB_IMG2].p };
 	uint16_t* dsym = (uint16_t*)e.user[UB_SYM].p;
 	std::thread up_th[2], wr_th[2];
 	int up_rc[2] = { 0, 0 }, wr_rc[2] = { 0, 0 };
 	auto upload = [&](uint64_t b, int slot) {
+		if (src.device) return;                                        // the kernels read the caller's device stack
 		cudaSetDevice(dev);
 		const Batch& bt = B[b];
 		if (src.base) h2d_staged(e, dimg[slot], src.frame(bt.f0, L.fpx), (size_t)bt.nf * L.fpx * 2, up_st);
@@ -424,7 +447,7 @@ static int compress_pipelined(const FrameSource& src, klb_image_header& h, const
 		if (b + 1 < nbatch) up_th[slot ^ 1] = std::thread(upload, b + 1, slot ^ 1);   // its image buffer was last read by batch b - 1 (done)
 		if (wr_th[slot].joinable()) { wr_th[slot].join(); if ((rc = wr_rc[slot])) break; }   // payload buffer `slot` (batch b - 2) is on disk
 		const Batch& bt = B[b];
-		const uint16_t* img_base = dimg[slot] - bt.f0 * L.fpx;         // virtual base: absolute frame indexing
+		const uint16_t* img_base = src.device ? src.base : dimg[slot] - bt.f0 * L.fpx;   // virtual base: absolute frame indexing
 		const uint16_t* sym_base = img_base;
 		CompressStats st;
 		if (k != 0) {
@@ -470,6 +493,7 @@ int compress_core(const FrameSource& src, klb_image_header& h, std::vector<Shard
 	if (rc) return rc;
 	const int ndev = current_ndev();
 	if (ndev <= 0) { std::cout << "ERROR: lfm_b200: no CUDA device available (this engine has no CPU fallback)" << std::endl; return LFM_ERR_CUDA; }
+	if (src.device && (rc = check_device_ptr(src.base, "d_im"))) return rc;
 	const int way = current_way();
 	for (int d = 0; d < 5; d++) h.blockSize[d] = std::min(h.blockSize[d], h.xyzct[d]);     // src/klb_imageIO.cpp:2407-2408
 	const Layout L = make_layout(h);
@@ -483,12 +507,16 @@ int compress_core(const FrameSource& src, klb_image_header& h, std::vector<Shard
 		// auto-select on frame 0 (branches A and B of writeImage, src/klb_imageIO.cpp:2273-2377)
 		Engine& e = Engine::for_device(g_set.first_device);
 		cudaSetDevice(e.device());
-		if (e.reserve(e.user[UB_F0], L.fpx * 2)) return LFM_ERR_CUDA;
-		// stream-ordered copy: a default-stream cudaMemcpy from pageable memory may return before the DMA has landed,
-		// and the engine's non-blocking stream does not wait for the default stream
-		cudaMemcpyAsync(e.user[UB_F0].p, src.frame(0, L.fpx), L.fpx * 2, cudaMemcpyHostToDevice, (cudaStream_t)e.stream());
+		const uint16_t* f0 = src.base;
+		if (!src.device) {
+			if (e.reserve(e.user[UB_F0], L.fpx * 2)) return LFM_ERR_CUDA;
+			// stream-ordered copy: a default-stream cudaMemcpy from pageable memory may return before the DMA has landed,
+			// and the engine's non-blocking stream does not wait for the default stream
+			cudaMemcpyAsync(e.user[UB_F0].p, src.frame(0, L.fpx), L.fpx * 2, cudaMemcpyHostToDevice, (cudaStream_t)e.stream());
+			f0 = (const uint16_t*)e.user[UB_F0].p;
+		}
 		double t0 = now_ms();
-		rc = e.select_mode((const uint16_t*)e.user[UB_F0].p, desc, g_stats.entropy, &k);
+		rc = e.select_mode(f0, desc, g_stats.entropy, &k);
 		if (rc) { g_err = e.last_error(); return rc; }
 		g_stats.ms_select = now_ms() - t0;
 		g_stats.selected = 1; g_stats.gpu_launches += 7 + 5;       // 7 candidate predictions + count, starts, sort, histogram, entropy
@@ -503,7 +531,8 @@ int compress_core(const FrameSource& src, klb_image_header& h, std::vector<Shard
 	h.headerVersion = (uint8_t)((hv_in & 0x80) | k);
 	g_stats.predictor = k;
 
-	const int D = (int)std::min<uint64_t>((uint64_t)ndev, L.nSlabs);
+	// a device stack lives on the first device: it is compressed there alone
+	const int D = src.device ? 1 : (int)std::min<uint64_t>((uint64_t)ndev, L.nSlabs);
 	if (sink && D == 1) {
 		const uint64_t per = slabs_per_batch(h, L, k != 0 && video);
 		if (per) {
@@ -527,12 +556,13 @@ int compress_core(const FrameSource& src, klb_image_header& h, std::vector<Shard
 		out.device = e.device();
 		cudaSetDevice(e.device());
 		cudaStream_t st = (cudaStream_t)e.stream();
-		if (e.reserve(e.user[UB_IMG], nf * L.fpx * 2) || (k != 0 && e.reserve(e.user[UB_SYM], nf * L.fpx * 2))) { out.rc = LFM_ERR_CUDA; return; }
+		if ((!src.device && e.reserve(e.user[UB_IMG], nf * L.fpx * 2)) || (k != 0 && e.reserve(e.user[UB_SYM], nf * L.fpx * 2))) { out.rc = LFM_ERR_CUDA; return; }
 		uint16_t* dimg = (uint16_t*)e.user[UB_IMG].p; uint16_t* dsym = (uint16_t*)e.user[UB_SYM].p;
 		double t0 = now_ms();
-		if (src.base) h2d_staged(e, dimg, src.frame(f0, L.fpx), nf * L.fpx * 2, st);
+		if (src.device) { /* the kernels read the caller's device stack */ }
+		else if (src.base) h2d_staged(e, dimg, src.frame(f0, L.fpx), nf * L.fpx * 2, st);
 		else for (uint64_t f = 0; f < nf; f++) cudaMemcpyAsync(dimg + f * L.fpx, src.frame(f0 + f, L.fpx), L.fpx * 2, cudaMemcpyHostToDevice, st);
-		const uint16_t* img_base = dimg - f0 * L.fpx;       // virtual base: absolute frame indexing
+		const uint16_t* img_base = src.device ? src.base : dimg - f0 * L.fpx;       // virtual base: absolute frame indexing
 		const uint16_t* sym_base = img_base;
 		if (k != 0) {
 			out.rc = e.predict(img_base, dsym - f0 * L.fpx, desc, k, video, (uint32_t)f0, (uint32_t)nf);
@@ -545,7 +575,7 @@ int compress_core(const FrameSource& src, klb_image_header& h, std::vector<Shard
 		out.sizes.resize(count);
 		out.rc = e.compress_blocks(sym_base, desc, first, count, out.sizes.data(), &out.d_payload, &out.payload_bytes, &out.st);
 		if (k != 0 && out.rc == 0) out.st.ms_predict = e.last_predict_ms();
-		out.ms_h2d = now_ms() - t0;                         // H2D + kernels (the copy is asynchronous and overlaps nothing yet)
+		out.ms_h2d = src.device ? 0 : now_ms() - t0;        // H2D + kernels (the copy is asynchronous and overlaps nothing yet)
 		if (out.rc) { out.err = e.last_error(); return; }
 	};
 	if (D == 1) work(0);
@@ -640,8 +670,9 @@ struct PayloadSource {
 // Full reads of large stacks on one GPU, the mirror image of compress_pipelined: while batch b (whole z-slabs) is decoded and
 // un-predicted, the streams of batch b + 1 are read from the file / host memory into the second payload buffer (pinned staging,
 // copy stream 0, own host thread) and the pixels of batch b - 1 travel to the caller's buffer (copy stream 1, own host thread).
+// With out_on_device, `out` is the caller's device buffer: the batches decode straight into it and there is no download stage.
 static int decompress_pipelined(const klb_image_header& h, const Layout& L, const StackDesc& desc, int k, int video,
-                                const PayloadSource& psrc, uint16_t* out, uint64_t per)
+                                const PayloadSource& psrc, uint16_t* out, bool out_on_device, uint64_t per)
 {
 	Engine& e = Engine::for_device(g_set.first_device);
 	cudaSetDevice(e.device());
@@ -661,8 +692,9 @@ static int decompress_pipelined(const klb_image_header& h, const Layout& L, cons
 		max_nf = std::max(max_nf, bt.nf); max_pay = std::max(max_pay, bt.end - bt.beg);
 	}
 	const size_t img_bytes = (size_t)max_nf * L.fpx * 2;
-	if (e.reserve(e.user[UB_PAY], max_pay + 16) || e.reserve(e.user[UB_PAY2], max_pay + 16) || e.reserve(e.user[UB_IMG], img_bytes) ||
-	    e.reserve(e.user[UB_IMG2], img_bytes) || (k != 0 && e.reserve(e.user[UB_SYM], img_bytes))) return LFM_ERR_CUDA;
+	if (e.reserve(e.user[UB_PAY], max_pay + 16) || e.reserve(e.user[UB_PAY2], max_pay + 16) ||
+	    (!out_on_device && (e.reserve(e.user[UB_IMG], img_bytes) || e.reserve(e.user[UB_IMG2], img_bytes))) ||
+	    (k != 0 && e.reserve(e.user[UB_SYM], img_bytes))) return LFM_ERR_CUDA;
 	if (!e.pinned(kStageBufs * kStageChunk, 0) || !e.pinned(kStageBufs * kStageChunk, 1)) return LFM_ERR_CUDA;
 	uint8_t* dpay[2] = { (uint8_t*)e.user[UB_PAY].p, (uint8_t*)e.user[UB_PAY2].p };
 	uint16_t* dimg[2] = { (uint16_t*)e.user[UB_IMG].p, (uint16_t*)e.user[UB_IMG2].p };
@@ -693,7 +725,7 @@ static int decompress_pipelined(const klb_image_header& h, const Layout& L, cons
 			ids[i] = id0 + i;
 			beg[i] = ((id0 + i) ? h.blockOffset[id0 + i - 1] : 0) - bt.beg; end[i] = h.blockOffset[id0 + i] - bt.beg;
 		}
-		uint16_t* res = dimg[slot] - bt.f0 * L.fpx;                     // virtual base: absolute frame indexing
+		uint16_t* res = out_on_device ? out : dimg[slot] - bt.f0 * L.fpx;   // virtual base: absolute frame indexing
 		uint16_t* sym_base = k != 0 ? dsym - bt.f0 * L.fpx : res;
 		DecompressStats st;
 		rc = e.decompress_blocks(dpay[slot], beg.data(), end.data(), ids.data(), cnt, sym_base, desc, &st);
@@ -707,6 +739,7 @@ static int decompress_pipelined(const klb_image_header& h, const Layout& L, cons
 		}
 		g_stats.ms_decode += st.ms_decode; g_stats.ms_imtf += st.ms_imtf; g_stats.ms_ibwt += st.ms_ibwt; g_stats.ms_unrle += st.ms_unrle;
 		g_stats.gpu_launches += st.launches;
+		if (out_on_device) continue;                                   // the pixels are in place and the engine stream is synchronised
 		const uint16_t* srcp = dimg[slot]; uint16_t* dstp = out + bt.f0 * L.fpx; const size_t nbytes = (size_t)bt.nf * L.fpx * 2;
 		// one download at a time (they share the pinned ring and copy stream 1): batch b - 1 had all of this batch's kernels to finish
 		if (dn_th[slot ^ 1].joinable()) { dn_th[slot ^ 1].join(); if ((rc = dn_rc[slot ^ 1])) break; }
@@ -722,7 +755,10 @@ static int decompress_pipelined(const klb_image_header& h, const Layout& L, cons
 	return rc;
 }
 
-int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16_t* out, const klb_ROI* roi)
+// Pixels go to the host buffer `out`, or with a DeviceSink to its device buffer (then `out` is ignored): full reads into a
+// 16-byte aligned buffer decode straight into it; ROI reads, and full reads into any other buffer, decode into the engine's
+// frame buffers and k_roi_gather copies the box out.
+int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16_t* out, const klb_ROI* roi, const DeviceSink* dsink = nullptr)
 {
 	const uint64_t payload_size = psrc.size;
 	memset(&g_stats, 0, sizeof(g_stats));
@@ -757,6 +793,15 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 		if (ub[d] >= h.xyzct[d] || lb[d] > ub[d]) return LFM_ERR_OPEN;
 		if (lb[d] != 0 || ub[d] != h.xyzct[d] - 1) full = false;
 	}
+	if (dsink) {
+		// the caller's buffer is checked before any kernel runs: nothing is written to it unless the whole box fits
+		uint64_t bytes = 2;
+		for (int d = 0; d < 5; d++) bytes *= (uint64_t)(ub[d] - lb[d] + 1);
+		if (dsink->out_bytes) *dsink->out_bytes = bytes;
+		if ((rc = check_device_ptr(dsink->d_out, "d_out"))) return rc;
+		if (dsink->capacity < bytes) { g_err = "d_out is smaller than the box (" + std::to_string(bytes) + " bytes)"; return LFM_ERR_CREATE; }
+		out = (uint16_t*)dsink->d_out;
+	}
 	// slabs intersecting the ROI along z, c, t
 	std::vector<uint64_t> slabs;
 	for (uint64_t s = 0; s < L.nSlabs; s++) {
@@ -771,13 +816,19 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 	}
 	const bool contiguous = !slabs.empty() && (slabs.back() - slabs.front() + 1 == slabs.size());
 	// Full reads are sharded over the GPUs by slab ranges whose frame ranges are disjoint: with c or t blocked (blockSize[3] or
-	// blockSize[4] > 1) the frames of neighbouring slabs interleave, and one GPU decodes the stack.
+	// blockSize[4] > 1) the frames of neighbouring slabs interleave, and one GPU decodes the stack.  A device buffer is on the
+	// first device, which decodes everything.
 	const bool disjoint = h.blockSize[3] == 1 && h.blockSize[4] == 1;
-	const int D = (full && contiguous && disjoint && slabs.size() == L.nSlabs) ? (int)std::min<uint64_t>((uint64_t)ndev, slabs.size()) : 1;
-	if (full && D == 1 && desc.codec == 1) {
+	const int D = (!dsink && full && contiguous && disjoint && slabs.size() == L.nSlabs) ? (int)std::min<uint64_t>((uint64_t)ndev, slabs.size()) : 1;
+	// The decode and inverse-predictor kernels take 16-byte vector paths from the frame width alone, assuming a frame buffer
+	// aligned as the engine's are: a caller's buffer that is not 16-byte aligned only receives k_roi_gather's copy of the box
+	// (the whole stack for a full read), which handles any alignment.
+	const bool sink_aligned = dsink && ((uintptr_t)dsink->d_out & 15) == 0;
+	if (full && D == 1 && desc.codec == 1 && (!dsink || sink_aligned)) {
 		const uint64_t per = slabs_per_batch(h, L, k != 0 && video);
-		if (per) return decompress_pipelined(h, L, desc, k, video, psrc, out, per);
+		if (per) return decompress_pipelined(h, L, desc, k, video, psrc, out, dsink != nullptr, per);
 	}
+	const bool direct = dsink && full && sink_aligned;   // decode into the caller's device buffer, no copy at the end
 	const std::vector<uint64_t> cut = shard_cuts(h, L, D, k != 0 && video);
 
 	std::vector<int> rcs(D, 0);
@@ -822,24 +873,29 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 		Engine& e = Engine::for_device(g_set.first_device + d);
 		cudaSetDevice(e.device());
 		cudaStream_t st = (cudaStream_t)e.stream();
-		if (e.reserve(e.user[UB_PAY], need_bytes + 16) || e.reserve(e.user[UB_SYM], nf * L.fpx * 2) || (k != 0 && e.reserve(e.user[UB_IMG], nf * L.fpx * 2))) { rcs[d] = LFM_ERR_CUDA; return; }
+		if (e.reserve(e.user[UB_PAY], need_bytes + 16) || (!(direct && k == 0) && e.reserve(e.user[UB_SYM], nf * L.fpx * 2)) ||
+		    (k != 0 && !direct && e.reserve(e.user[UB_IMG], nf * L.fpx * 2))) { rcs[d] = LFM_ERR_CUDA; return; }
 		struct { void* p; } dpay{ e.user[UB_PAY].p }, dsym{ e.user[UB_SYM].p }, dimg{ e.user[UB_IMG].p };
 		double t0 = now_ms();
 		if ((rcs[d] = psrc.to_device(e, dpay.p, ranges, st))) { if (rcs[d] == LFM_ERR_BZIP) std::cerr << "ERROR: lfm_b200: file is truncated" << std::endl; return; }
 		if (!full) cudaMemsetAsync(dsym.p, 0, nf * L.fpx * 2, st);
 		h2d[d] = now_ms() - t0;
-		uint16_t* sym_base = (uint16_t*)dsym.p - f0 * L.fpx;
+		// a direct read covers the whole stack (f0 == 0): the caller's buffer is the frame buffer
+		uint16_t* sym_base = (direct && k == 0) ? out : (uint16_t*)dsym.p - f0 * L.fpx;
 		rcs[d] = e.decompress_blocks((const uint8_t*)dpay.p, beg.data(), end.data(), ids.data(), ids.size(), sym_base, desc, &sts[d]);
 		if (rcs[d]) { errs[d] = e.last_error(); return; }
 		const uint16_t* res_base = sym_base;
 		if (k != 0) {
-			rcs[d] = e.unpredict(sym_base, (uint16_t*)dimg.p - f0 * L.fpx, desc, k, video, (uint32_t)f0, (uint32_t)nf);
+			uint16_t* res = direct ? out : (uint16_t*)dimg.p - f0 * L.fpx;
+			rcs[d] = e.unpredict(sym_base, res, desc, k, video, (uint32_t)f0, (uint32_t)nf);
 			sts[d].launches += video ? 2 : 1;
 			if (rcs[d]) return;
-			res_base = (const uint16_t*)dimg.p - f0 * L.fpx;
+			res_base = res;
 		}
 		t0 = now_ms();
-		if (full) {
+		if (dsink) {
+			if (!direct) { rcs[d] = e.roi_gather(res_base, desc, lb, ub, out); sts[d].launches++; if (rcs[d]) { errs[d] = e.last_error(); return; } }
+		} else if (full) {
 			// this shard's frames, contiguous in the output
 			uint64_t a, b; slab_frames(h, L, my.front(), my.back() + 1, a, b);
 			d2h_staged(e, out + a * L.fpx, res_base + a * L.fpx, (b - a + 1) * L.fpx * 2, st);
@@ -855,7 +911,7 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 			}
 		}
 		cudaStreamSynchronize(st);
-		d2h[d] = now_ms() - t0;
+		d2h[d] = dsink ? 0 : now_ms() - t0;
 		if (k != 0) sts[d].ms_unpredict = e.last_unpredict_ms();
 		if (cudaGetLastError() != cudaSuccess) rcs[d] = LFM_ERR_CUDA;
 	};
@@ -1024,7 +1080,8 @@ try {
 } LFM_CATCH
 
 // header (+ blockOffset table) of the file, then decode straight from the open file: only the needed byte ranges are read
-static int read_from_file(const std::string& filename, klb_image_header& header, uint16_t* out, const klb_ROI* roi)
+static int read_from_file(const std::string& filename, klb_image_header& header, uint16_t* out, const klb_ROI* roi,
+                          const DeviceSink* dsink = nullptr)
 try {
 	LFM_API_LOCK();
 	if (filename.empty()) { std::cerr << "ERROR: Filename has not been defined. We cannot read image" << std::endl; return LFM_ERR_OPEN; }
@@ -1038,7 +1095,7 @@ try {
 	struct stat sb;
 	PayloadSource ps; ps.fd = fd; ps.file_off = header.getSizeInBytes();
 	ps.size = (fstat(fd, &sb) == 0 && (uint64_t)sb.st_size > ps.file_off) ? (uint64_t)sb.st_size - ps.file_off : 0;
-	const int rc = decompress_core(header, ps, out, roi);
+	const int rc = decompress_core(header, ps, out, roi, dsink);
 	close(fd);
 	return rc;
 } LFM_CATCH
@@ -1069,6 +1126,31 @@ try {
 	klb_imageIO io{ std::string(filename) };
 	io.header.setHeader(xyzct, dataType, pixelSize, blockSize, compressionType, metadata, headerVersion, Nnum);
 	return io.writeImage((const char*)im, numThreads);
+} LFM_CATCH
+
+int writeLFMstackDevice(const void* d_im, const char* filename, const uint32_t xyzct[5], enum KLB_DATA_TYPE dataType, int /*numThreads*/,
+                        const float32_t pixelSize[5], const uint32_t blockSize[5], enum KLB_COMPRESSION_TYPE compressionType,
+                        const char metadata[256], uint8_t headerVersion, uint8_t Nnum)
+try {
+	g_err.clear();
+	if (!filename || !*filename) return LFM_ERR_OPEN;
+	klb_image_header h;
+	h.setHeader(xyzct, dataType, pixelSize, blockSize, compressionType, metadata, headerVersion, Nnum);
+	FrameSource src; src.base = (const uint16_t*)d_im; src.device = true;
+	return write_stack_to_file(std::string(filename), src, h);
+} LFM_CATCH
+
+int readLFMroiDevice(const char* filename, const uint32_t lb[5], const uint32_t ub[5], void* d_out, uint64_t capacity, uint64_t* out_bytes)
+try {
+	g_err.clear();
+	if (out_bytes) *out_bytes = 0;
+	if (!filename || !*filename || (lb == nullptr) != (ub == nullptr)) return LFM_ERR_OPEN;
+	if (access(filename, R_OK) != 0) { g_err = std::string("cannot open ") + filename; return LFM_ERR_OPEN; }
+	klb_image_header h;
+	klb_ROI roi;
+	if (lb) for (int d = 0; d < 5; d++) { roi.xyzctLB[d] = lb[d]; roi.xyzctUB[d] = ub[d]; }
+	DeviceSink sink; sink.d_out = d_out; sink.capacity = capacity; sink.out_bytes = out_bytes;
+	return read_from_file(std::string(filename), h, nullptr, lb ? &roi : nullptr, &sink);
 } LFM_CATCH
 
 int readLFMheaderEx(const char* filename, uint8_t* headerVersion, uint8_t* Nnum)
