@@ -347,18 +347,19 @@ int Engine::unpredict(const uint16_t* d_sym, uint16_t* d_out, const StackDesc& s
 	static const bool poison = getenv("LFM_B200_DEBUG_POISON") != nullptr;
 	if (poison) cudaMemsetAsync(d_out + (size_t)z0 * W * H, 0xAB, (size_t)nz * W * H * 2, st);
 	int bad = 0;
+	const char* failed = "?";
 	cudaEventRecord((cudaEvent_t)ev_[2], st);
-	if (!video) bad |= launch_unpredict(d_sym, d_out, W, H, s.Nnum, s.way, predictor, 0, z0, 1, nz, sm_count_, st);
+	if (!video) bad |= launch_unpredict(d_sym, d_out, W, H, s.Nnum, s.way, predictor, 0, z0, 1, nz, sm_count_, st, &failed);
 	else {
 		// odd frames need the decoded even frame before them: evens first, then odds (z0 must be even)
 		uint32_t first_even = z0 + (z0 & 1), first_odd = z0 + 1 - (z0 & 1);
 		uint32_t n_even = first_even < z0 + nz ? (z0 + nz - first_even + 1) / 2 : 0;
 		uint32_t n_odd = first_odd < z0 + nz ? (z0 + nz - first_odd + 1) / 2 : 0;
-		bad |= launch_unpredict(d_sym, d_out, W, H, s.Nnum, s.way, predictor, 1, first_even, 2, n_even, sm_count_, st);
-		bad |= launch_unpredict(d_sym, d_out, W, H, s.Nnum, s.way, predictor, 1, first_odd, 2, n_odd, sm_count_, st);
+		bad |= launch_unpredict(d_sym, d_out, W, H, s.Nnum, s.way, predictor, 1, first_even, 2, n_even, sm_count_, st, &failed);
+		if (!bad) bad |= launch_unpredict(d_sym, d_out, W, H, s.Nnum, s.way, predictor, 1, first_odd, 2, n_odd, sm_count_, st, &failed);
 	}
 	cudaEventRecord((cudaEvent_t)ev_[3], st);
-	if (bad) { cudaGetLastError(); err_ = "cluster launch of k_unpredict failed"; return LFM_ERR_CUDA; }
+	if (bad) { cudaGetLastError(); err_ = std::string("inverse predictor: launch of ") + failed + " failed"; return LFM_ERR_CUDA; }
 	return check("unpredict");
 }
 

@@ -8,7 +8,7 @@ namespace lfm {
 void launch_predict_fwd(const uint16_t* img, uint16_t* sym, int W, int H, int T, int way, int k, int video,
                         uint32_t z0, uint32_t nz, cudaStream_t st);
 int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, int way, int k, int video,
-                     uint32_t z_start, uint32_t z_step, uint32_t count, int sm_count, cudaStream_t st);
+                     uint32_t z_start, uint32_t z_step, uint32_t count, int sm_count, cudaStream_t st, const char** failed);
 // lfm_roi.cu: the box lb..ub (inclusive x,y,z,c,t) of frames (absolute frame indexing) -> dense [t][c][z][y][x] at out, one launch
 void launch_roi_gather(const uint16_t* frames, const uint32_t xyzct[5], const uint32_t lb[5], const uint32_t ub[5], uint16_t* out,
                        int sm_count, cudaStream_t st);

@@ -1218,7 +1218,9 @@ k_unscan_rows(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H, int
 	if (nrows <= 0) return;
 	const uint16_t* src = (SRC_OUT ? (const uint16_t*)out : sym) + fbase;
 	const uint16_t* o = out + fbase;
-	if ((W & 7) == 0) {                                                 // rows are whole 16-byte vectors
+	// rows are whole 16-byte vectors of 16-byte aligned buffers (a view into a caller's tensor need not be)
+	const bool vec = ((W & 7) == 0) && ((((uintptr_t)sym | (uintptr_t)out) & 15) == 0);
+	if (vec) {
 		const int vpr = W >> 3;
 		for (int i = tid; i < nrows * vpr; i += SC_ROWS_NT) {
 			const int r = i / vpr, xv = i - r * vpr;
@@ -1256,7 +1258,7 @@ k_unscan_rows(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H, int
 	}
 	__syncthreads();
 	uint16_t* dst = out + fbase;
-	if ((W & 7) == 0) {
+	if (vec) {
 		const int vpr = W >> 3;
 		for (int i = tid; i < nrows * vpr; i += SC_ROWS_NT) {
 			const int r = i / vpr, xv = i - r * vpr;
@@ -1584,10 +1586,16 @@ void launch_predict_fwd(const uint16_t* img, uint16_t* sym, int W, int H, int T,
 	else launch_predict_fwd_way<2>(img, sym, W, H, T, k, video, z0, nz, st);
 }
 
+static int failed_launch(const char* kernel, const char** failed)
+{
+	if (failed) *failed = kernel;
+	return 1;
+}
+
 // frames z_start, z_start+z_step, ... (count of them); video stacks: even frames first, then odd frames.
-// Returns 0, or 1 if the cluster launch fails.
+// Returns 0, or 1 if a launch fails; *failed then names the kernel(s) of the branch that failed.
 int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, int way, int k, int video,
-                     uint32_t z_start, uint32_t z_step, uint32_t count, int sm_count, cudaStream_t st)
+                     uint32_t z_start, uint32_t z_step, uint32_t count, int sm_count, cudaStream_t st, const char** failed)
 {
 	(void)sm_count;
 	if (count == 0) return 0;
@@ -1595,7 +1603,7 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 	if (bands_all >= 2 && !video && ((way == 1 && k != 2) || way == 2)) {      // measurement switch: every way through the band pipeline
 		const int rcb = way == 1 ? launch_unpredict_bands<1>(sym, out, W, H, T, k, 0, z_start, z_step, count, st)
 		                         : launch_unpredict_bands<2>(sym, out, W, H, T, k, 0, z_start, z_step, count, st);
-		if (rcb != 2) return rcb;
+		if (rcb != 2) return rcb ? failed_launch("k_unpredict_bands", failed) : 0;
 	}
 	const int tilesX = (W + T - 1) / T, tilesY = (H + T - 1) / T;
 	const unsigned wpb = UF_NT / 32;
@@ -1608,14 +1616,14 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 	static const int scans_on = getenv("LFM_B200_SCANS") ? atoi(getenv("LFM_B200_SCANS")) : 1;
 	if (!video && way == 2 && scans_on) {                    // linear rules: strided prefix sums
 		const int rcs = launch_unpredict_space_scans(sym, out, W, H, T, k, z_start, z_step, count, st);
-		if (rcs != 2) return rcs;
+		if (rcs != 2) return rcs ? failed_launch("k_unscan_rows / k_unscan_cols", failed) : 0;
 	}
 	if (!video && way == 2 && grid_ok) {                    // tile (0,0), then T*T sub-aperture recurrences per frame
 		k_unpredict_seed<<<(count + wpb - 1) / wpb, UF_NT, 0, st>>>(sym, out, W, H, T, way, k, z_start, z_step, count, 0);
 		const size_t smem = (size_t)G * plane_b + 16;
 		const int ugroups = (T + G - 1) / G;
 		launch_unpredict_grid<2>(sym, out, W, H, T, k, z_start, z_step, (unsigned)((uint64_t)count * T * ugroups), (unsigned)(G * nxr), smem, G, ugroups, T, nxr, st);
-		return cudaGetLastError() == cudaSuccess ? 0 : 1;
+		return cudaGetLastError() == cudaSuccess ? 0 : failed_launch("k_unpredict_seed / k_unpredict_grid", failed);
 	}
 	const size_t strip_smem = (size_t)T * T * UT_NT * 2 + 16;
 	if (!video && way == 1 && k != 2 && grid_ok && strip_smem <= (size_t)UG_MAX_SMEM) {   // DC grid, then every tile on its own
@@ -1629,19 +1637,19 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 		case 6: launch_tiles_angle<6>(sym, out, W, H, T, z_start, z_step, count, tilesX, tilesY, chunks, strip_smem, st); break;
 		default: launch_tiles_angle<7>(sym, out, W, H, T, z_start, z_step, count, tilesX, tilesY, chunks, strip_smem, st); break;
 		}
-		return cudaGetLastError() == cudaSuccess ? 0 : 1;
+		return cudaGetLastError() == cudaSuccess ? 0 : failed_launch("k_unpredict_grid / k_unpredict_tiles_angle", failed);
 	}
 	if (!video && way == 2) {                               // (fallback for tile grids that do not fit shared memory)
 		k_unpredict_seed<<<(count + wpb - 1) / wpb, UF_NT, 0, st>>>(sym, out, W, H, T, way, k, z_start, z_step, count, 0);
 		const uint64_t warps = (uint64_t)count * T * T;
 		k_unpredict_space<<<(unsigned)((warps + wpb - 1) / wpb), UF_NT, 0, st>>>(sym, out, W, H, T, k, z_start, z_step, count);
-		return cudaGetLastError() == cudaSuccess ? 0 : 1;
+		return cudaGetLastError() == cudaSuccess ? 0 : failed_launch("k_unpredict_seed / k_unpredict_space", failed);
 	}
 	if (!video && way == 1 && k != 2) {
 		k_unpredict_seed<<<(count + wpb - 1) / wpb, UF_NT, 0, st>>>(sym, out, W, H, T, way, k, z_start, z_step, count, 1);
 		const uint64_t warps = (uint64_t)count * tilesX * tilesY;
 		k_unpredict_angle<<<(unsigned)((warps + wpb - 1) / wpb), UF_NT, 0, st>>>(sym, out, W, H, T, k, z_start, z_step, count);
-		return cudaGetLastError() == cudaSuccess ? 0 : 1;
+		return cudaGetLastError() == cudaSuccess ? 0 : failed_launch("k_unpredict_seed / k_unpredict_angle", failed);
 	}
 	// way tiles (image stacks and video), every predictor but 2: the band pipeline
 	static const int bands_on = getenv("LFM_B200_BANDS") ? atoi(getenv("LFM_B200_BANDS")) : 1;
@@ -1650,7 +1658,7 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 	static const int bands_min = getenv("LFM_B200_BANDS_MIN") ? atoi(getenv("LFM_B200_BANDS_MIN")) : 3;
 	if (bands_on && way == 0 && k != 2 && (int)count >= bands_min) {
 		const int rcb = launch_unpredict_bands<0>(sym, out, W, H, T, k, (video && (z_start & 1u)) ? 1 : 0, z_start, z_step, count, st);
-		if (rcb != 2) return rcb;
+		if (rcb != 2) return rcb ? failed_launch("k_unpredict_bands", failed) : 0;
 	}
 	// remaining cases (way tiles, video, predictor 2 of tiles/angle): many frames -> one CTA per frame in shared memory;
 	// few frames -> the cluster wavefront below (all SMs on one frame)
@@ -1662,7 +1670,7 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 		const int rcs = way == 0 ? launch_unpredict_strips<0>(sym, out, W, H, T, k, video, z_start, z_step, count, st)
 		              : way == 1 ? launch_unpredict_strips<1>(sym, out, W, H, T, k, video, z_start, z_step, count, st)
 		                         : launch_unpredict_strips<2>(sym, out, W, H, T, k, video, z_start, z_step, count, st);
-		if (rcs != 2) return rcs;
+		if (rcs != 2) return rcs ? failed_launch("k_unpredict_strips", failed) : 0;
 	}
 	const uint64_t steps = (k == 2 && way != 2) ? (uint64_t)H : (uint64_t)(tilesX + tilesY + 2 * T);
 	const uint64_t per_step = ((uint64_t)W * H + steps - 1) / steps;              // mean ready pixels per step and frame
@@ -1676,20 +1684,24 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 	cfg.attrs = attr; cfg.numAttrs = 1;
 	if (cols) {
 		const size_t smem0 = (size_t)W * 2 * 2;
-		const dim3 grid((unsigned)((W + UC_NT - 1) / UC_NT), count);
 		const size_t smem = (size_t)T * UC_NT * 2;
 		if (way == 0) {
 			cudaFuncSetAttribute(k_unpredict_row0<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem0);
 			k_unpredict_row0<0><<<count, 32, smem0, st>>>(sym, out, W, H, T, video, z_start, z_step);
-			k_unpredict_cols2<0><<<grid, UC_NT, smem, st>>>(sym, out, W, H, T, video, z_start, z_step);
 		} else {
 			cudaFuncSetAttribute(k_unpredict_row0<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem0);
 			k_unpredict_row0<1><<<count, 32, smem0, st>>>(sym, out, W, H, T, video, z_start, z_step);
-			k_unpredict_cols2<1><<<grid, UC_NT, smem, st>>>(sym, out, W, H, T, video, z_start, z_step);
 		}
-		return cudaGetLastError() == cudaSuccess ? 0 : 1;
+		if (cudaGetLastError() != cudaSuccess) return failed_launch("k_unpredict_row0", failed);
+		for (uint32_t f0 = 0; f0 < count; f0 += 65535u) {          // frames in gridDim.y: at most 65535 per launch
+			const dim3 grid((unsigned)((W + UC_NT - 1) / UC_NT), std::min(65535u, count - f0));
+			if (way == 0) k_unpredict_cols2<0><<<grid, UC_NT, smem, st>>>(sym, out, W, H, T, video, z_start + f0 * z_step, z_step);
+			else k_unpredict_cols2<1><<<grid, UC_NT, smem, st>>>(sym, out, W, H, T, video, z_start + f0 * z_step, z_step);
+		}
+		return cudaGetLastError() == cudaSuccess ? 0 : failed_launch("k_unpredict_cols2", failed);
 	}
-	return cudaLaunchKernelEx(&cfg, k_unpredict, sym, out, W, H, T, way, k, video, z_start, z_step, count, H) == cudaSuccess ? 0 : 1;
+	return cudaLaunchKernelEx(&cfg, k_unpredict, sym, out, W, H, T, way, k, video, z_start, z_step, count, H) == cudaSuccess ? 0
+	       : failed_launch("k_unpredict (cluster)", failed);
 }
 
 }  // namespace lfm

@@ -17,7 +17,6 @@ G = json.load(open(os.path.join(GOLDEN, "golden.json")))
 @pytest.fixture(scope="module")
 def L():
     os.environ["LFM_B200_DEBUG_POISON"] = "1"      # poison decode buffers so ordering bugs cannot hide behind stale data
-    os.environ["LFM_B200_STRIPS_MIN"] = "8"        # fall-back inverse kernels (Nnum > 32, predictor 2 with Nnum > 32): strips from 8 frames on, cluster below
     import lfm_b200
     import torch
     assert torch.cuda.is_available(), "gpu tests need a CUDA device"
@@ -382,9 +381,10 @@ def test_pageable_stacks_take_the_staged_copy_path(L, tmp_path):
 
 @pytest.mark.parametrize("frames", [3, 9])
 def test_inverse_fallback_kernels_large_nnum(L, oracle, frames):
-    """Nnum = 33: a tile no longer fits the band pipeline (Nnum^2 threads) nor the column kernel's shuffle chain (Nnum <= 32), so
-    the way tiles / angle inverses fall back to the strips kernel (>= 8 frames here) and the cluster wavefront / row schedule.
-    Every predictor, image and video mode: forward symbols of frame 0 equal the oracle's, inverse(forward) restores the stack."""
+    """Nnum = 33: a tile no longer fits the band pipeline (Nnum^2 threads) nor the column kernel's shuffle chain (Nnum <= 32), and
+    the strips kernel's shared memory only holds Nnum <= 22, so the way tiles / angle inverses fall back to the cluster wavefront
+    (predictor 2 of those ways: its row schedule).  Every predictor, image and video mode: forward symbols of frame 0 equal the
+    oracle's, inverse(forward) restores the stack.  (tests/test_predict_dispatch.py pins the strips kernel.)"""
     import ctypes as C
     import torch
     T, H, W = 33, 100, 136
