@@ -159,7 +159,10 @@ k_huff_decode(const uint8_t* __restrict__ payload, const uint64_t* __restrict__ 
 	const int alpha = (int)n_in_use + 2;
 	const int n_groups = (int)get(3);
 	const int n_sel = (int)get(15);
-	if (n_groups < 2 || n_groups > 6 || n_sel < 1 || (uint32_t)n_sel > selcap) FAIL(2);
+	if (n_groups < 2 || n_groups > 6 || n_sel < 1) FAIL(2);
+	// all n_sel (<= 32767) selectors are read, as libbz2 1.0.8 does; only the first selcap are kept (more than any block of this
+	// slot geometry can use: other encoders may round the count up), and a group past them is corrupt (decompress.c:287-300)
+	const int n_sel_kept = min(n_sel, (int)selcap);
 	{
 		uint32_t pos = 0x543210u;                          // 6 nibbles: move-to-front list of table ids
 		for (int i = 0; i < n_sel; i++) {
@@ -171,7 +174,7 @@ k_huff_decode(const uint8_t* __restrict__ payload, const uint64_t* __restrict__ 
 			uint32_t t = (pos >> (4 * j)) & 15u;
 			uint32_t lowmask = (1u << (4 * j)) - 1u;
 			pos = (pos & ~((lowmask << 4) | 15u)) | ((pos & lowmask) << 4) | t;
-			if (lane == 0) selector[i >> 1] = (i & 1) ? (uint8_t)((selector[i >> 1] & 15u) | (t << 4)) : (uint8_t)t;
+			if (lane == 0 && i < n_sel_kept) selector[i >> 1] = (i & 1) ? (uint8_t)((selector[i >> 1] & 15u) | (t << 4)) : (uint8_t)t;
 		}
 	}
 	// code lengths (decompress.c:314-331): per symbol a run of (1, d) bit pairs -- d = 0: +1, d = 1: -1 -- closed by a 0 bit.  The
@@ -276,7 +279,7 @@ k_huff_decode(const uint8_t* __restrict__ payload, const uint64_t* __restrict__ 
 		nxt = sw[wi & (DEC_RING - 1)];
 	};
 	for (int grp = 0; !done; grp++) {
-		if (grp >= n_sel) FAIL(2);
+		if (grp >= n_sel_kept) FAIL(2);
 		const int t = (selector[grp >> 1] >> ((grp & 1) * 4)) & 15;
 		if (t >= n_groups) FAIL(2);
 		const uint16_t* lut = S.lut[t];
@@ -595,11 +598,10 @@ size_t imtf_smem_bytes() { return (size_t)64 * IM_STS * 4 + 64 * 4 + (IM_NT + 4)
 //      position (+ the start): ~n/32 sublists.  Every thread measures four sublists at a time (four independent pointer
 //      chases in flight), the sublists are ranked by pointer jumping in shared memory (ceil(log2) rounds), and then
 //      written, again four at a time per thread.
-//   A block whose rotations are not all distinct (exactly periodic text) walks a shorter cycle several times; the
-//   ranking then does not cover the block and the sublists are chained sequentially from the start instead.
+//   A block whose rotations are not all distinct (exactly periodic text, u repeated r times) walks a cycle of c = n / r
+//   steps r times.  The path from the start is then one lap: it is written as above, and the rest of the text repeats it.
 // =====================================================================================================
 constexpr int IB_MAXS = 6144;     // max number of regular splitters
-constexpr int IB_VIS  = 2 * (IB_MAXS + 2);   // max sublist visits (a periodic block laps its cycle)
 constexpr int IB_ILP  = 4;        // sublists walked concurrently by one thread
 constexpr uint32_t IB_NIL = 0xFFFFu;
 
@@ -616,12 +618,10 @@ k_inv_bwt(const uint8_t* __restrict__ bwt_all, uint32_t cap, DecJob* __restrict_
 	__shared__ uint32_t wcnt[(NT / 32) * BWT_WS];
 	__shared__ uint32_t run[256];
 	__shared__ uint32_t red[64];
-	__shared__ uint32_t s_nvis;
 	uint32_t* s_dist = reinterpret_cast<uint32_t*>(ib_smem);                         // [2][maxs + 2]
 	uint16_t* s_nxt = reinterpret_cast<uint16_t*>(s_dist + 2 * (maxs + 2));         // [2][maxs + 2]
 	const uint32_t tid = threadIdx.x;
 	uint32_t* tt = tt_all + (size_t)blockIdx.x * cap;          // per-CTA scratch
-	uint32_t* vis = tt_all + (size_t)gridDim.x * cap + (size_t)blockIdx.x * 2 * IB_VIS;   // visit list (id, offset)
 
 	for (uint32_t job = blockIdx.x; job < njobs; job += gridDim.x) {
 		DecJob& J = jobs[job];
@@ -648,7 +648,7 @@ k_inv_bwt(const uint8_t* __restrict__ bwt_all, uint32_t cap, DecJob* __restrict_
 		const bool p0_regular = (p0 & (K - 1)) == 0;
 		const uint32_t nspl = S + (p0_regular ? 0 : 1);
 		const uint32_t start_id = p0_regular ? (p0 >> kshift) : S;
-		auto measure = [&](uint32_t* dist, uint16_t* nxt, bool cut) {
+		{   // ---- measure: length of every sublist and the sublist it runs into
 			for (uint32_t q0 = tid; q0 < nspl; q0 += BWT_NT * IB_ILP) {
 				uint32_t p[IB_ILP], len[IB_ILP]; bool act[IB_ILP];
 				#pragma unroll
@@ -669,13 +669,12 @@ k_inv_bwt(const uint8_t* __restrict__ bwt_all, uint32_t cap, DecJob* __restrict_
 					const uint32_t q = q0 + j * BWT_NT;
 					if (q < nspl) {
 						uint32_t id = (p[j] == p0) ? start_id : (p[j] >> kshift);
-						if (cut && id == start_id) id = IB_NIL;                 // open the cycle at the start: a path
-						dist[q] = len[j]; nxt[q] = (uint16_t)id;
+						if (id == start_id) id = IB_NIL;                         // open the cycle at the start: a path
+						s_dist[q] = len[j]; s_nxt[q] = (uint16_t)id;
 					}
 				}
 			}
-		};
-		measure(s_dist, s_nxt, true);
+		}
 		__syncthreads();
 		// ---- rank the sublists: distance to the end of the path by pointer jumping (double buffered)
 		uint32_t cur = 0;
@@ -693,10 +692,14 @@ k_inv_bwt(const uint8_t* __restrict__ bwt_all, uint32_t cap, DecJob* __restrict_
 		}
 		const uint32_t* dfin = s_dist + cur * (maxs + 2);
 		const uint16_t* nfin = s_nxt + cur * (maxs + 2);
-		const bool ranked = (dfin[start_id] == n) && (nfin[start_id] == IB_NIL);     // the path from the start covers the block
+		// the path from the start is one lap of the walk's cycle: c = n steps, or n / r for a text that is some u repeated r times;
+		// the sublists off the path lie on other cycles and never reach the end of the path
+		const uint32_t c = dfin[start_id];
+		const bool lap = nfin[start_id] == IB_NIL && c >= 1 && c <= n;              // always (tt is a permutation)
 		__syncthreads();
-		if (ranked) {
-			// ---- write: sublist q starts at output offset n - dist_to_end(q)
+		if (!lap) { if (tid == 0) J.status = 2; continue; }                         // uniform
+		{
+			// ---- write the lap: sublist q on the path starts at output offset c - dist_to_end(q)
 			for (uint32_t q0 = tid; q0 < nspl; q0 += BWT_NT * IB_ILP) {
 				// 147 KB blocks: the bytes of a sublist leave as aligned 32-bit words (byte stores only for the ragged first and last word: a
 				// word shared with the neighbouring sublist): a quarter of the store instructions (16-frame slice: 5.43 -> 4.99 ms)
@@ -705,7 +708,7 @@ k_inv_bwt(const uint8_t* __restrict__ bwt_all, uint32_t cap, DecJob* __restrict_
 				for (int j = 0; j < IB_ILP; j++) {
 					const uint32_t q = q0 + j * BWT_NT;
 					p[j] = q < S ? (q << kshift) : p0; off[j] = 0; end[j] = 0; acc[j] = 0;
-					if (q < nspl) { off[j] = n - dfin[q]; end[j] = n; }     // end: upper bound, the walk stops at the next splitter
+					if (q < nspl && nfin[q] == IB_NIL) { off[j] = c - dfin[q]; end[j] = c; }     // end: upper bound, the walk stops at the next splitter
 					beg[j] = off[j];
 				}
 				bool any = true;
@@ -730,25 +733,11 @@ k_inv_bwt(const uint8_t* __restrict__ bwt_all, uint32_t cap, DecJob* __restrict_
 					}
 				}
 			}
-		} else {
-			// ---- exactly periodic block: chain the sublists from the start for exactly n steps (laps its cycle)
-			uint32_t* s_len = s_dist; uint16_t* s_next = s_nxt;
-			measure(s_len, s_next, false);
-			__syncthreads();
-			if (tid == 0) {
-				uint32_t q = start_id, off = 0, nv = 0;
-				while (off < n && nv < (uint32_t)IB_VIS) { vis[2 * nv] = q; vis[2 * nv + 1] = off; nv++; off += s_len[q]; q = s_next[q]; }
-				if (off < n) J.status = 2;
-				s_nvis = nv;
-			}
-			__syncthreads();
-			const uint32_t nvis = s_nvis;
-			for (uint32_t i = tid; i < nvis; i += BWT_NT) {
-				uint32_t q = vis[2 * i], off = vis[2 * i + 1];
-				uint32_t p = q < S ? (q << kshift) : p0, len = s_len[q];
-				for (uint32_t k = 0; k < len && off + k < n; k++) { uint32_t e = tt[p]; txt[off + k] = (uint8_t)e; p = e >> 8; }
-			}
 		}
+		__syncthreads();
+		// ---- exactly periodic block: bzip2's n-step walk laps the cycle, so the rest of the text repeats the first lap (when c does
+		// not divide n, which only corrupt data gives, this is still what the walk gives; the block CRC decides)
+		for (uint32_t k = c + tid; k < n; k += BWT_NT) txt[k] = txt[k % c];
 		__syncthreads();
 		// de-randomisation (decompress.c BZ_RAND_INIT_MASK / BZ_RAND_UPD_MASK / BZ_RAND_MASK, bzlib.c:577-640): byte j of the block is
 		// XORed with 1 when j + 2 is a partial sum of the cyclic BZ2_rNums sequence -- a few hundred bytes per block, walked by one
@@ -1017,7 +1006,7 @@ int launch_decode(const uint8_t* payload, const uint64_t* begin, const uint64_t*
 	k_imtf<<<njobs * nsub, IM_NT, smem2, st>>>(mtfv, mcap, jobs, njobs * nsub, q_scratch, bwt, cap);
 	return 0;
 }
-size_t inv_bwt_scratch_elems(int grid, uint32_t cap) { return (size_t)grid * cap + (size_t)grid * 2 * IB_VIS; }
+size_t inv_bwt_scratch_elems(int grid, uint32_t cap) { return (size_t)grid * cap; }
 constexpr uint32_t IB_MAXS_SMALL = 3072;
 // resident CTAs per SM of the variant launch_inv_bwt picks: 4 (256 threads) for slots of up to 48 KB
 int inv_bwt_ctas_per_sm(uint32_t cap)
