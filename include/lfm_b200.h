@@ -53,6 +53,36 @@ int writeLFMstackDevice(const void* d_im, const char* filename, const uint32_t x
 int readLFMroiDevice(const char* filename, const uint32_t lb[KLB_DATA_DIMS], const uint32_t ub[KLB_DATA_DIMS],
                      void* d_out, uint64_t capacity, uint64_t* out_bytes);
 
+/* ---- recording: a stack written frame by frame as its frames arrive, in device and host memory that do not grow with its length.
+   lfmStackWriterOpen takes the arguments of writeLFMstackEx; xyzct is the shape of the whole recording.  Frames arrive in the order
+   writeLFMstackEx reads im: frame f = z + Z*(c + C*t), x fastest within a frame.  Append copies its frames before it returns (the
+   caller may reuse its buffer at once): host frames are staged into the writer's batch buffer on the GPU, device frames (device or
+   managed memory on the first device of lfmSetDevices, code 3 otherwise; the caller synchronises its stream first) are copied
+   device to device.  Mode selection (headerVersion 0..7, with or without the video bit) runs on frame 0 when it arrives.  Every
+   batch of whole z-slabs (>= 96 MB and >= 2048 KLB blocks) is predicted and compressed once all its frames are in, and its payload
+   goes to its final file offset while the next batch fills; when the GPU is two batches behind, Append blocks.  A recording runs on
+   the first device of lfmSetDevices only.  Until Close, the file is not a valid .lfm file (the header and table are written last).
+   Close with every declared frame: the file is byte-identical to writeLFMstackEx of the whole stack with the same arguments, for any
+   append chunking and any mix of host and device frames; lfmGetLastStats reports the recording's totals.
+   Close earlier: with d the slowest of z, c, t whose extent is above 1 and u the frames per step of d, the largest multiple of u
+   received is kept (*frames_kept), xyzct[d] becomes kept / u and the file is byte-identical to writeLFMstackEx of that prefix
+   (blockSize clamped to the new extent); later frames are dropped.  Nothing kept: code 2 and an empty file.
+   Return codes.  Open: those of writeLFMstackEx for the same arguments (7 pixels that are not 16-bit, ZLIB, a forced predictor on a
+   video stack with way != 0; 3 a bad filename; 5 a file that cannot be created; 6 no device), and 7 for blockSize[3] or [4] above 1
+   after clamping (such blocks span frames that do not arrive one after the other); no file is created on an error.  Append: 3 past
+   the declared frame count (nothing is taken, the writer stays usable).  Any other failure (7 when auto-selection picks a predictor
+   a video stack with way != 0 cannot use, 6 CUDA, 5 file I/O, 3 a bad frames pointer) fails the writer: later appends return the
+   same code, and Close cuts the file to 0 bytes and returns it.  Close always frees w.  Calls on one writer come from one thread at a
+   time; writers and every other call of this library may be used side by side. */
+typedef struct lfm_stack_writer lfm_stack_writer;
+int lfmStackWriterOpen(lfm_stack_writer** w, const char* filename, const uint32_t xyzct[KLB_DATA_DIMS], enum KLB_DATA_TYPE dataType,
+                       const float32_t pixelSize[KLB_DATA_DIMS], const uint32_t blockSize[KLB_DATA_DIMS],
+                       enum KLB_COMPRESSION_TYPE compressionType, const char metadata[KLB_METADATA_SIZE], uint8_t headerVersion,
+                       uint8_t Nnum);
+int lfmStackWriterAppend(lfm_stack_writer* w, const void* frames, uint64_t nframes);             /* host memory */
+int lfmStackWriterAppendDevice(lfm_stack_writer* w, const void* d_frames, uint64_t nframes);     /* device memory */
+int lfmStackWriterClose(lfm_stack_writer* w, uint64_t* frames_kept);                               /* finishes the file, frees w */
+
 /* header byte 0 / byte 1 of a file (stored predictor | video bit, Nnum); 0 ok */
 int readLFMheaderEx(const char* filename, uint8_t* headerVersion, uint8_t* Nnum);
 

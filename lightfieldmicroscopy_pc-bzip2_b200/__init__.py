@@ -101,6 +101,11 @@ lib.lfmBz2Decompress.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,
 lib.lfmBz2Decompress.restype = C.c_int
 lib.lfmBz2DecompressDevice.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
 lib.lfmBz2DecompressDevice.restype = C.c_int
+lib.lfmStackWriterOpen.argtypes = [C.POINTER(C.c_void_p), C.c_char_p, _u32x5, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_uint8, C.c_uint8]
+lib.lfmStackWriterOpen.restype = C.c_int
+lib.lfmStackWriterAppend.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]; lib.lfmStackWriterAppend.restype = C.c_int
+lib.lfmStackWriterAppendDevice.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]; lib.lfmStackWriterAppendDevice.restype = C.c_int
+lib.lfmStackWriterClose.argtypes = [C.c_void_p, C.POINTER(C.c_uint64)]; lib.lfmStackWriterClose.restype = C.c_int
 
 _libc = C.CDLL(None)
 _libc.free.argtypes = [C.c_void_p]
@@ -111,7 +116,8 @@ EXPORTS = ["writeKLBstack", "writeKLBstackSlices", "readKLBheader", "readKLBstac
            "lfmGetLastStats", "lfmLastError", "lfmDebugEncodeBlock", "lfmDebugPredictDevice", "lfmDebugParMemcpy",
            "lfmShardCompress", "lfmShardWritePayload", "lfmShardFetchPayload", "lfmWriteHeader", "lfmSelectDevice",
            "lfmBz2Compress", "lfmBz2CompressDevice", "lfmBz2Decompress", "lfmBz2DecompressDevice",
-           "writeLFMstackDevice", "readLFMroiDevice"]
+           "writeLFMstackDevice", "readLFMroiDevice",
+           "lfmStackWriterOpen", "lfmStackWriterAppend", "lfmStackWriterAppendDevice", "lfmStackWriterClose"]
 
 
 class LfmError(RuntimeError):
@@ -165,6 +171,86 @@ def write_stack(img, filename, header_version=0, nnum=13, block_size=None, way=N
     if rc:
         raise LfmError(rc, "writeLFMstackEx")
     return rc
+
+
+class StackWriter:
+    """Records a stack frame by frame into `filename` (lfmStackWriterOpen / Append / Close, include/lfm_b200.h).
+
+    shape: [z][y][x] or [t][c][z][y][x] of the whole recording; frames arrive in that order, x fastest.  .append takes a numpy uint16
+    array of [n][y][x] or [y][x], or a CUDA torch.uint16 / torch.int16 tensor of the same shapes on the first device of
+    set_devices; the frames are copied before it returns.  .close() finishes the file and returns the number of frames kept: all of
+    them gives the file write_stack writes for the whole stack, fewer keeps the whole steps of the slowest dimension received.  As a
+    context manager the writer is closed on exit, also when the block raises, so that what was recorded is kept.  Errors raise
+    LfmError with the library's code."""
+
+    def __init__(self, filename, shape, header_version=0, nnum=13, block_size=None, way=None, codec=BZIP2):
+        if len(shape) not in (3, 5):
+            raise ValueError("shape is [z][y][x] or [t][c][z][y][x]")
+        if way is not None:
+            set_way(way)
+        self.frame_shape = (int(shape[-2]), int(shape[-1]))
+        self._kept = 0
+        self._w = C.c_void_p()
+        bs = _bs(block_size)
+        rc = lib.lfmStackWriterOpen(C.byref(self._w), os.fsencode(filename), _xyzct(shape), UINT16_TYPE, None,
+                                    C.cast(bs, C.c_void_p) if bs is not None else None, codec, None, header_version, nnum)
+        if rc:
+            self._w = None
+            raise LfmError(rc, "lfmStackWriterOpen")
+
+    def append(self, frames):
+        if self._w is None:
+            raise ValueError("the writer is closed")
+        if tuple(frames.shape[-2:]) != self.frame_shape or frames.ndim not in (2, 3):
+            raise ValueError("append takes [n][y][x] or [y][x] frames of %dx%d pixels" % self.frame_shape)
+        n = 1 if frames.ndim == 2 else int(frames.shape[0])
+        if _is_cuda_tensor(frames):
+            import torch
+            if frames.dtype not in (torch.uint16, torch.int16):
+                raise TypeError("append takes a torch.uint16 or torch.int16 tensor")
+            src = frames.view(torch.int16).contiguous()
+            with torch.cuda.device(src.device):
+                torch.cuda.current_stream().synchronize()           # the writer copies on its own stream
+                rc = lib.lfmStackWriterAppendDevice(self._w, src.data_ptr(), n)
+        else:
+            if not isinstance(frames, np.ndarray) or frames.dtype != np.uint16:
+                raise TypeError("append takes a numpy uint16 array")
+            src = np.ascontiguousarray(frames)
+            rc = lib.lfmStackWriterAppend(self._w, src.ctypes.data, n)
+        if rc:
+            raise LfmError(rc, "lfmStackWriterAppend")
+
+    def close(self):
+        """finish the file; returns the frames kept"""
+        if self._w is None:
+            return self._kept
+        kept = C.c_uint64()
+        rc = lib.lfmStackWriterClose(self._w, C.byref(kept))
+        self._w = None
+        self._kept = kept.value
+        if rc:
+            raise LfmError(rc, "lfmStackWriterClose")
+        return self._kept
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        if exc[0] is None:
+            self.close()
+        else:
+            try:
+                self.close()
+            except LfmError:
+                pass                                                # the exception of the block is the one to report
+        return False
+
+    def __del__(self):
+        if getattr(self, "_w", None) is not None:
+            try:
+                self.close()
+            except Exception:
+                pass
 
 
 def read_header(filename):

@@ -382,7 +382,7 @@ static uint64_t host_block_bytes(const Geom& g, uint64_t id)
 }
 
 int Engine::compress_blocks_none(const uint16_t* d_sym, const StackDesc& s, uint64_t first, uint64_t count,
-                                 uint32_t* sizes_out, const uint8_t** d_payload, uint64_t* payload_bytes, CompressStats* stt)
+                                 uint32_t* sizes_out, const uint8_t** d_payload, uint64_t* payload_bytes, CompressStats* stt, Buf& pay)
 {
 	cudaStream_t st = (cudaStream_t)stream_;
 	const Geom g = make_geom(s);
@@ -395,17 +395,17 @@ int Engine::compress_blocks_none(const uint16_t* d_sym, const StackDesc& s, uint
 		starts[i] = acc; sizes_out[i] = (uint32_t)n; acc += n;
 	}
 	int rc;
-	if ((rc = reserve(payload2_[pay_sel_], acc + 16))) return rc;
+	if ((rc = reserve(pay, acc + 16))) return rc;
 	if ((rc = reserve(offs_, count * 8))) return rc;
 	cudaMemcpyAsync(offs_.p, starts.data(), count * 8, cudaMemcpyHostToDevice, st);
 	for (uint64_t b0 = 0; b0 < count; b0 += 0x40000000ull) {
 		const uint32_t nj = (uint32_t)std::min<uint64_t>(0x40000000ull, count - b0);
-		k_none_gather<<<nj, 256, 0, st>>>(d_sym, g, first + b0, (const uint64_t*)offs_.p + b0, (uint8_t*)payload2_[pay_sel_].p);
+		k_none_gather<<<nj, 256, 0, st>>>(d_sym, g, first + b0, (const uint64_t*)offs_.p + b0, (uint8_t*)pay.p);
 		if (stt) stt->launches++;
 	}
 	cudaStreamSynchronize(st);                                  // `starts` is pageable host memory
 	if ((rc = check("compress_blocks_none"))) return rc;
-	*d_payload = (const uint8_t*)payload2_[pay_sel_].p; *payload_bytes = acc;
+	*d_payload = (const uint8_t*)pay.p; *payload_bytes = acc;
 	return LFM_OK;
 }
 
@@ -433,10 +433,11 @@ int Engine::decompress_blocks_none(const uint8_t* d_payload, const uint64_t* beg
 
 // ------------------------------------------------------------------------------------------------ compress
 int Engine::compress_blocks(const uint16_t* d_sym, const StackDesc& s, uint64_t first, uint64_t count,
-                            uint32_t* sizes_out, const uint8_t** d_payload, uint64_t* payload_bytes, CompressStats* stt)
+                            uint32_t* sizes_out, const uint8_t** d_payload, uint64_t* payload_bytes, CompressStats* stt, Buf* payload)
 {
 	cudaSetDevice(device_);
-	if (s.codec == 0) return compress_blocks_none(d_sym, s, first, count, sizes_out, d_payload, payload_bytes, stt);
+	Buf& pay = payload ? *payload : payload_;
+	if (s.codec == 0) return compress_blocks_none(d_sym, s, first, count, sizes_out, d_payload, payload_bytes, stt, pay);
 	cudaStream_t st = (cudaStream_t)stream_;
 	const Geom g = make_geom(s);
 	EncSizes z;
@@ -460,7 +461,7 @@ int Engine::compress_blocks(const uint16_t* d_sym, const StackDesc& s, uint64_t 
 	if ((rc = reserve(out_, BS * (size_t)z.ocap + 16))) return rc;
 	const int Gres = groups_for((uint32_t)B);                                  // forked groups need a scratch region each
 	if ((rc = reserve(scratch_, (size_t)Gres * grid * bwt_scratch_elems_per_cta(z.cap) * 4))) return rc;
-	if ((rc = reserve(payload2_[pay_sel_], pcap + 16))) return rc;
+	if ((rc = reserve(pay, pcap + 16))) return rc;
 	if ((rc = reserve(sizes_, count * 4))) return rc;
 	if ((rc = reserve(offs_, B * 8 + sizeof(Totals)))) return rc;
 	Totals* tot = (Totals*)((uint8_t*)offs_.p + B * 8);
@@ -497,7 +498,7 @@ int Engine::compress_blocks(const uint16_t* d_sym, const StackDesc& s, uint64_t 
 			if (G > 1) { cudaEvent_t je = (cudaEvent_t)ev_[5 + gi]; cudaEventRecord(je, sg); cudaStreamWaitEvent(st, je, 0); }
 		}
 		k_offsets<<<1, 1024, 0, st>>>((EncJob*)jobs_.p, nj, z.nsub, tot, (uint64_t*)offs_.p, (uint32_t*)sizes_.p + b0, pcap);
-		k_compact<<<nj, 256, 0, st>>>((uint8_t*)out_.p, z.ocap, (EncJob*)jobs_.p, z.nsub, (uint64_t*)offs_.p, (uint32_t*)sizes_.p + b0, (uint8_t*)payload2_[pay_sel_].p, pcap);
+		k_compact<<<nj, 256, 0, st>>>((uint8_t*)out_.p, z.ocap, (EncJob*)jobs_.p, z.nsub, (uint64_t*)offs_.p, (uint32_t*)sizes_.p + b0, (uint8_t*)pay.p, pcap);
 		launches += 4 * G + 2;
 		last_njobs_ = ns;
 	}
@@ -521,7 +522,7 @@ int Engine::compress_blocks(const uint16_t* d_sym, const StackDesc& s, uint64_t 
 	if (h.overflow) { err_ = "payload buffer overflow"; return LFM_ERR_BZIP; }
 	if (h.err & 4u) { err_ = "a KLB block needs more bzip2 blocks than the engine reserves per stream"; return LFM_ERR_UNSUPPORTED; }
 	if (h.err) { err_ = "block encoder reported an error"; return LFM_ERR_BZIP; }
-	*d_payload = (const uint8_t*)payload2_[pay_sel_].p;
+	*d_payload = (const uint8_t*)pay.p;
 	*payload_bytes = h.running;
 	return LFM_OK;
 }

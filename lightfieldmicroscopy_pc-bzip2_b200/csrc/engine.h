@@ -55,9 +55,11 @@ public:
 
 	// Compress KLB blocks [first, first+count) of the device-resident SYMBOL image.
 	// sizes_out[count] (host) receives each block's stream size; the streams are left compacted, in block order,
-	// in an engine-owned device buffer (*d_payload, *payload_bytes) that stays valid until the next call.
+	// in an engine-owned device buffer (*d_payload, *payload_bytes) that stays valid until the next call, or in `payload` (grown as
+	// needed) when the caller owns the buffer: a stack writer keeps its payload there while other calls use the engine.
+	struct Buf { void* p = nullptr; size_t cap = 0; };
 	int compress_blocks(const uint16_t* d_sym, const StackDesc& s, uint64_t first, uint64_t count,
-	                    uint32_t* sizes_out, const uint8_t** d_payload, uint64_t* payload_bytes, CompressStats* st);
+	                    uint32_t* sizes_out, const uint8_t** d_payload, uint64_t* payload_bytes, CompressStats* st, Buf* payload = nullptr);
 
 	// Decode the listed KLB blocks from a device-resident payload into the device-resident symbol image.
 	// begin/end: byte range of each listed block inside d_payload (host arrays).
@@ -93,18 +95,15 @@ public:
 	const std::string& last_error() const { return err_; }
 
 	// growable device scratch, kept across calls
-	struct Buf { void* p = nullptr; size_t cap = 0; };
 	int reserve(Buf& b, size_t bytes);
 	// buffers the orchestrator (klb_imageIO.cpp) keeps on this GPU between calls: image, symbol image, payload, frame 0, and
-	// the second image / payload buffer of the slab pipeline
+	// the second image / payload buffer of the read pipeline
 	Buf user[6];
-	// growable pinned host staging buffers: slot 0 = towards the GPU, slot 1 = from the GPU (the two directions of the slab
+	// growable pinned host staging buffers: slot 0 = towards the GPU, slot 1 = from the GPU (the two directions of the read
 	// pipeline run on different host threads at the same time)
 	void* pinned(size_t bytes, int slot = 0);
-	// copy streams of the slab pipeline (0: host -> device, 1: device -> host), beside the compute stream
+	// copy streams of the read pipeline (0: host -> device, 1: device -> host), beside the compute stream
 	void* copy_stream(int i) { return aux_stream(kMaxGroups + i); }
-	// which of the two payload buffers compress_blocks fills next (the other one may still be on its way to the host)
-	void use_payload_buffer(int i) { pay_sel_ = i & 1; }
 
 	// debugging / stage-parity hook: copies of the intermediate arrays of the LAST compress_blocks batch
 	struct EncodeTrace {
@@ -120,7 +119,7 @@ private:
 	int check(const char* what);
 	// KLB_COMPRESSION_TYPE::NONE (src/klb_imageIO.cpp:207-210, :620-623): gather / scatter only
 	int compress_blocks_none(const uint16_t* d_sym, const StackDesc& s, uint64_t first, uint64_t count,
-	                         uint32_t* sizes_out, const uint8_t** d_payload, uint64_t* payload_bytes, CompressStats* st);
+	                         uint32_t* sizes_out, const uint8_t** d_payload, uint64_t* payload_bytes, CompressStats* st, Buf& pay);
 	int decompress_blocks_none(const uint8_t* d_payload, const uint64_t* begin, const uint64_t* end, const uint64_t* block_ids,
 	                           uint64_t count, uint16_t* d_sym, const StackDesc& s, DecompressStats* st);
 
@@ -128,8 +127,7 @@ private:
 	void* stream_ = nullptr;
 	std::string err_;
 	// workspace
-	Buf jobs_, txt_, bwt_, rank_, mtfv_, sel_, out_, scratch_, payload2_[2], sizes_, offs_;
-	int pay_sel_ = 0;
+	Buf jobs_, txt_, bwt_, rank_, mtfv_, sel_, out_, scratch_, payload_, sizes_, offs_;
 	Buf djobs_, dbegin_, dend_, dids_, tt_;
 	Buf sel_sorted_, sel_hist_, sel_e_, sel_cand_;
 	Buf sz_tiles_, sz_bits_, sz_blocks_, sz_out_, sz_in_;      // bz2_compress: tile records, record-end bitmap, block records, stream, staging

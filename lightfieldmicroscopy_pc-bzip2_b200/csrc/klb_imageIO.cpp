@@ -24,6 +24,7 @@
 #include <functional>
 #include <mutex>
 #include <new>
+#include <system_error>
 #include <thread>
 #include <vector>
 #include <cuda_runtime.h>
@@ -297,9 +298,10 @@ inline size_t stage_chunk(size_t bytes)
 	return bytes >= ((size_t)64 << 20) ? kStageChunk : small;
 }
 
-void h2d_staged(Engine& e, void* dst, const void* src, size_t bytes, cudaStream_t st)
+// pageable source: through `ring` (kStageBufs * kStageChunk pinned bytes); pinned / registered / device memory, or no ring: one copy
+static void h2d_ring(uint8_t* ring, void* dst, const void* src, size_t bytes, cudaStream_t st)
 {
-	uint8_t* pin = (bytes >= kStageMin && is_pageable(src)) ? (uint8_t*)e.pinned(kStageBufs * kStageChunk, 0) : nullptr;
+	uint8_t* pin = (ring && bytes >= kStageMin && is_pageable(src)) ? ring : nullptr;
 	if (!pin) { cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st); return; }
 	const size_t CH = stage_chunk(bytes);
 	cudaEvent_t ev[kStageBufs];
@@ -313,8 +315,13 @@ void h2d_staged(Engine& e, void* dst, const void* src, size_t bytes, cudaStream_
 		cudaMemcpyAsync((uint8_t*)dst + off, buf, len, cudaMemcpyHostToDevice, st);
 		cudaEventRecord(ev[i % kStageBufs], st);
 	}
-	cudaStreamSynchronize(st);                                   // the staging buffers are shared: free them before anyone else asks
+	cudaStreamSynchronize(st);                                   // the ring is free again when this returns
 	for (auto& x : ev) cudaEventDestroy(x);
+}
+void h2d_staged(Engine& e, void* dst, const void* src, size_t bytes, cudaStream_t st)
+{
+	const bool staged = bytes >= kStageMin && is_pageable(src);        // the engine's ring is only allocated when it is needed
+	h2d_ring(staged ? (uint8_t*)e.pinned(kStageBufs * kStageChunk, 0) : nullptr, dst, src, bytes, st);
 }
 
 void d2h_staged(Engine& e, void* dst, const void* src, size_t bytes, cudaStream_t st)
@@ -347,19 +354,18 @@ struct ShardOut {
 };
 enum { UB_IMG = 0, UB_SYM = 1, UB_PAY = 2, UB_F0 = 3, UB_IMG2 = 4, UB_PAY2 = 5 };
 
-// ------------------------------------------------------------------------------------------------ slab pipeline (one GPU)
-// Large stacks written to a file go through the GPU in batches of whole z-slabs: while batch b is predicted and compressed, batch
-// b + 1 is on its way to the GPU (pinned staging + copy stream 0, own host thread) and the streams of batch b - 1 are on their
-// way to the file (copy stream 1 + pwrite at the final offset, own host thread) -- the counterpart of the reference's block
-// threads feeding blockWriter through a staging queue (src/klb_imageIO.cpp:1152-1217, :2446).  Two image and two payload buffers.
-struct FileSink { int fd = -1; uint64_t base = 0; };               // payload byte 0 lives at file offset `base`
+// ------------------------------------------------------------------------------------------------ stack writer (one GPU)
+// A recording is compressed in batches of whole z-slabs as its frames arrive (DESIGN.md §4c): lfmStackWriterAppend copies frames
+// into one of two batch image buffers (pinned staging ring + upload stream), a worker thread predicts and compresses every
+// complete batch on the engine under the API lock, and a file thread streams its payload to its final offset behind the
+// blockOffset table of the declared stack (pinned ring + download stream + pwrite) while the next batch fills.  Large stacks of
+// writeLFMstackEx / writeLFMstackDevice go through the same writer (write_stack_with_writer).  Everything a writer needs
+// between two calls is its own (WriterRes): other calls may use the engine's buffers, pinned slots and streams in between.
 constexpr uint64_t kBatchBytes = (uint64_t)96 << 20;               // raw bytes per batch (at least one slab)
 constexpr uint64_t kBatchBlocks = 2048;                            // ... and at least this many KLB blocks
 
-static int payload_to_fd(Engine& e, const uint8_t* d_payload, uint64_t bytes, int fd, uint64_t file_off, cudaStream_t st)
+static int payload_to_fd(uint8_t* pin, const uint8_t* d_payload, uint64_t bytes, int fd, uint64_t file_off, cudaStream_t st)
 {
-	uint8_t* pin = (uint8_t*)e.pinned(kStageBufs * kStageChunk, 1);
-	if (!pin) return LFM_ERR_CUDA;
 	cudaEvent_t ev[kStageBufs];
 	for (auto& x : ev) cudaEventCreateWithFlags(&x, cudaEventDisableTiming);
 	const size_t nch = (size_t)((bytes + kStageChunk - 1) / kStageChunk);
@@ -374,119 +380,442 @@ static int payload_to_fd(Engine& e, const uint8_t* d_payload, uint64_t bytes, in
 		if (i + kStageBufs - 1 < nch) issue(i + kStageBufs - 1);           // its buffer was written out in the previous iteration
 		if (cudaEventSynchronize(ev[i % kStageBufs]) != cudaSuccess) { cudaGetLastError(); rc = LFM_ERR_CUDA; break; }
 		const uint64_t o = (uint64_t)i * kStageChunk; const size_t len = (size_t)std::min<uint64_t>(kStageChunk, bytes - o);
-		const uint8_t* buf = pin + (i % kStageBufs) * kStageChunk;
-		size_t done = 0;
-		while (done < len) {
-			const ssize_t w = pwrite(fd, buf + done, len - done, (off_t)(file_off + o + done));
-			if (w <= 0) { rc = LFM_ERR_CREATE; break; }
-			done += (size_t)w;
-		}
+		rc = write_all(fd, pin + (i % kStageBufs) * kStageChunk, len, file_off + o);
 	}
 	cudaStreamSynchronize(st);
 	for (auto& x : ev) cudaEventDestroy(x);
 	return rc;
 }
 
-// slabs per batch; 0 when the stack is not worth / not fit for batching (few slabs, c or t blocked)
-static uint64_t slabs_per_batch(const klb_image_header& h, const Layout& L, bool pair_frames)
+// slabs per batch of a stack written or read in batches (at least; batch_cuts may make a batch longer)
+static uint64_t batch_slabs(const klb_image_header& h, const Layout& L)
 {
-	if (env_int("LFM_B200_NO_PIPELINE", 0) || h.blockSize[3] != 1 || h.blockSize[4] != 1) return 0;
 	const uint64_t batch_bytes = env_int("LFM_B200_BATCH_KB", 0) > 0 ? (uint64_t)env_int("LFM_B200_BATCH_KB", 0) << 10 : kBatchBytes;   // test knob
 	const uint64_t slab_bytes = (uint64_t)h.blockSize[2] * L.fpx * 2;
 	uint64_t n = std::max<uint64_t>(1, batch_bytes / std::max<uint64_t>(1, slab_bytes));
 	// the block codec kernels are latency bound: a batch needs a few thousand KLB blocks to fill the GPU (k_huff_decode alone keeps
 	// ~1500 streams in flight), or the overlap won is lost again in half-empty kernels
 	if (env_int("LFM_B200_BATCH_KB", 0) <= 0) n = std::max<uint64_t>(n, (kBatchBlocks + L.blocksPerSlab - 1) / L.blocksPerSlab);
-	if (pair_frames && (h.blockSize[2] & 1)) n = (n + 1) & ~(uint64_t)1;         // batches start on even frames
+	return n;
+}
+// slabs per batch of the pipelined paths; 0 when the stack is not worth / not fit for batching (few slabs, c or t blocked)
+static uint64_t slabs_per_batch(const klb_image_header& h, const Layout& L)
+{
+	if (env_int("LFM_B200_NO_PIPELINE", 0) || h.blockSize[3] != 1 || h.blockSize[4] != 1) return 0;
+	const uint64_t n = batch_slabs(h, L);
 	return L.nSlabs >= 2 * n ? n : 0;
 }
-
-static int compress_pipelined(const FrameSource& src, klb_image_header& h, const Layout& L, const StackDesc& desc, int k, int video,
-                              const FileSink& sink, uint64_t per)
+// first flattened frame of slab s (c and t not blocked: the slabs tile the frames in order); L.F past the last slab
+static uint64_t slab_first_frame(const klb_image_header& h, const Layout& L, uint64_t s)
 {
-	Engine& e = Engine::for_device(g_set.first_device);
-	cudaSetDevice(e.device());
-	const int dev = e.device();
-	cudaStream_t up_st = (cudaStream_t)e.copy_stream(0), down_st = (cudaStream_t)e.copy_stream(1);   // created on this thread
-	const uint64_t nbatch = (L.nSlabs + per - 1) / per;
-	struct Batch { uint64_t s0, s1, f0, nf; };
-	std::vector<Batch> B(nbatch);
-	uint64_t max_nf = 0;
-	for (uint64_t b = 0; b < nbatch; b++) {
-		B[b].s0 = b * per; B[b].s1 = std::min(L.nSlabs, (b + 1) * per);
-		uint64_t f0, f1; slab_frames(h, L, B[b].s0, B[b].s1, f0, f1);
-		B[b].f0 = f0; B[b].nf = f1 - f0 + 1;
-		max_nf = std::max(max_nf, B[b].nf);
+	return s >= L.nSlabs ? L.F : (s / L.nb[2]) * h.xyzct[2] + (s % L.nb[2]) * h.blockSize[2];
+}
+// Batch boundaries: slab indices, cut[0] = 0, cut.back() = L.nSlabs, at least `per` slabs apart.  With pair_frames (video stack +
+// predictor: an odd frame is predicted from the even frame before it) a batch only starts on a slab whose first frame is even, so
+// that it holds the frame each of its odd frames needs; a cut moves forward to the next such slab.  Slab s starts at frame
+// (s / nb[2]) * Z + (s % nb[2]) * blockSize[2]: with Z not a multiple of the block depth and c or t above 1, slabs in the middle of
+// the stack start on odd frames whatever the batch length (with Z odd and an even depth, every slab of an odd volume does).
+static std::vector<uint64_t> batch_cuts(const klb_image_header& h, const Layout& L, uint64_t per, bool pair_frames)
+{
+	std::vector<uint64_t> cut(1, 0);
+	for (;;) {
+		uint64_t c = cut.back() + per;
+		while (pair_frames && c < L.nSlabs && (slab_first_frame(h, L, c) & 1)) c++;
+		if (c >= L.nSlabs) break;
+		cut.push_back(c);
 	}
-	const size_t img_bytes = (size_t)max_nf * L.fpx * 2;
-	if ((!src.device && (e.reserve(e.user[UB_IMG], img_bytes) || e.reserve(e.user[UB_IMG2], img_bytes))) ||
-	    (k != 0 && e.reserve(e.user[UB_SYM], img_bytes))) return LFM_ERR_CUDA;
-	if (!e.pinned(kStageBufs * kStageChunk, 0) || !e.pinned(kStageBufs * kStageChunk, 1)) return LFM_ERR_CUDA;
-	uint16_t* dimg[2] = { (uint16_t*)e.user[UB_IMG].p, (uint16_t*)e.user[UB_IMG2].p };
-	uint16_t* dsym = (uint16_t*)e.user[UB_SYM].p;
-	std::thread up_th[2], wr_th[2];
-	int up_rc[2] = { 0, 0 }, wr_rc[2] = { 0, 0 };
-	auto upload = [&](uint64_t b, int slot) {
-		if (src.device) return;                                        // the kernels read the caller's device stack
+	cut.push_back(L.nSlabs);
+	return cut;
+}
+
+struct WriterRes {                // device memory, pinned staging rings and copy streams of one open writer
+	int dev = -1;
+	Engine::Buf img[2], sym, pay[2];
+	uint8_t* up_pin = nullptr;    // kStageBufs * kStageChunk bytes each
+	uint8_t* down_pin = nullptr;
+	cudaStream_t up_st = nullptr, down_st = nullptr;
+	int init(int device)
+	{
+		dev = device;
 		cudaSetDevice(dev);
-		const Batch& bt = B[b];
-		if (src.base) h2d_staged(e, dimg[slot], src.frame(bt.f0, L.fpx), (size_t)bt.nf * L.fpx * 2, up_st);
-		else for (uint64_t f = 0; f < bt.nf; f++) h2d_staged(e, dimg[slot] + f * L.fpx, src.frame(bt.f0 + f, L.fpx), (size_t)L.fpx * 2, up_st);
-		if (cudaStreamSynchronize(up_st) != cudaSuccess) { cudaGetLastError(); up_rc[slot] = LFM_ERR_CUDA; }
-	};
-	auto join_all = [&]() { for (auto& t : up_th) if (t.joinable()) t.join(); for (auto& t : wr_th) if (t.joinable()) t.join(); };
-	int rc = LFM_OK;
-	uint64_t pay_off = 0, blk = 0;
-	std::vector<uint32_t> sizes;
-	const double t0 = now_ms();
-	up_th[0] = std::thread(upload, 0, 0);
-	for (uint64_t b = 0; b < nbatch && rc == LFM_OK; b++) {
-		const int slot = (int)(b & 1);
-		up_th[slot].join();                                            // batch b is resident
-		if ((rc = up_rc[slot])) break;
-		if (b + 1 < nbatch) up_th[slot ^ 1] = std::thread(upload, b + 1, slot ^ 1);   // its image buffer was last read by batch b - 1 (done)
-		if (wr_th[slot].joinable()) { wr_th[slot].join(); if ((rc = wr_rc[slot])) break; }   // payload buffer `slot` (batch b - 2) is on disk
-		const Batch& bt = B[b];
-		const uint16_t* img_base = src.device ? src.base : dimg[slot] - bt.f0 * L.fpx;   // virtual base: absolute frame indexing
-		const uint16_t* sym_base = img_base;
-		CompressStats st;
-		if (k != 0) {
-			rc = e.predict(img_base, dsym - bt.f0 * L.fpx, desc, k, video, (uint32_t)bt.f0, (uint32_t)bt.nf);
-			st.launches++;
-			if (rc) break;
-			sym_base = dsym - bt.f0 * L.fpx;
-		}
-		const uint64_t first = bt.s0 * L.blocksPerSlab, count = (bt.s1 - bt.s0) * L.blocksPerSlab;
-		sizes.resize(count);
-		const uint8_t* dpay = nullptr; uint64_t pbytes = 0;
-		e.use_payload_buffer(slot);
-		rc = e.compress_blocks(sym_base, desc, first, count, sizes.data(), &dpay, &pbytes, &st);
-		if (rc) { g_err = e.last_error(); break; }
-		if (k != 0) g_stats.ms_predict += e.last_predict_ms();
-		uint64_t acc = blk ? h.blockOffset[blk - 1] : 0;
-		for (uint64_t i = 0; i < count; i++) { acc += sizes[i]; h.blockOffset[blk + i] = acc; }
-		blk += count;
-		g_stats.ms_rle += st.ms_rle; g_stats.ms_bwt += st.ms_bwt; g_stats.ms_mtf += st.ms_mtf; g_stats.ms_huff += st.ms_huff;
-		g_stats.gpu_launches += st.launches; g_stats.periodic_blocks += st.periodic_blocks;
-		const uint64_t at = sink.base + pay_off;
-		// one writer at a time (they share the pinned ring and copy stream 1): batch b - 1 had all of this batch's kernels to finish
-		if (wr_th[slot ^ 1].joinable()) { wr_th[slot ^ 1].join(); if ((rc = wr_rc[slot ^ 1])) break; }
-		wr_th[slot] = std::thread([&, slot, dpay, pbytes, at]() { cudaSetDevice(dev); wr_rc[slot] = pbytes ? payload_to_fd(e, dpay, pbytes, sink.fd, at, down_st) : LFM_OK; });
-		pay_off += pbytes;
+		if (cudaStreamCreateWithFlags(&up_st, cudaStreamNonBlocking) != cudaSuccess || cudaStreamCreateWithFlags(&down_st, cudaStreamNonBlocking) != cudaSuccess ||
+		    cudaHostAlloc((void**)&up_pin, kStageBufs * kStageChunk, cudaHostAllocDefault) != cudaSuccess ||
+		    cudaHostAlloc((void**)&down_pin, kStageBufs * kStageChunk, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return LFM_ERR_CUDA; }
+		return LFM_OK;
 	}
-	join_all();
-	e.use_payload_buffer(0);
-	for (int i = 0; i < 2; i++) { if (!rc && up_rc[i]) rc = up_rc[i]; if (!rc && wr_rc[i]) rc = wr_rc[i]; }
-	g_stats.payload_bytes = pay_off;
-	g_stats.ms_total += now_ms() - t0;
+	~WriterRes()
+	{
+		if (dev < 0) return;
+		DeviceGuard g;
+		cudaSetDevice(dev);
+		for (Engine::Buf* b : { &img[0], &img[1], &sym, &pay[0], &pay[1] }) if (b->p) cudaFree(b->p);
+		if (up_pin) cudaFreeHost(up_pin);
+		if (down_pin) cudaFreeHost(down_pin);
+		if (up_st) cudaStreamDestroy(up_st);
+		if (down_st) cudaStreamDestroy(down_st);
+	}
+};
+// The resources of the last closed writer wait for the next one on the same device: writeLFMstackEx opens a writer per large stack,
+// and pinning 64 MB of staging memory costs more than compressing a batch.  Never destroyed (CUDA may be gone at exit).
+std::mutex g_spare_mu;
+WriterRes* g_spare = nullptr;
+WriterRes* take_res(int dev)
+{
+	std::lock_guard<std::mutex> lk(g_spare_mu);
+	WriterRes* r = g_spare;
+	if (r && r->dev == dev) { g_spare = nullptr; return r; }
+	return nullptr;
+}
+void give_res(WriterRes* r)
+{
+	std::lock_guard<std::mutex> lk(g_spare_mu);
+	std::swap(r, g_spare);
+	delete r;
+}
+}  // namespace
+
+struct lfm_stack_writer {
+	klb_image_header h;               // the declared recording (blockSize clamped); headerVersion stored once the predictor is known
+	int fd = -1;
+	uint8_t hv_in = 0;
+	int video = 0, k = -1;            // k: predictor, -1 until frame 0 has been through mode selection
+	Layout L;
+	StackDesc desc;
+	std::vector<uint64_t> cut;        // batch b = slabs [cut[b], cut[b + 1]) (batch_cuts)
+	uint64_t nbatch = 0, base = 0;    // batches, file offset of payload byte 0 (declared table)
+	Engine* e = nullptr;
+	WriterRes* res = nullptr;
+	uint64_t received = 0;            // frames taken by Append (calling thread only)
+	std::mutex mu;                    // guards the fields below
+	std::condition_variable cv;
+	uint64_t ready = 0, computed = 0; // batches whose frames are all on the GPU / that are predicted and compressed
+	bool closing = false;
+	int rc = LFM_OK;                  // first failure: the writer is failed from then on
+	std::string err;
+	std::thread worker, wr_th[2];     // wr_th[i]: the payload of the last batch compressed into res->pay[i] on its way to the file
+	int wr_rc[2] = { 0, 0 };
+	uint64_t pay_off = 0;             // payload bytes of the batches compressed so far (worker thread)
+	lfm_stats st;
+	double t_open = 0;
+
+	int fail(int code, const std::string& what)
+	{
+		std::lock_guard<std::mutex> lk(mu);
+		if (!rc) { rc = code; err = what; }
+		cv.notify_all();
+		return rc;
+	}
+	int failed() { std::lock_guard<std::mutex> lk(mu); return rc; }
+	uint64_t batch_of_frame(uint64_t f) const
+	{
+		const uint64_t s = (f / h.xyzct[2]) * L.nb[2] + (f % h.xyzct[2]) / h.blockSize[2];
+		return (uint64_t)(std::upper_bound(cut.begin(), cut.end(), s) - cut.begin()) - 1;
+	}
+	uint64_t batch_first_frame(uint64_t b) const { return slab_first_frame(h, L, cut[b]); }
+	// predict + compress slabs [s0, s1) of image buffer `slot`, whose first frame is slab s0's, as the stack `d` (the declared one,
+	// or at an early close the kept prefix); block sizes -> h.blockOffset (kept blocks are a prefix of the declared ones)
+	int compress(const StackDesc& d, const klb_image_header& hd, const Layout& Ld, uint64_t s0, uint64_t s1, int slot,
+	             const uint8_t** dpay, uint64_t* pbytes)
+	{
+		LFM_API_LOCK();
+		cudaSetDevice(e->device());
+		const uint64_t f0 = slab_first_frame(hd, Ld, s0), nf = slab_first_frame(hd, Ld, s1) - f0;
+		const uint16_t* img_base = (const uint16_t*)res->img[slot].p - f0 * L.fpx;     // virtual base: absolute frame indexing
+		const uint16_t* sym_base = img_base;
+		CompressStats cs;
+		int r;
+		if (k != 0) {
+			uint16_t* sb = (uint16_t*)res->sym.p - f0 * L.fpx;
+			if ((r = e->predict(img_base, sb, d, k, video, (uint32_t)f0, (uint32_t)nf))) return fail(r, "predictor launch failed");
+			cs.launches++;
+			sym_base = sb;
+		}
+		const uint64_t first = s0 * L.blocksPerSlab, count = (s1 - s0) * L.blocksPerSlab;
+		std::vector<uint32_t> sizes(count);
+		if ((r = e->compress_blocks(sym_base, d, first, count, sizes.data(), dpay, pbytes, &cs, &res->pay[slot]))) return fail(r, e->last_error());
+		if (k != 0) st.ms_predict += e->last_predict_ms();
+		uint64_t acc = first ? h.blockOffset[first - 1] : 0;
+		for (uint64_t i = 0; i < count; i++) { acc += sizes[i]; h.blockOffset[first + i] = acc; }
+		st.ms_rle += cs.ms_rle; st.ms_bwt += cs.ms_bwt; st.ms_mtf += cs.ms_mtf; st.ms_huff += cs.ms_huff;
+		st.gpu_launches += cs.launches; st.periodic_blocks += cs.periodic_blocks;
+		return LFM_OK;
+	}
+	// the worker: every batch once all its frames are on the GPU; its payload leaves on a file thread while the next one computes
+	void run()
+	{
+		try { run_batches(); }
+		catch (const std::bad_alloc&) { fail(LFM_ERR_CREATE, "out of host memory"); }
+		catch (const std::exception& ex) { fail(LFM_ERR_BZIP, ex.what()); }
+		for (int i = 0; i < 2; i++) if (wr_th[i].joinable()) { wr_th[i].join(); if (wr_rc[i]) fail(wr_rc[i], "payload write failed"); }
+	}
+	void run_batches()
+	{
+		cudaSetDevice(res->dev);
+		for (uint64_t b = 0; b < nbatch; b++) {
+			{
+				std::unique_lock<std::mutex> lk(mu);
+				cv.wait(lk, [&] { return ready > b || closing || rc; });
+				if (rc || ready <= b) break;
+			}
+			const int slot = (int)(b & 1);
+			if (wr_th[slot].joinable()) { wr_th[slot].join(); if (wr_rc[slot]) { fail(wr_rc[slot], "payload write failed"); break; } }
+			const uint8_t* dpay = nullptr; uint64_t pbytes = 0;
+			if (compress(desc, h, L, cut[b], cut[b + 1], slot, &dpay, &pbytes)) break;
+			{ std::lock_guard<std::mutex> lk(mu); computed = b + 1; }
+			cv.notify_all();                                            // image buffer `slot` is free for batch b + 2
+			// one file thread at a time (they share the download ring and stream)
+			if (wr_th[slot ^ 1].joinable()) { wr_th[slot ^ 1].join(); if (wr_rc[slot ^ 1]) { fail(wr_rc[slot ^ 1], "payload write failed"); break; } }
+			const uint64_t at = base + pay_off;
+			wr_th[slot] = std::thread([this, slot, dpay, pbytes, at]() {
+				cudaSetDevice(res->dev);
+				try { wr_rc[slot] = pbytes ? payload_to_fd(res->down_pin, dpay, pbytes, fd, at, res->down_st) : LFM_OK; }
+				catch (const std::exception&) { wr_rc[slot] = LFM_ERR_CREATE; }
+			});
+			pay_off += pbytes;
+		}
+	}
+};
+
+namespace {
+// xyzct / blockSize of `h` checked as writeLFMstackEx checks them, plus what a writer cannot do; `h` comes back clamped
+int writer_open(lfm_stack_writer** out, const std::string& filename, const klb_image_header& h_in)
+{
+	*out = nullptr;
+	klb_image_header h(h_in);
+	int rc = validate(h, true);
+	if (rc) return rc;
+	if (current_ndev() <= 0) { std::cout << "ERROR: lfm_b200: no CUDA device available (this engine has no CPU fallback)" << std::endl; return LFM_ERR_CUDA; }
+	for (int d = 0; d < 5; d++) h.blockSize[d] = std::min(h.blockSize[d], h.xyzct[d]);     // src/klb_imageIO.cpp:2407-2408
+	if (h.blockSize[3] != 1 || h.blockSize[4] != 1) {
+		g_err = "blocks over several channels or time points span frames that do not arrive one after the other"; return LFM_ERR_UNSUPPORTED;
+	}
+	const uint8_t hv = h.headerVersion;
+	const int video = (hv & 0x80) ? 1 : 0, way = current_way();
+	int k = -1;
+	if ((hv & 0x7F) >= NUM_PREDICTORS) {
+		k = hv & 0x77 & 0x7F;                          // `hv & 0x7F - 8` parses as hv & 0x77 (src/klb_imageIO.cpp:2380)
+		if (k > 7) { std::cout << "ERROR: The predictors hava not selected!" << std::endl; return LFM_ERR_UNSUPPORTED; }
+		if (k != 0 && video && way != 0) {
+			std::cout << "ERROR: lfm_b200: video stacks are only invertible with predictor way 0 (tiles); refusing to write" << std::endl;
+			return LFM_ERR_UNSUPPORTED;
+		}
+	}
+	std::unique_ptr<lfm_stack_writer> w(new lfm_stack_writer);
+	w->t_open = now_ms();
+	memset(&w->st, 0, sizeof(w->st));
+	w->L = make_layout(h);
+	h.resizeBlockOffset(w->L.Nb);
+	w->h = h;
+	w->hv_in = hv; w->video = video; w->k = k;
+	w->desc = make_desc(h, way);
+	// the predictor is not known before frame 0 with auto-selection: video batches start on even frames in any case
+	w->cut = batch_cuts(h, w->L, batch_slabs(h, w->L), video != 0);
+	w->nbatch = w->cut.size() - 1;
+	uint64_t max_nf = 0;
+	for (uint64_t b = 0; b < w->nbatch; b++) max_nf = std::max(max_nf, w->batch_first_frame(b + 1) - w->batch_first_frame(b));
+	w->base = 320 + w->L.Nb * sizeof(uint64_t);
+	w->e = &Engine::for_device(g_set.first_device);
+	const int dev = w->e->device();
+	cudaSetDevice(dev);
+	std::unique_ptr<WriterRes> res(take_res(dev));
+	if (!res) { res.reset(new WriterRes); if (res->init(dev)) { g_err = "pinned staging memory or copy streams could not be allocated"; return LFM_ERR_CUDA; } }
+	const size_t img_bytes = (size_t)max_nf * w->L.fpx * 2;
+	if (w->e->reserve(res->img[0], img_bytes) || w->e->reserve(res->img[1], img_bytes) || (k > 0 && w->e->reserve(res->sym, img_bytes))) {
+		give_res(res.release()); g_err = "batch buffers could not be allocated"; return LFM_ERR_CUDA;
+	}
+	const bool existed = access(filename.c_str(), F_OK) == 0;
+	const int fd = open(filename.c_str(), O_RDWR | O_CREAT, 0666);
+	if (fd < 0) { give_res(res.release()); std::cout << "ERROR: file " << filename << " could not be opened" << std::endl; return LFM_ERR_CREATE; }
+	// an existing file is overwritten in place (its pages are kept) and cut to size at Close; until then its old header must not
+	// make it look like a valid .lfm file
+	uint8_t zero[320] = { 0 };
+	struct stat sb;
+	if (fstat(fd, &sb) == 0 && sb.st_size > 0 && write_all(fd, zero, std::min<size_t>(sizeof(zero), (size_t)sb.st_size), 0)) {
+		close(fd); give_res(res.release()); return LFM_ERR_CREATE;
+	}
+	w->fd = fd;
+	w->res = res.release();
+	lfm_stack_writer* p = w.get();
+	try { w->worker = std::thread([p]() { p->run(); }); }
+	catch (const std::system_error&) {
+		close(fd); if (!existed) unlink(filename.c_str());
+		give_res(w->res); g_err = "the writer thread could not be started"; return LFM_ERR_CREATE;
+	}
+	*out = w.release();
+	return LFM_OK;
+}
+
+int writer_append(lfm_stack_writer* w, const void* frames, uint64_t n, bool device)
+{
+	if (int r = w->failed()) { g_err = w->err; return r; }
+	if (n == 0) return LFM_OK;
+	if (w->received + n > w->L.F || w->received + n < n) {
+		g_err = "append past the declared frame count (" + std::to_string(w->L.F) + " frames)"; return LFM_ERR_OPEN;
+	}
+	int rc = LFM_OK;
+	if (!frames) w->fail(LFM_ERR_OPEN, "frames is NULL");
+	else if (device && (rc = check_device_ptr(frames, "d_frames"))) w->fail(rc, g_err);
+	if (int r = w->failed()) { g_err = w->err; return r; }
+	WriterRes& R = *w->res;
+	cudaSetDevice(R.dev);
+	const size_t frame_bytes = (size_t)w->L.fpx * 2;
+	const uint8_t* src = (const uint8_t*)frames;
+	uint64_t f = w->received;
+	const uint64_t end = w->received + n;
+	while (f < end) {
+		const uint64_t b = w->batch_of_frame(f), f0 = w->batch_first_frame(b), f1 = w->batch_first_frame(b + 1);
+		const int slot = (int)(b & 1);
+		{
+			// back-pressure: image buffer `slot` is free once batch b - 2 has been compressed
+			std::unique_lock<std::mutex> lk(w->mu);
+			w->cv.wait(lk, [&] { return b < 2 || w->computed >= b - 1 || w->rc; });
+			if (w->rc) break;
+		}
+		const uint64_t m = std::min(f1, end) - f;
+		uint8_t* dst = (uint8_t*)R.img[slot].p + (f - f0) * frame_bytes;
+		if (device) cudaMemcpyAsync(dst, src, m * frame_bytes, cudaMemcpyDeviceToDevice, R.up_st);
+		else h2d_ring(R.up_pin, dst, src, m * frame_bytes, R.up_st);
+		const bool batch_done = f + m == f1;
+		if ((f == 0 || batch_done) && cudaStreamSynchronize(R.up_st) != cudaSuccess) { cudaGetLastError(); w->fail(LFM_ERR_CUDA, "frame upload failed"); break; }
+		if (f == 0 && w->k < 0) {
+			// mode selection on frame 0 (branches A and B of writeImage, src/klb_imageIO.cpp:2273-2377)
+			LFM_API_LOCK();
+			const double t0 = now_ms();
+			int k = 0;
+			if ((rc = w->e->select_mode((const uint16_t*)R.img[0].p, w->desc, w->st.entropy, &k))) { w->fail(rc, w->e->last_error()); break; }
+			w->st.ms_select = now_ms() - t0;
+			w->st.selected = 1; w->st.gpu_launches += 7 + 5;       // 7 candidate predictions + count, starts, sort, histogram, entropy
+			if (k != 0 && w->video && w->desc.way != 0) {
+				std::cout << "ERROR: lfm_b200: video stacks are only invertible with predictor way 0 (tiles); refusing to write" << std::endl;
+				w->fail(LFM_ERR_UNSUPPORTED, "video stacks are only invertible with predictor way 0"); break;
+			}
+			if (k != 0 && w->e->reserve(R.sym, R.img[0].cap)) { w->fail(LFM_ERR_CUDA, "symbol buffer could not be allocated"); break; }
+			w->k = k;
+		}
+		if (f == 0) {
+			w->h.headerVersion = (uint8_t)((w->hv_in & 0x80) | w->k);
+			w->st.predictor = w->k;
+		}
+		f += m; src += m * frame_bytes;
+		if (batch_done) {
+			{ std::lock_guard<std::mutex> lk(w->mu); w->ready = b + 1; }
+			w->cv.notify_all();
+		}
+	}
+	// the caller may reuse its buffer when this returns: a pinned or device source is read by copies still in flight
+	if (cudaStreamSynchronize(R.up_st) != cudaSuccess) { cudaGetLastError(); w->fail(LFM_ERR_CUDA, "frame upload failed"); }
+	w->received = f;
+	if (int r = w->failed()) { g_err = w->err; return r; }
+	return LFM_OK;
+}
+
+// the kept prefix of an early close: whole steps of the slowest of z, c, t with more than one entry; its last partial batch is
+// compressed here, the payload already in the file moves left by the table entries it no longer needs
+int writer_finish(lfm_stack_writer* w, uint64_t* kept_out)
+{
+	const klb_image_header& H = w->h;
+	const Layout& L = w->L;
+	int d = 2; uint64_t u = 1;
+	if (H.xyzct[4] > 1) { d = 4; u = (uint64_t)H.xyzct[2] * H.xyzct[3]; }
+	else if (H.xyzct[3] > 1) { d = 3; u = H.xyzct[2]; }
+	const uint64_t kept = w->received / u * u;
+	*kept_out = kept;
+	if (kept == 0) { g_err = "no frame was recorded"; return LFM_ERR_BZIP; }
+	klb_image_header h2(H);
+	const uint64_t done_slabs = w->cut[w->computed];
+	Layout L2 = L;
+	if (kept < L.F) {
+		h2.xyzct[d] = (uint32_t)(kept / u);
+		for (int i = 0; i < 5; i++) h2.blockSize[i] = std::min(h2.blockSize[i], h2.xyzct[i]);
+		L2 = make_layout(h2);
+	}
+	const uint64_t done = std::min(done_slabs, L2.nSlabs);
+	uint64_t bytes = done ? H.blockOffset[done * L.blocksPerSlab - 1] : 0;     // payload of the kept blocks already in the file
+	int rc = LFM_OK;
+	if (done < L2.nSlabs) {
+		// the tail: slabs [done, kept) sit in the image buffer of batch `computed`, which starts at slab `done`
+		const StackDesc d2 = make_desc(h2, w->desc.way);
+		const int slot = (int)(w->computed & 1);
+		const uint8_t* dpay = nullptr; uint64_t pbytes = 0;
+		if ((rc = w->compress(d2, h2, L2, done, L2.nSlabs, slot, &dpay, &pbytes))) return rc;
+		cudaSetDevice(w->res->dev);
+		if (pbytes && (rc = payload_to_fd(w->res->down_pin, dpay, pbytes, w->fd, w->base + bytes, w->res->down_st))) return rc;
+		bytes += pbytes;
+	}
+	h2.resizeBlockOffset(L2.Nb);
+	memcpy(h2.blockOffset, H.blockOffset, L2.Nb * sizeof(uint64_t));
+	const uint64_t base2 = 320 + L2.Nb * sizeof(uint64_t);
+	// front to back: the destination lies before the source
+	for (uint64_t o = 0; base2 != w->base && o < bytes; o += kStageBufs * kStageChunk) {
+		const size_t len = (size_t)std::min<uint64_t>(kStageBufs * kStageChunk, bytes - o);
+		if ((rc = read_all(w->fd, w->res->down_pin, len, w->base + o))) return LFM_ERR_CREATE;
+		if ((rc = write_all(w->fd, w->res->down_pin, len, base2 + o))) return rc;
+	}
+	uint8_t fixed[320]; h2.packFixed(fixed);
+	if ((rc = write_all(w->fd, fixed, sizeof(fixed), 0)) || (rc = write_all(w->fd, h2.blockOffset, L2.Nb * sizeof(uint64_t), sizeof(fixed)))) return rc;
+	if (ftruncate(w->fd, (off_t)(base2 + bytes)) != 0) return LFM_ERR_CREATE;
+	w->st.payload_bytes = bytes;
+	w->h = h2;
+	return LFM_OK;
+}
+
+// finishes the file (or cuts it to 0 bytes after a failure), frees w; the recording's statistics become the calling thread's
+int writer_close(lfm_stack_writer* w, uint64_t* frames_kept, klb_image_header* h_out = nullptr)
+{
+	{ std::lock_guard<std::mutex> lk(w->mu); w->closing = true; }
+	w->cv.notify_all();
+	w->worker.join();
+	uint64_t kept = 0;
+	int rc = w->rc;
+	std::string err = w->err;
+	if (!rc) rc = writer_finish(w, &kept);
+	if (rc && ftruncate(w->fd, 0) != 0) { /* nothing more to do */ }
+	if (close(w->fd) != 0 && !rc) rc = LFM_ERR_CREATE;
+	if (frames_kept) *frames_kept = rc ? 0 : kept;
+	w->st.ms_total = now_ms() - w->t_open;
+	g_stats = w->st;
+	if (w->rc) g_err = err;
+	if (!rc && h_out) *h_out = w->h;
+	give_res(w->res);
+	delete w;
 	return rc;
 }
 
+// writeLFMstackEx / writeLFMstackDevice of a stack that fills at least two batches on one GPU: open a writer, append the stack, close
+bool takes_writer(const FrameSource& src, const klb_image_header& header)
+{
+	klb_image_header h(header);
+	if ((h.compressionType != KLB_COMPRESSION_TYPE::BZIP2 && h.compressionType != KLB_COMPRESSION_TYPE::NONE) || h.getBytesPerPixel() != 2) return false;
+	for (int d = 0; d < 5; d++) { if (h.xyzct[d] == 0 || h.blockSize[d] == 0) return false; h.blockSize[d] = std::min(h.blockSize[d], h.xyzct[d]); }
+	const int ndev = current_ndev();
+	if (ndev <= 0) return false;
+	const Layout L = make_layout(h);
+	if (!src.device && std::min<uint64_t>((uint64_t)ndev, L.nSlabs) != 1) return false;   // sharded over several GPUs
+	return slabs_per_batch(h, L) != 0;
+}
+
+int write_stack_with_writer(const std::string& filename, const FrameSource& src, klb_image_header& header)
+{
+	memset(&g_stats, 0, sizeof(g_stats));
+	lfm_stack_writer* w = nullptr;
+	int rc = writer_open(&w, filename, header);
+	if (rc) {
+		// as the one-shot path, which has created the file before it meets the error: an empty file is left
+		const int fd = rc == LFM_ERR_CREATE ? -1 : open(filename.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0666);
+		if (fd >= 0) close(fd);
+		return rc;
+	}
+	const uint64_t F = w->L.F;
+	try {
+		if (src.slices) { for (uint64_t f = 0; f < F && rc == LFM_OK; f++) rc = writer_append(w, src.slices[f], 1, false); }
+		else rc = writer_append(w, src.base, F, src.device);
+	} catch (const std::exception&) { rc = w->fail(LFM_ERR_CREATE, "out of host memory"); }   // the writer is closed all the same
+	uint64_t kept = 0;
+	const int rc2 = writer_close(w, &kept, &header);
+	return rc ? rc : rc2;
+}
 // Phase 1: everything up to the compacted streams in device memory + header.blockOffset[].
-// With a FileSink and one GPU, large stacks take the slab pipeline: the payload is then already in the file when this returns
-// (shards stays empty) and only the header + table are left to write.
-int compress_core(const FrameSource& src, klb_image_header& h, std::vector<ShardOut>& shards, std::vector<uint64_t>& shardFirstBlock,
-                  const FileSink* sink = nullptr)
+int compress_core(const FrameSource& src, klb_image_header& h, std::vector<ShardOut>& shards, std::vector<uint64_t>& shardFirstBlock)
 {
 	memset(&g_stats, 0, sizeof(g_stats));
 	int rc = validate(h, true);
@@ -533,14 +862,6 @@ int compress_core(const FrameSource& src, klb_image_header& h, std::vector<Shard
 
 	// a device stack lives on the first device: it is compressed there alone
 	const int D = src.device ? 1 : (int)std::min<uint64_t>((uint64_t)ndev, L.nSlabs);
-	if (sink && D == 1) {
-		const uint64_t per = slabs_per_batch(h, L, k != 0 && video);
-		if (per) {
-			FileSink fs = *sink; fs.base = sizeof(uint8_t) * 320 + L.Nb * sizeof(uint64_t);
-			shards.clear(); shardFirstBlock.clear();
-			return compress_pipelined(src, h, L, desc, k, video, fs, per);
-		}
-	}
 	const std::vector<uint64_t> cut = shard_cuts(h, L, D, k != 0 && video);
 	shards.assign(D, ShardOut());
 	shardFirstBlock.assign(D, 0);
@@ -667,7 +988,7 @@ struct PayloadSource {
 	}
 };
 
-// Full reads of large stacks on one GPU, the mirror image of compress_pipelined: while batch b (whole z-slabs) is decoded and
+// Full reads of large stacks on one GPU, the mirror image of the stack writer: while batch b (whole z-slabs) is decoded and
 // un-predicted, the streams of batch b + 1 are read from the file / host memory into the second payload buffer (pinned staging,
 // copy stream 0, own host thread) and the pixels of batch b - 1 travel to the caller's buffer (copy stream 1, own host thread).
 // With out_on_device, `out` is the caller's device buffer: the batches decode straight into it and there is no download stage.
@@ -678,13 +999,14 @@ static int decompress_pipelined(const klb_image_header& h, const Layout& L, cons
 	cudaSetDevice(e.device());
 	const int dev = e.device();
 	cudaStream_t up_st = (cudaStream_t)e.copy_stream(0), down_st = (cudaStream_t)e.copy_stream(1);
-	const uint64_t nbatch = (L.nSlabs + per - 1) / per;
+	const std::vector<uint64_t> cut = batch_cuts(h, L, per, k != 0 && video);
+	const uint64_t nbatch = cut.size() - 1;
 	struct Batch { uint64_t s0, s1, f0, nf, beg, end; };
 	std::vector<Batch> B(nbatch);
 	uint64_t max_nf = 0, max_pay = 0;
 	for (uint64_t b = 0; b < nbatch; b++) {
 		Batch& bt = B[b];
-		bt.s0 = b * per; bt.s1 = std::min(L.nSlabs, (b + 1) * per);
+		bt.s0 = cut[b]; bt.s1 = cut[b + 1];
 		uint64_t f0, f1; slab_frames(h, L, bt.s0, bt.s1, f0, f1);
 		bt.f0 = f0; bt.nf = f1 - f0 + 1;
 		const uint64_t id0 = bt.s0 * L.blocksPerSlab, id1 = bt.s1 * L.blocksPerSlab;
@@ -825,7 +1147,7 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 	// (the whole stack for a full read), which handles any alignment.
 	const bool sink_aligned = dsink && ((uintptr_t)dsink->d_out & 15) == 0;
 	if (full && D == 1 && desc.codec == 1 && (!dsink || sink_aligned)) {
-		const uint64_t per = slabs_per_batch(h, L, k != 0 && video);
+		const uint64_t per = slabs_per_batch(h, L);
 		if (per) return decompress_pipelined(h, L, desc, k, video, psrc, out, dsink != nullptr, per);
 	}
 	const bool direct = dsink && full && sink_aligned;   // decode into the caller's device buffer, no copy at the end
@@ -1016,6 +1338,10 @@ static int write_file(int fd, klb_image_header& h, std::vector<ShardOut>& shards
 
 static int write_stack_to_file(const std::string& filename, const FrameSource& src, klb_image_header& header)
 {
+	{
+		DeviceGuard g;
+		if (takes_writer(src, header)) return write_stack_with_writer(filename, src, header);
+	}
 	LFM_API_LOCK();
 	// the file is overwritten in place and cut to its final size at the end (same result as "wb", but an existing file of about
 	// the same size keeps its pages: rewriting a stack does not pay for page allocation again)
@@ -1024,9 +1350,8 @@ static int write_stack_to_file(const std::string& filename, const FrameSource& s
 	int rc;
 	try {
 		std::vector<ShardOut> shards; std::vector<uint64_t> first;
-		FileSink sink; sink.fd = fd;
-		rc = compress_core(src, header, shards, first, &sink);
-		if (rc == 0) rc = write_file(fd, header, shards);              // header + table (+ whatever payload is still on the GPUs)
+		rc = compress_core(src, header, shards, first);
+		if (rc == 0) rc = write_file(fd, header, shards);
 		if (rc == 0 && ftruncate(fd, (off_t)header.getCompressedFileSizeInBytes()) != 0) rc = LFM_ERR_CREATE;
 		if (rc != 0 && ftruncate(fd, 0) != 0) { /* nothing more to do */ }
 	} catch (const std::bad_alloc&) { g_err = "out of host memory"; rc = LFM_ERR_CREATE; }
@@ -1138,6 +1463,47 @@ try {
 	h.setHeader(xyzct, dataType, pixelSize, blockSize, compressionType, metadata, headerVersion, Nnum);
 	FrameSource src; src.base = (const uint16_t*)d_im; src.device = true;
 	return write_stack_to_file(std::string(filename), src, h);
+} LFM_CATCH
+
+int lfmStackWriterOpen(lfm_stack_writer** w, const char* filename, const uint32_t xyzct[5], enum KLB_DATA_TYPE dataType,
+                       const float32_t pixelSize[5], const uint32_t blockSize[5], enum KLB_COMPRESSION_TYPE compressionType,
+                       const char metadata[256], uint8_t headerVersion, uint8_t Nnum)
+try {
+	g_err.clear();
+	if (!w) return LFM_ERR_OPEN;
+	*w = nullptr;
+	if (!filename || !*filename || !xyzct) return LFM_ERR_OPEN;
+	DeviceGuard g;
+	klb_image_header h;
+	h.setHeader(xyzct, dataType, pixelSize, blockSize, compressionType, metadata, headerVersion, Nnum);
+	return writer_open(w, std::string(filename), h);
+} LFM_CATCH
+
+int lfmStackWriterAppend(lfm_stack_writer* w, const void* frames, uint64_t nframes)
+try {
+	g_err.clear();
+	if (!w) return LFM_ERR_OPEN;
+	DeviceGuard g;
+	try { return writer_append(w, frames, nframes, false); }
+	catch (const std::exception&) { g_err = "out of host memory"; return w->fail(LFM_ERR_CREATE, g_err); }   // fails the writer, as every other error
+} LFM_CATCH
+
+int lfmStackWriterAppendDevice(lfm_stack_writer* w, const void* d_frames, uint64_t nframes)
+try {
+	g_err.clear();
+	if (!w) return LFM_ERR_OPEN;
+	DeviceGuard g;
+	try { return writer_append(w, d_frames, nframes, true); }
+	catch (const std::exception&) { g_err = "out of host memory"; return w->fail(LFM_ERR_CREATE, g_err); }   // fails the writer, as every other error
+} LFM_CATCH
+
+int lfmStackWriterClose(lfm_stack_writer* w, uint64_t* frames_kept)
+try {
+	g_err.clear();
+	if (frames_kept) *frames_kept = 0;
+	if (!w) return LFM_ERR_OPEN;
+	DeviceGuard g;
+	return writer_close(w, frames_kept);
 } LFM_CATCH
 
 int readLFMroiDevice(const char* filename, const uint32_t lb[5], const uint32_t ub[5], void* d_out, uint64_t capacity, uint64_t* out_bytes)
