@@ -83,6 +83,29 @@ int lfmStackWriterAppend(lfm_stack_writer* w, const void* frames, uint64_t nfram
 int lfmStackWriterAppendDevice(lfm_stack_writer* w, const void* d_frames, uint64_t nframes);     /* device memory */
 int lfmStackWriterClose(lfm_stack_writer* w, uint64_t* frames_kept);                               /* finishes the file, frees w */
 
+/* ---- playing a stack back frame by frame, in bounded memory (single GPU: the first device of lfmSetDevices).
+   lfmStackReaderOpen opens `filename` for reading the inclusive x,y,z,c,t box lb..ub (NULL, NULL: the whole stack) as
+   readLFMroiDevice takes it; *frames = frames the box holds (its z*c*t extent), *frame_bytes = 2 * (x extent) * (y extent).  The
+   header and blockOffset table are read and checked once, and the same codes as readLFMroiDevice's come back in the same order:
+   2 corrupt or truncated table or payload, 3 file that cannot be opened or box outside the stack, 6 no device, 7 ZLIB payloads,
+   pixels that are not 16-bit, video written with way != 0, and blockSize[3] or [4] above 1 (blocks over several channels or time
+   points interleave their frames).
+   lfmStackReaderRead / ReadDevice deliver the next n frames of the box, dense [t][c][z][y][x] order, into host memory (pageable
+   or pinned) / device memory of the first device of lfmSetDevices (any even byte offset; code 3 for anything else), and return
+   once the frames are in dst.  *got = frames delivered: fewer than n only at the end, 0 past it (the reader stays usable).  The
+   concatenation of all reads is readLFMroiDevice's output for the box, bit for bit, whatever the chunking; host and device reads
+   may be mixed.  While the caller holds frames of batch b, batch b + 1 is decoded and batch b + 2 read from the file.  Any other
+   failure (a payload found truncated or corrupt on the way: 2) fails the reader: later reads and Close return its code, and
+   nothing is written past n frames of dst.  One reader is used from one thread at a time; other readers, writers and calls may
+   run between its reads.  Memory: two batches of frames and payload on the GPU, the staging rings, and the table.
+   lfmStackReaderClose frees the reader; lfmGetLastStats then holds the reader's totals. */
+typedef struct lfm_stack_reader lfm_stack_reader;
+int lfmStackReaderOpen(lfm_stack_reader** r, const char* filename, const uint32_t lb[KLB_DATA_DIMS], const uint32_t ub[KLB_DATA_DIMS],
+                       uint64_t* frames, uint64_t* frame_bytes);
+int lfmStackReaderRead(lfm_stack_reader* r, void* dst, uint64_t n, uint64_t* got);              /* host memory */
+int lfmStackReaderReadDevice(lfm_stack_reader* r, void* d_dst, uint64_t n, uint64_t* got);      /* device memory */
+int lfmStackReaderClose(lfm_stack_reader* r);                                                     /* frees r, returns its failure code */
+
 /* header byte 0 / byte 1 of a file (stored predictor | video bit, Nnum); 0 ok */
 int readLFMheaderEx(const char* filename, uint8_t* headerVersion, uint8_t* Nnum);
 

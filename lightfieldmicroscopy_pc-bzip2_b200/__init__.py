@@ -106,6 +106,11 @@ lib.lfmStackWriterOpen.restype = C.c_int
 lib.lfmStackWriterAppend.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]; lib.lfmStackWriterAppend.restype = C.c_int
 lib.lfmStackWriterAppendDevice.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]; lib.lfmStackWriterAppendDevice.restype = C.c_int
 lib.lfmStackWriterClose.argtypes = [C.c_void_p, C.POINTER(C.c_uint64)]; lib.lfmStackWriterClose.restype = C.c_int
+lib.lfmStackReaderOpen.argtypes = [C.POINTER(C.c_void_p), C.c_char_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+lib.lfmStackReaderOpen.restype = C.c_int
+lib.lfmStackReaderRead.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]; lib.lfmStackReaderRead.restype = C.c_int
+lib.lfmStackReaderReadDevice.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]; lib.lfmStackReaderReadDevice.restype = C.c_int
+lib.lfmStackReaderClose.argtypes = [C.c_void_p]; lib.lfmStackReaderClose.restype = C.c_int
 
 _libc = C.CDLL(None)
 _libc.free.argtypes = [C.c_void_p]
@@ -117,7 +122,8 @@ EXPORTS = ["writeKLBstack", "writeKLBstackSlices", "readKLBheader", "readKLBstac
            "lfmShardCompress", "lfmShardWritePayload", "lfmShardFetchPayload", "lfmWriteHeader", "lfmSelectDevice",
            "lfmBz2Compress", "lfmBz2CompressDevice", "lfmBz2Decompress", "lfmBz2DecompressDevice",
            "writeLFMstackDevice", "readLFMroiDevice",
-           "lfmStackWriterOpen", "lfmStackWriterAppend", "lfmStackWriterAppendDevice", "lfmStackWriterClose"]
+           "lfmStackWriterOpen", "lfmStackWriterAppend", "lfmStackWriterAppendDevice", "lfmStackWriterClose",
+           "lfmStackReaderOpen", "lfmStackReaderRead", "lfmStackReaderReadDevice", "lfmStackReaderClose"]
 
 
 class LfmError(RuntimeError):
@@ -281,19 +287,28 @@ def _write_stack_device(img, filename, header_version, nnum, block_size, way, co
     return rc
 
 
+def _device_out(shape, device, out):
+    """`out` checked to be a contiguous CUDA tensor of `shape`'s size in bytes on `device` (when given), or a new torch.uint16
+    tensor of `shape` on `device`"""
+    import torch
+    nbytes = 2 * int(np.prod(shape))
+    if out is None:
+        return torch.empty(shape, dtype=torch.uint16, device=device)
+    if not _is_cuda_tensor(out) or not out.is_contiguous() or out.numel() * out.element_size() != nbytes:
+        raise ValueError("out= takes a contiguous CUDA tensor of %d bytes" % nbytes)
+    if device is not None:
+        d = torch.device(device)
+        if d.type != "cuda" or (d.index if d.index is not None else torch.cuda.current_device()) != out.device.index:
+            raise ValueError("device=%s and out= on %s name different devices" % (device, out.device))
+    return out
+
+
 def _read_device(filename, lb, ub, shape, device, out):
     """decode the box lb..ub (None, None: the whole stack) of a file into a CUDA tensor: `out`, or a new torch.uint16 tensor of
     `shape` on `device`"""
     import torch
     nbytes = 2 * int(np.prod(shape))
-    if out is None:
-        out = torch.empty(shape, dtype=torch.uint16, device=device)
-    elif not _is_cuda_tensor(out) or not out.is_contiguous() or out.numel() * out.element_size() != nbytes:
-        raise ValueError("out= takes a contiguous CUDA tensor of %d bytes" % nbytes)
-    elif device is not None:
-        d = torch.device(device)
-        if d.type != "cuda" or (d.index if d.index is not None else torch.cuda.current_device()) != out.device.index:
-            raise ValueError("device=%s and out= on %s name different devices" % (device, out.device))
+    out = _device_out(shape, device, out)
     n = C.c_uint64()
     with torch.cuda.device(out.device):
         torch.cuda.current_stream().synchronize()               # the engine runs on its own stream
@@ -335,6 +350,101 @@ def read_roi(filename, lb, ub, way=None, device=None, out=None):
     if rc:
         raise LfmError(rc, "readKLBroiInPlace")
     return out
+
+
+class StackReader:
+    """Plays the box lb..ub (inclusive x,y,z,c,t bounds; None, None: the whole stack) of a .lfm file back frame by frame, in
+    bounded memory (lfmStackReaderOpen / Read / ReadDevice / Close, include/lfm_b200.h).  The next batch of frames is decoded on the
+    GPU while the caller works on the current one.
+
+    .frames is the number of frames of the box (its z*c*t extent, in [t][c][z] order) and .shape = (frames, y extent, x extent).
+    .read(n=1, out=None) returns the next n frames (fewer at the end, none past it) as a numpy uint16 array [n][y][x], or as a CUDA
+    torch.uint16 tensor when the reader was opened with device= or `out` (a contiguous CUDA tensor of n frames' bytes, at any even
+    byte offset) is given; the rules of read_roi apply.  Iterating yields one frame at a time.  As a context manager the reader is
+    closed on exit.  Errors raise LfmError with the library's code."""
+
+    def __init__(self, path, lb=None, ub=None, way=None, device=None):
+        if (lb is None) != (ub is None) or (lb is not None and (len(lb) != 5 or len(ub) != 5)):
+            raise ValueError("lb and ub are both None or both 5 inclusive x,y,z,c,t bounds")
+        if device is not None:
+            import torch
+            if torch.device(device).type != "cuda":
+                raise ValueError("device= names a CUDA device")
+        if way is not None:
+            set_way(way)
+        self._device = device
+        self._r = C.c_void_p()
+        frames, fb = C.c_uint64(), C.c_uint64()
+        rc = lib.lfmStackReaderOpen(C.byref(self._r), os.fsencode(path), _u32x5(*lb) if lb is not None else None,
+                                    _u32x5(*ub) if ub is not None else None, C.byref(frames), C.byref(fb))
+        if rc:
+            self._r = None
+            raise LfmError(rc, "lfmStackReaderOpen")
+        if lb is None:
+            x, y = read_header(path)["xyzct"][:2]
+        else:
+            x, y = ub[0] - lb[0] + 1, ub[1] - lb[1] + 1
+        self.frames = frames.value
+        self.shape = (self.frames, int(y), int(x))
+
+    def read(self, n=1, out=None):
+        if self._r is None:
+            raise ValueError("the reader is closed")
+        n = int(n)
+        if n < 0:
+            raise ValueError("n must be >= 0")
+        shape = (n,) + self.shape[1:]
+        got = C.c_uint64()
+        if self._device is not None or out is not None:
+            import torch
+            out = _device_out(shape, self._device, out)
+            with torch.cuda.device(out.device):
+                torch.cuda.current_stream().synchronize()           # the reader copies on its own stream
+                rc = lib.lfmStackReaderReadDevice(self._r, out.data_ptr() if n else None, n, C.byref(got))
+            if rc:
+                raise LfmError(rc, "lfmStackReaderReadDevice")
+            return out if got.value == n and out.shape == shape else out.reshape(-1)[:got.value * shape[1] * shape[2]].view(
+                (got.value,) + shape[1:])
+        a = np.empty(shape, dtype=np.uint16)
+        rc = lib.lfmStackReaderRead(self._r, a.ctypes.data, n, C.byref(got))
+        if rc:
+            raise LfmError(rc, "lfmStackReaderRead")
+        return a[:got.value]
+
+    def __iter__(self):
+        while True:
+            f = self.read(1)
+            if len(f) == 0:
+                return
+            yield f[0]
+
+    def close(self):
+        if self._r is None:
+            return
+        rc = lib.lfmStackReaderClose(self._r)
+        self._r = None
+        if rc:
+            raise LfmError(rc, "lfmStackReaderClose")
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        if exc[0] is None:
+            self.close()
+        else:
+            try:
+                self.close()
+            except LfmError:
+                pass                                                # the exception of the block is the one to report
+        return False
+
+    def __del__(self):
+        if getattr(self, "_r", None) is not None:
+            try:
+                self.close()
+            except Exception:
+                pass
 
 
 def shard_compress(frames, header_version, nnum=13, block_size=None, way=None):

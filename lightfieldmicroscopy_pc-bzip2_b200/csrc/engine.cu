@@ -363,10 +363,10 @@ int Engine::unpredict(const uint16_t* d_sym, uint16_t* d_out, const StackDesc& s
 	return check("unpredict");
 }
 
-int Engine::roi_gather(const uint16_t* d_frames, const StackDesc& s, const uint32_t lb[5], const uint32_t ub[5], uint16_t* d_out)
+int Engine::roi_gather(const uint16_t* d_frames, const StackDesc& s, const uint32_t lb[5], const uint32_t ub[5], uint16_t* d_out, void* stream)
 {
 	cudaSetDevice(device_);
-	launch_roi_gather(d_frames, s.xyzct, lb, ub, d_out, sm_count_, (cudaStream_t)stream_);
+	launch_roi_gather(d_frames, s.xyzct, lb, ub, d_out, sm_count_, (cudaStream_t)(stream ? stream : stream_));
 	return check("roi_gather");
 }
 

@@ -82,8 +82,8 @@ public:
 	int unpredict(const uint16_t* d_sym, uint16_t* d_out, const StackDesc& s, int predictor, int video, uint32_t z0, uint32_t nz);
 
 	// The box lb..ub (inclusive x,y,z,c,t bounds) of the decoded frames d_frames (absolute frame indexing) -> dense
-	// [t][c][z][y][x] at d_out, one k_roi_gather launch on the engine stream (not synchronised).
-	int roi_gather(const uint16_t* d_frames, const StackDesc& s, const uint32_t lb[5], const uint32_t ub[5], uint16_t* d_out);
+	// [t][c][z][y][x] at d_out, one k_roi_gather launch on `stream` (NULL: the engine stream), not synchronised.
+	int roi_gather(const uint16_t* d_frames, const StackDesc& s, const uint32_t lb[5], const uint32_t ub[5], uint16_t* d_out, void* stream = nullptr);
 
 	// device time of the last predict() / unpredict() call (valid once the stream has been synchronised)
 	double last_predict_ms();
@@ -96,14 +96,10 @@ public:
 
 	// growable device scratch, kept across calls
 	int reserve(Buf& b, size_t bytes);
-	// buffers the orchestrator (klb_imageIO.cpp) keeps on this GPU between calls: image, symbol image, payload, frame 0, and
-	// the second image / payload buffer of the read pipeline
-	Buf user[6];
-	// growable pinned host staging buffers: slot 0 = towards the GPU, slot 1 = from the GPU (the two directions of the read
-	// pipeline run on different host threads at the same time)
+	// buffers the orchestrator (klb_imageIO.cpp) keeps on this GPU between calls: image, symbol image, payload, frame 0
+	Buf user[4];
+	// growable pinned host staging buffers: slot 0 = towards the GPU, slot 1 = from the GPU
 	void* pinned(size_t bytes, int slot = 0);
-	// copy streams of the read pipeline (0: host -> device, 1: device -> host), beside the compute stream
-	void* copy_stream(int i) { return aux_stream(kMaxGroups + i); }
 
 	// debugging / stage-parity hook: copies of the intermediate arrays of the LAST compress_blocks batch
 	struct EncodeTrace {

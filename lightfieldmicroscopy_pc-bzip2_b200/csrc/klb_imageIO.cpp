@@ -324,9 +324,10 @@ void h2d_staged(Engine& e, void* dst, const void* src, size_t bytes, cudaStream_
 	h2d_ring(staged ? (uint8_t*)e.pinned(kStageBufs * kStageChunk, 0) : nullptr, dst, src, bytes, st);
 }
 
-void d2h_staged(Engine& e, void* dst, const void* src, size_t bytes, cudaStream_t st)
+// pageable destination: through `ring` (kStageBufs * kStageChunk pinned bytes); pinned / registered memory, or no ring: one copy
+static void d2h_ring(uint8_t* ring, void* dst, const void* src, size_t bytes, cudaStream_t st)
 {
-	uint8_t* pin = (bytes >= kStageMin && is_pageable(dst)) ? (uint8_t*)e.pinned(kStageBufs * kStageChunk, 1) : nullptr;
+	uint8_t* pin = (ring && bytes >= kStageMin && is_pageable(dst)) ? ring : nullptr;
 	if (!pin) { cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st); return; }
 	const size_t CH = stage_chunk(bytes);
 	cudaEvent_t ev[kStageBufs];
@@ -346,13 +347,18 @@ void d2h_staged(Engine& e, void* dst, const void* src, size_t bytes, cudaStream_
 	}
 	for (auto& x : ev) cudaEventDestroy(x);
 }
+void d2h_staged(Engine& e, void* dst, const void* src, size_t bytes, cudaStream_t st)
+{
+	const bool staged = bytes >= kStageMin && is_pageable(dst);
+	d2h_ring(staged ? (uint8_t*)e.pinned(kStageBufs * kStageChunk, 1) : nullptr, dst, src, bytes, st);
+}
 
 // ------------------------------------------------------------------------------------------------ compress core
 struct ShardOut {
 	std::vector<uint32_t> sizes; int rc = 0; CompressStats st; double ms_h2d = 0, ms_d2h = 0; std::string err;
 	const uint8_t* d_payload = nullptr; uint64_t payload_bytes = 0; int device = 0;      // streams stay on the GPU until fetched
 };
-enum { UB_IMG = 0, UB_SYM = 1, UB_PAY = 2, UB_F0 = 3, UB_IMG2 = 4, UB_PAY2 = 5 };
+enum { UB_IMG = 0, UB_SYM = 1, UB_PAY = 2, UB_F0 = 3 };
 
 // ------------------------------------------------------------------------------------------------ stack writer (one GPU)
 // A recording is compressed in batches of whole z-slabs as its frames arrive (DESIGN.md §4c): lfmStackWriterAppend copies frames
@@ -360,7 +366,7 @@ enum { UB_IMG = 0, UB_SYM = 1, UB_PAY = 2, UB_F0 = 3, UB_IMG2 = 4, UB_PAY2 = 5 }
 // complete batch on the engine under the API lock, and a file thread streams its payload to its final offset behind the
 // blockOffset table of the declared stack (pinned ring + download stream + pwrite) while the next batch fills.  Large stacks of
 // writeLFMstackEx / writeLFMstackDevice go through the same writer (write_stack_with_writer).  Everything a writer needs
-// between two calls is its own (WriterRes): other calls may use the engine's buffers, pinned slots and streams in between.
+// between two calls is its own (PipeRes): other calls may use the engine's buffers, pinned slots and streams in between.
 constexpr uint64_t kBatchBytes = (uint64_t)96 << 20;               // raw bytes per batch (at least one slab)
 constexpr uint64_t kBatchBlocks = 2048;                            // ... and at least this many KLB blocks
 
@@ -410,27 +416,28 @@ static uint64_t slab_first_frame(const klb_image_header& h, const Layout& L, uin
 {
 	return s >= L.nSlabs ? L.F : (s / L.nb[2]) * h.xyzct[2] + (s % L.nb[2]) * h.blockSize[2];
 }
-// Batch boundaries: slab indices, cut[0] = 0, cut.back() = L.nSlabs, at least `per` slabs apart.  With pair_frames (video stack +
+// Batch boundaries of slabs [s_begin, s_end): cut[0] = s_begin, cut.back() = s_end, at least `per` slabs apart.  With pair_frames (video stack +
 // predictor: an odd frame is predicted from the even frame before it) a batch only starts on a slab whose first frame is even, so
 // that it holds the frame each of its odd frames needs; a cut moves forward to the next such slab.  Slab s starts at frame
 // (s / nb[2]) * Z + (s % nb[2]) * blockSize[2]: with Z not a multiple of the block depth and c or t above 1, slabs in the middle of
 // the stack start on odd frames whatever the batch length (with Z odd and an even depth, every slab of an odd volume does).
-static std::vector<uint64_t> batch_cuts(const klb_image_header& h, const Layout& L, uint64_t per, bool pair_frames)
+static std::vector<uint64_t> batch_cuts(const klb_image_header& h, const Layout& L, uint64_t per, bool pair_frames,
+                                        uint64_t s_begin, uint64_t s_end)
 {
-	std::vector<uint64_t> cut(1, 0);
+	std::vector<uint64_t> cut(1, s_begin);
 	for (;;) {
 		uint64_t c = cut.back() + per;
-		while (pair_frames && c < L.nSlabs && (slab_first_frame(h, L, c) & 1)) c++;
-		if (c >= L.nSlabs) break;
+		while (pair_frames && c < s_end && (slab_first_frame(h, L, c) & 1)) c++;
+		if (c >= s_end) break;
 		cut.push_back(c);
 	}
-	cut.push_back(L.nSlabs);
+	cut.push_back(s_end);
 	return cut;
 }
 
-struct WriterRes {                // device memory, pinned staging rings and copy streams of one open writer
+struct PipeRes {                  // device memory, pinned staging rings and copy streams of one open writer or reader
 	int dev = -1;
-	Engine::Buf img[2], sym, pay[2];
+	Engine::Buf img[2], sym, pay[2], stage;     // stage: a reader's cropped frames on their way to host memory
 	uint8_t* up_pin = nullptr;    // kStageBufs * kStageChunk bytes each
 	uint8_t* down_pin = nullptr;
 	cudaStream_t up_st = nullptr, down_st = nullptr;
@@ -443,30 +450,30 @@ struct WriterRes {                // device memory, pinned staging rings and cop
 		    cudaHostAlloc((void**)&down_pin, kStageBufs * kStageChunk, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return LFM_ERR_CUDA; }
 		return LFM_OK;
 	}
-	~WriterRes()
+	~PipeRes()
 	{
 		if (dev < 0) return;
 		DeviceGuard g;
 		cudaSetDevice(dev);
-		for (Engine::Buf* b : { &img[0], &img[1], &sym, &pay[0], &pay[1] }) if (b->p) cudaFree(b->p);
+		for (Engine::Buf* b : { &img[0], &img[1], &sym, &pay[0], &pay[1], &stage }) if (b->p) cudaFree(b->p);
 		if (up_pin) cudaFreeHost(up_pin);
 		if (down_pin) cudaFreeHost(down_pin);
 		if (up_st) cudaStreamDestroy(up_st);
 		if (down_st) cudaStreamDestroy(down_st);
 	}
 };
-// The resources of the last closed writer wait for the next one on the same device: writeLFMstackEx opens a writer per large stack,
-// and pinning 64 MB of staging memory costs more than compressing a batch.  Never destroyed (CUDA may be gone at exit).
+// The resources of the last closed writer or reader wait for the next one on the same device: writeLFMstackEx and full reads open
+// one per large stack, and pinning 64 MB of staging memory costs more than a batch.  Never destroyed (CUDA may be gone at exit).
 std::mutex g_spare_mu;
-WriterRes* g_spare = nullptr;
-WriterRes* take_res(int dev)
+PipeRes* g_spare = nullptr;
+PipeRes* take_res(int dev)
 {
 	std::lock_guard<std::mutex> lk(g_spare_mu);
-	WriterRes* r = g_spare;
+	PipeRes* r = g_spare;
 	if (r && r->dev == dev) { g_spare = nullptr; return r; }
 	return nullptr;
 }
-void give_res(WriterRes* r)
+void give_res(PipeRes* r)
 {
 	std::lock_guard<std::mutex> lk(g_spare_mu);
 	std::swap(r, g_spare);
@@ -484,7 +491,7 @@ struct lfm_stack_writer {
 	std::vector<uint64_t> cut;        // batch b = slabs [cut[b], cut[b + 1]) (batch_cuts)
 	uint64_t nbatch = 0, base = 0;    // batches, file offset of payload byte 0 (declared table)
 	Engine* e = nullptr;
-	WriterRes* res = nullptr;
+	PipeRes* res = nullptr;
 	uint64_t received = 0;            // frames taken by Append (calling thread only)
 	std::mutex mu;                    // guards the fields below
 	std::condition_variable cv;
@@ -609,7 +616,7 @@ int writer_open(lfm_stack_writer** out, const std::string& filename, const klb_i
 	w->hv_in = hv; w->video = video; w->k = k;
 	w->desc = make_desc(h, way);
 	// the predictor is not known before frame 0 with auto-selection: video batches start on even frames in any case
-	w->cut = batch_cuts(h, w->L, batch_slabs(h, w->L), video != 0);
+	w->cut = batch_cuts(h, w->L, batch_slabs(h, w->L), video != 0, 0, w->L.nSlabs);
 	w->nbatch = w->cut.size() - 1;
 	uint64_t max_nf = 0;
 	for (uint64_t b = 0; b < w->nbatch; b++) max_nf = std::max(max_nf, w->batch_first_frame(b + 1) - w->batch_first_frame(b));
@@ -617,8 +624,8 @@ int writer_open(lfm_stack_writer** out, const std::string& filename, const klb_i
 	w->e = &Engine::for_device(g_set.first_device);
 	const int dev = w->e->device();
 	cudaSetDevice(dev);
-	std::unique_ptr<WriterRes> res(take_res(dev));
-	if (!res) { res.reset(new WriterRes); if (res->init(dev)) { g_err = "pinned staging memory or copy streams could not be allocated"; return LFM_ERR_CUDA; } }
+	std::unique_ptr<PipeRes> res(take_res(dev));
+	if (!res) { res.reset(new PipeRes); if (res->init(dev)) { g_err = "pinned staging memory or copy streams could not be allocated"; return LFM_ERR_CUDA; } }
 	const size_t img_bytes = (size_t)max_nf * w->L.fpx * 2;
 	if (w->e->reserve(res->img[0], img_bytes) || w->e->reserve(res->img[1], img_bytes) || (k > 0 && w->e->reserve(res->sym, img_bytes))) {
 		give_res(res.release()); g_err = "batch buffers could not be allocated"; return LFM_ERR_CUDA;
@@ -656,7 +663,7 @@ int writer_append(lfm_stack_writer* w, const void* frames, uint64_t n, bool devi
 	if (!frames) w->fail(LFM_ERR_OPEN, "frames is NULL");
 	else if (device && (rc = check_device_ptr(frames, "d_frames"))) w->fail(rc, g_err);
 	if (int r = w->failed()) { g_err = w->err; return r; }
-	WriterRes& R = *w->res;
+	PipeRes& R = *w->res;
 	cudaSetDevice(R.dev);
 	const size_t frame_bytes = (size_t)w->L.fpx * 2;
 	const uint8_t* src = (const uint8_t*)frames;
@@ -952,9 +959,9 @@ struct PayloadSource {
 	int fd = -1; uint64_t file_off = 0; // or: file descriptor + offset of the payload inside the file
 	uint64_t size = 0;                  // payload bytes available
 	// the payload byte ranges [r.first, r.second) -> device memory, packed one after the other at dst, on stream st.  File sources
-	// go through two pinned staging buffers of the engine: chunk i+1 is read from the file while chunk i crosses PCIe.
-	// Returns 0, or LFM_ERR_BZIP on a short read.
-	int to_device(Engine& e, void* dst, const std::vector<std::pair<uint64_t, uint64_t>>& ranges, cudaStream_t st) const
+	// go through two halves of the pinned staging ring `pin` (kStageBufs * kStageChunk bytes): chunk i+1 is read from the file while
+	// chunk i crosses PCIe.  Returns 0, or LFM_ERR_BZIP on a short read.
+	int to_device(uint8_t* pin, void* dst, const std::vector<std::pair<uint64_t, uint64_t>>& ranges, cudaStream_t st) const
 	{
 		uint64_t dpos = 0;
 		if (base) {
@@ -964,7 +971,6 @@ struct PayloadSource {
 		uint64_t total = 0;
 		for (const auto& r : ranges) total += r.second - r.first;
 		const uint64_t CH = total >= ((uint64_t)64 << 20) ? (uint64_t)16 << 20 : (uint64_t)2 << 20;      // two buffers: 16 MB chunks fit the 32 MB ring
-		uint8_t* pin = (uint8_t*)e.pinned(kStageBufs * kStageChunk, 0);
 		if (!pin) return LFM_ERR_CUDA;
 		cudaEvent_t ev[2]; cudaEventCreateWithFlags(&ev[0], cudaEventDisableTiming); cudaEventCreateWithFlags(&ev[1], cudaEventDisableTiming);
 		int rc = LFM_OK;
@@ -982,114 +988,20 @@ struct PayloadSource {
 			}
 			if (rc) break;
 		}
-		cudaStreamSynchronize(st);                                // the staging buffers are free again (they are shared with the write path)
+		cudaStreamSynchronize(st);                                // the staging buffers are free again
 		cudaEventDestroy(ev[0]); cudaEventDestroy(ev[1]);
 		return rc;
 	}
 };
 
-// Full reads of large stacks on one GPU, the mirror image of the stack writer: while batch b (whole z-slabs) is decoded and
-// un-predicted, the streams of batch b + 1 are read from the file / host memory into the second payload buffer (pinned staging,
-// copy stream 0, own host thread) and the pixels of batch b - 1 travel to the caller's buffer (copy stream 1, own host thread).
-// With out_on_device, `out` is the caller's device buffer: the batches decode straight into it and there is no download stage.
-static int decompress_pipelined(const klb_image_header& h, const Layout& L, const StackDesc& desc, int k, int video,
-                                const PayloadSource& psrc, uint16_t* out, bool out_on_device, uint64_t per)
+// What every read checks of a file's header and table before it decodes anything, in this order; *k, *video: the stored predictor
+// and video bit
+int check_stack(const klb_image_header& h, uint64_t payload_size, int* k, int* video)
 {
-	Engine& e = Engine::for_device(g_set.first_device);
-	cudaSetDevice(e.device());
-	const int dev = e.device();
-	cudaStream_t up_st = (cudaStream_t)e.copy_stream(0), down_st = (cudaStream_t)e.copy_stream(1);
-	const std::vector<uint64_t> cut = batch_cuts(h, L, per, k != 0 && video);
-	const uint64_t nbatch = cut.size() - 1;
-	struct Batch { uint64_t s0, s1, f0, nf, beg, end; };
-	std::vector<Batch> B(nbatch);
-	uint64_t max_nf = 0, max_pay = 0;
-	for (uint64_t b = 0; b < nbatch; b++) {
-		Batch& bt = B[b];
-		bt.s0 = cut[b]; bt.s1 = cut[b + 1];
-		uint64_t f0, f1; slab_frames(h, L, bt.s0, bt.s1, f0, f1);
-		bt.f0 = f0; bt.nf = f1 - f0 + 1;
-		const uint64_t id0 = bt.s0 * L.blocksPerSlab, id1 = bt.s1 * L.blocksPerSlab;
-		bt.beg = id0 ? h.blockOffset[id0 - 1] : 0; bt.end = h.blockOffset[id1 - 1];
-		max_nf = std::max(max_nf, bt.nf); max_pay = std::max(max_pay, bt.end - bt.beg);
-	}
-	const size_t img_bytes = (size_t)max_nf * L.fpx * 2;
-	if (e.reserve(e.user[UB_PAY], max_pay + 16) || e.reserve(e.user[UB_PAY2], max_pay + 16) ||
-	    (!out_on_device && (e.reserve(e.user[UB_IMG], img_bytes) || e.reserve(e.user[UB_IMG2], img_bytes))) ||
-	    (k != 0 && e.reserve(e.user[UB_SYM], img_bytes))) return LFM_ERR_CUDA;
-	if (!e.pinned(kStageBufs * kStageChunk, 0) || !e.pinned(kStageBufs * kStageChunk, 1)) return LFM_ERR_CUDA;
-	uint8_t* dpay[2] = { (uint8_t*)e.user[UB_PAY].p, (uint8_t*)e.user[UB_PAY2].p };
-	uint16_t* dimg[2] = { (uint16_t*)e.user[UB_IMG].p, (uint16_t*)e.user[UB_IMG2].p };
-	uint16_t* dsym = (uint16_t*)e.user[UB_SYM].p;
-	std::thread up_th[2], dn_th[2];
-	int up_rc[2] = { 0, 0 }, dn_rc[2] = { 0, 0 };
-	auto fetch = [&](uint64_t b, int slot) {
-		cudaSetDevice(dev);
-		std::vector<std::pair<uint64_t, uint64_t>> ranges(1, std::make_pair(B[b].beg, B[b].end));
-		up_rc[slot] = psrc.to_device(e, dpay[slot], ranges, up_st);
-		if (cudaStreamSynchronize(up_st) != cudaSuccess) { cudaGetLastError(); up_rc[slot] = LFM_ERR_CUDA; }
-	};
-	auto join_all = [&]() { for (auto& t : up_th) if (t.joinable()) t.join(); for (auto& t : dn_th) if (t.joinable()) t.join(); };
-	int rc = LFM_OK;
-	std::vector<uint64_t> ids, beg, end;
-	const double t0 = now_ms();
-	up_th[0] = std::thread(fetch, 0, 0);
-	for (uint64_t b = 0; b < nbatch && rc == LFM_OK; b++) {
-		const int slot = (int)(b & 1);
-		up_th[slot].join();
-		if ((rc = up_rc[slot])) { if (rc == LFM_ERR_BZIP) std::cerr << "ERROR: lfm_b200: file is truncated" << std::endl; break; }
-		if (b + 1 < nbatch) up_th[slot ^ 1] = std::thread(fetch, b + 1, slot ^ 1);    // its payload buffer was decoded by batch b - 1 (done)
-		if (dn_th[slot].joinable()) { dn_th[slot].join(); if ((rc = dn_rc[slot])) break; }   // image buffer `slot` (batch b - 2) has left
-		const Batch& bt = B[b];
-		const uint64_t id0 = bt.s0 * L.blocksPerSlab, cnt = (bt.s1 - bt.s0) * L.blocksPerSlab;
-		ids.resize(cnt); beg.resize(cnt); end.resize(cnt);
-		for (uint64_t i = 0; i < cnt; i++) {
-			ids[i] = id0 + i;
-			beg[i] = ((id0 + i) ? h.blockOffset[id0 + i - 1] : 0) - bt.beg; end[i] = h.blockOffset[id0 + i] - bt.beg;
-		}
-		uint16_t* res = out_on_device ? out : dimg[slot] - bt.f0 * L.fpx;   // virtual base: absolute frame indexing
-		uint16_t* sym_base = k != 0 ? dsym - bt.f0 * L.fpx : res;
-		DecompressStats st;
-		rc = e.decompress_blocks(dpay[slot], beg.data(), end.data(), ids.data(), cnt, sym_base, desc, &st);
-		if (rc) { g_err = e.last_error(); break; }
-		if (k != 0) {
-			rc = e.unpredict(sym_base, res, desc, k, video, (uint32_t)bt.f0, (uint32_t)bt.nf);
-			st.launches += video ? 2 : 1;
-			if (rc) break;
-			if (cudaStreamSynchronize((cudaStream_t)e.stream()) != cudaSuccess) { cudaGetLastError(); rc = LFM_ERR_CUDA; break; }
-			g_stats.ms_unpredict += e.last_unpredict_ms();
-		}
-		g_stats.ms_decode += st.ms_decode; g_stats.ms_imtf += st.ms_imtf; g_stats.ms_ibwt += st.ms_ibwt; g_stats.ms_unrle += st.ms_unrle;
-		g_stats.gpu_launches += st.launches;
-		if (out_on_device) continue;                                   // the pixels are in place and the engine stream is synchronised
-		const uint16_t* srcp = dimg[slot]; uint16_t* dstp = out + bt.f0 * L.fpx; const size_t nbytes = (size_t)bt.nf * L.fpx * 2;
-		// one download at a time (they share the pinned ring and copy stream 1): batch b - 1 had all of this batch's kernels to finish
-		if (dn_th[slot ^ 1].joinable()) { dn_th[slot ^ 1].join(); if ((rc = dn_rc[slot ^ 1])) break; }
-		dn_th[slot] = std::thread([&, slot, srcp, dstp, nbytes]() {
-			cudaSetDevice(dev);
-			d2h_staged(e, dstp, srcp, nbytes, down_st);
-			if (cudaStreamSynchronize(down_st) != cudaSuccess) { cudaGetLastError(); dn_rc[slot] = LFM_ERR_CUDA; }
-		});
-	}
-	join_all();
-	for (int i = 0; i < 2; i++) { if (!rc && up_rc[i]) rc = up_rc[i]; if (!rc && dn_rc[i]) rc = dn_rc[i]; }
-	g_stats.ms_total = now_ms() - t0;
-	return rc;
-}
-
-// Pixels go to the host buffer `out`, or with a DeviceSink to its device buffer (then `out` is ignored): full reads into a
-// 16-byte aligned buffer decode straight into it; ROI reads, and full reads into any other buffer, decode into the engine's
-// frame buffers and k_roi_gather copies the box out.
-int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16_t* out, const klb_ROI* roi, const DeviceSink* dsink = nullptr)
-{
-	const uint64_t payload_size = psrc.size;
-	memset(&g_stats, 0, sizeof(g_stats));
 	int rc = validate(h, false);
 	if (rc) return rc;
-	const int ndev = current_ndev();
-	if (ndev <= 0) { std::cout << "ERROR: lfm_b200: no CUDA device available (this engine has no CPU fallback)" << std::endl; return LFM_ERR_CUDA; }
+	if (current_ndev() <= 0) { std::cout << "ERROR: lfm_b200: no CUDA device available (this engine has no CPU fallback)" << std::endl; return LFM_ERR_CUDA; }
 	if (h.Nb == 0) { std::cerr << "ERROR: Image to read has not blocks" << std::endl; return LFM_ERR_BZIP; }
-	const int way = current_way();
 	const Layout L = make_layout(h);
 	if (L.Nb != h.Nb) return LFM_ERR_BZIP;
 	if (h.blockOffset[L.Nb - 1] > payload_size) { std::cerr << "ERROR: lfm_b200: file is truncated" << std::endl; return LFM_ERR_BZIP; }
@@ -1097,24 +1009,421 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 	// skips blocks, so checking only the last one is not enough)
 	for (uint64_t i = 1; i < L.Nb; i++)
 		if (h.blockOffset[i] < h.blockOffset[i - 1]) { std::cerr << "ERROR: lfm_b200: corrupt blockOffset table" << std::endl; return LFM_ERR_BZIP; }
-	const StackDesc desc = make_desc(h, way);
-	const int k = h.headerVersion & 0x7F, video = (h.headerVersion & 0x80) ? 1 : 0;
-	if (k > 7) return LFM_ERR_UNSUPPORTED;
-	if (k != 0 && video && way != 0) {
+	*k = h.headerVersion & 0x7F; *video = (h.headerVersion & 0x80) ? 1 : 0;
+	if (*k > 7) return LFM_ERR_UNSUPPORTED;
+	if (*k != 0 && *video && current_way() != 0) {
 		std::cout << "ERROR: lfm_b200: video stack written with predictor way != 0 cannot be inverted (reference defect, see DESIGN.md)" << std::endl;
 		return LFM_ERR_UNSUPPORTED;
 	}
+	return LFM_OK;
+}
+// the inclusive box in_lb..in_ub (NULL: the whole stack) -> lb, ub; LFM_ERR_OPEN when it does not lie inside the stack
+int check_box(const klb_image_header& h, const uint32_t* in_lb, const uint32_t* in_ub, uint32_t lb[5], uint32_t ub[5], bool* full)
+{
+	*full = true;
+	for (int d = 0; d < 5; d++) {
+		lb[d] = in_lb ? in_lb[d] : 0; ub[d] = in_ub ? in_ub[d] : h.xyzct[d] - 1;
+		if (ub[d] >= h.xyzct[d] || lb[d] > ub[d]) return LFM_ERR_OPEN;
+		if (lb[d] != 0 || ub[d] != h.xyzct[d] - 1) *full = false;
+	}
+	return LFM_OK;
+}
+// Block b of a slab (x fastest) is decoded for a read of the box lb..ub.  Without a predictor: the blocks that intersect it.  With
+// a predictor: every operand of the prediction rules lies up and/or left of the pixel (lfm_predict.cuh), so a pixel only depends on
+// the pixels with x' <= x and y' <= y of its frame (and of the previous frame, video) -> the blocks that start at or before the
+// box's lower right corner; what lies right of / below it keeps zero symbols and decodes to values nobody reads.
+bool block_needed(const klb_image_header& h, const Layout& L, uint64_t b, const uint32_t lb[5], const uint32_t ub[5], int k)
+{
+	const uint64_t bx = b % L.nb[0], by = b / L.nb[0];
+	const uint64_t x0 = bx * h.blockSize[0], x1 = std::min<uint64_t>(h.xyzct[0], x0 + h.blockSize[0]) - 1;
+	const uint64_t y0 = by * h.blockSize[1], y1 = std::min<uint64_t>(h.xyzct[1], y0 + h.blockSize[1]) - 1;
+	if (x0 > ub[0] || y0 > ub[1]) return false;
+	return k != 0 || (x1 >= lb[0] && y1 >= lb[1]);
+}
+}  // namespace
+
+// ------------------------------------------------------------------------------------------------ stack reader (one GPU)
+// The read side of the slab pipeline (DESIGN.md §4d): the slabs a box touches are decoded in batches of whole z-slabs (batch_cuts)
+// and handed out frame by frame.  A fetch thread reads the needed byte ranges of batch b + 2 into payload buffer (b + 2) & 1
+// (pinned ring + upload stream), a worker thread decodes and un-predicts batch b + 1 into frame buffer (b + 1) & 1 on the engine
+// under the API lock, and lfmStackReaderRead crops the box out of batch b (k_roi_gather on the download stream) into the caller's
+// device buffer, or into a staging buffer drained to host memory through the download ring.  Everything a reader needs between
+// two calls is its own (PipeRes).  Full reads of large single-GPU stacks go through a reader too (read_with_reader).
+struct lfm_stack_reader {
+	klb_image_header h;
+	Layout L;
+	StackDesc desc;
+	int k = 0, video = 0;
+	bool pair = false;                // video + predictor: an odd frame is predicted from the even frame before it
+	uint32_t lb[5], ub[5];
+	bool full = false;
+	PayloadSource src;
+	int own_fd = -1;                  // the file Open opened, closed by Close
+	uint64_t frames = 0, box_fpx = 0; // frames of the box, pixels of one cropped frame
+	struct Batch { uint64_t s0, s1, f0, f1, u0, u1, i0, i1; };   // slabs [s0, s1) hold frames [f0, f1); [u0, u1) are un-predicted;
+	std::vector<Batch> B;                                        // box frames [i0, i1) come from this batch
+	uint64_t max_box_frames = 0;      // box frames of the largest batch
+	uint16_t* direct = nullptr;       // full read into a 16-byte aligned device buffer: the batches decode straight into it
+	Engine* e = nullptr;
+	PipeRes* res = nullptr;
+	uint64_t pos = 0, cur = 0;        // box frames delivered, batch they come from (calling thread)
+	std::mutex mu;                    // guards the fields below
+	std::condition_variable cv;
+	uint64_t fetched = 0, decoded = 0, delivered = 0;   // batches whose payload is on the GPU / that are decoded / handed out
+	bool closing = false;
+	int rc = LFM_OK;                  // first failure: the reader is failed from then on
+	std::string err;
+	std::vector<uint64_t> ids[2], beg[2], end[2];       // blocks of the batch in payload buffer i (fetch thread -> worker)
+	std::thread fetch_th, worker;
+	lfm_stats st;
+	double t_open = 0;
+
+	int fail(int code, const std::string& what)
+	{
+		std::lock_guard<std::mutex> lk(mu);
+		if (!rc) { rc = code; err = what; }
+		cv.notify_all();
+		return rc;
+	}
+	int failed() { std::lock_guard<std::mutex> lk(mu); return rc; }
+	// box frame i (t slowest, z fastest) -> frame of the stack
+	uint64_t flat(uint64_t i) const
+	{
+		const uint64_t nz = ub[2] - lb[2] + 1, nc = ub[3] - lb[3] + 1;
+		return (lb[2] + i % nz) + (uint64_t)h.xyzct[2] * ((lb[3] + (i / nz) % nc) + (uint64_t)h.xyzct[3] * (lb[4] + i / (nz * nc)));
+	}
+	// box frames whose frame of the stack lies below f
+	uint64_t box_before(uint64_t f) const
+	{
+		const uint64_t Z = h.xyzct[2], C = h.xyzct[3];
+		const uint64_t t = f / (Z * C), c = (f / Z) % C, z = f % Z;
+		const uint64_t nz = ub[2] - lb[2] + 1, nc = ub[3] - lb[3] + 1;
+		auto below = [](uint64_t v, uint32_t a, uint32_t b) { return std::min<uint64_t>(std::max<uint64_t>(v, a), (uint64_t)b + 1) - a; };
+		uint64_t n = below(t, lb[4], ub[4]) * nc * nz;
+		if (t >= lb[4] && t <= ub[4]) {
+			n += below(c, lb[3], ub[3]) * nz;
+			if (c >= lb[3] && c <= ub[3]) n += below(z, lb[2], ub[2]);
+		}
+		return n;
+	}
+	bool touched(uint64_t s) const
+	{
+		const uint64_t bz = s % L.nb[2], c = (s / L.nb[2]) % h.xyzct[3], t = s / ((uint64_t)L.nb[2] * h.xyzct[3]);
+		const uint64_t z0 = bz * h.blockSize[2], z1 = std::min<uint64_t>(h.xyzct[2], z0 + h.blockSize[2]) - 1;
+		return z0 <= ub[2] && z1 >= lb[2] && c >= lb[3] && c <= ub[3] && t >= lb[4] && t <= ub[4];
+	}
+	// slabs decoded: those the box touches, and with pair frames the slab before one whose odd first frame is in the box
+	bool slab_needed(uint64_t s) const
+	{
+		if (touched(s)) return true;
+		if (!pair || s + 1 >= L.nSlabs || !touched(s + 1) || !(slab_first_frame(h, L, s + 1) & 1)) return false;
+		return ((s + 1) % L.nb[2]) * h.blockSize[2] >= lb[2];
+	}
+	void fetch_loop()
+	{
+		cudaSetDevice(res->dev);
+		std::vector<std::pair<uint64_t, uint64_t>> ranges;
+		for (uint64_t b = 0; b < B.size(); b++) {
+			{
+				// payload buffer b & 1 is free once batch b - 2 is decoded
+				std::unique_lock<std::mutex> lk(mu);
+				cv.wait(lk, [&] { return b < 2 || decoded + 1 >= b || closing || rc; });
+				if (closing || rc) return;
+			}
+			const int slot = (int)(b & 1);
+			const double t0 = now_ms();
+			std::vector<uint64_t>& I = ids[slot]; std::vector<uint64_t>& Bg = beg[slot]; std::vector<uint64_t>& E = end[slot];
+			I.clear(); Bg.clear(); E.clear(); ranges.clear();
+			uint64_t packed = 0;                                     // the needed runs of consecutive blocks, packed back to back
+			for (uint64_t s = B[b].s0; s < B[b].s1; s++) {
+				if (!slab_needed(s)) continue;
+				for (uint64_t i = 0; i < L.blocksPerSlab; i++) {
+					if (!block_needed(h, L, i, lb, ub, k)) continue;
+					const uint64_t id = s * L.blocksPerSlab + i, a = id ? h.blockOffset[id - 1] : 0, z = h.blockOffset[id];
+					if (!ranges.empty() && ranges.back().second == a) ranges.back().second = z;
+					else ranges.emplace_back(a, z);
+					I.push_back(id); Bg.push_back(packed); packed += z - a; E.push_back(packed);
+				}
+			}
+			int r = src.to_device(res->up_pin, res->pay[slot].p, ranges, res->up_st);
+			if (!r && cudaStreamSynchronize(res->up_st) != cudaSuccess) { cudaGetLastError(); r = LFM_ERR_CUDA; }
+			if (r) { fail(r, r == LFM_ERR_BZIP ? "file is truncated" : "payload upload failed"); return; }
+			{ std::lock_guard<std::mutex> lk(mu); fetched = b + 1; st.ms_h2d += now_ms() - t0; }
+			cv.notify_all();
+		}
+	}
+	void decode_loop()
+	{
+		cudaSetDevice(res->dev);
+		for (uint64_t b = 0; b < B.size(); b++) {
+			{
+				// frame buffer b & 1 is free once batch b - 2 has been handed out
+				std::unique_lock<std::mutex> lk(mu);
+				cv.wait(lk, [&] { return (fetched > b && (direct || b < 2 || delivered + 1 >= b)) || closing || rc; });
+				if (closing || rc) return;
+			}
+			const int slot = (int)(b & 1);
+			const Batch& bt = B[b];
+			uint16_t* fb = direct ? direct : (uint16_t*)res->img[slot].p - bt.f0 * L.fpx;      // virtual bases: absolute frame indexing
+			uint16_t* sym = k != 0 ? (uint16_t*)res->sym.p - bt.f0 * L.fpx : fb;
+			DecompressStats ds;
+			double ms_unpredict = 0;
+			if (!ids[slot].empty()) {
+				LFM_API_LOCK();
+				cudaSetDevice(e->device());
+				cudaStream_t es = (cudaStream_t)e->stream();
+				if (!full) cudaMemsetAsync(sym + bt.f0 * L.fpx, 0, (bt.f1 - bt.f0) * L.fpx * 2, es);
+				int r = e->decompress_blocks((const uint8_t*)res->pay[slot].p, beg[slot].data(), end[slot].data(), ids[slot].data(),
+				                             ids[slot].size(), sym, desc, &ds);
+				if (r) { fail(r, e->last_error()); return; }
+				if (k != 0 && bt.u1 > bt.u0) {
+					if ((r = e->unpredict(sym, fb, desc, k, video, (uint32_t)bt.u0, (uint32_t)(bt.u1 - bt.u0)))) { fail(r, e->last_error()); return; }
+					ds.launches += video ? 2 : 1;
+				}
+				if (cudaStreamSynchronize(es) != cudaSuccess) { cudaGetLastError(); fail(LFM_ERR_CUDA, "decode failed"); return; }
+				if (k != 0 && bt.u1 > bt.u0) ms_unpredict = e->last_unpredict_ms();
+			}
+			{
+				std::lock_guard<std::mutex> lk(mu);
+				st.ms_decode += ds.ms_decode; st.ms_imtf += ds.ms_imtf; st.ms_ibwt += ds.ms_ibwt; st.ms_unrle += ds.ms_unrle;
+				st.ms_unpredict += ms_unpredict; st.gpu_launches += ds.launches;
+				decoded = b + 1;
+			}
+			cv.notify_all();                                            // payload buffer `slot` is free for batch b + 2
+		}
+	}
+};
+
+namespace {
+// header, table and box checked as readLFMroiDevice checks them, plus what a reader cannot do (c or t blocked); the batches are cut
+int reader_init(std::unique_ptr<lfm_stack_reader>& r, const klb_image_header& h, const PayloadSource& src, const uint32_t* lb, const uint32_t* ub)
+{
+	r.reset(new lfm_stack_reader);
+	r->t_open = now_ms();
+	memset(&r->st, 0, sizeof(r->st));
+	int rc = check_stack(h, src.size, &r->k, &r->video);
+	if (rc) return rc;
+	if ((rc = check_box(h, lb, ub, r->lb, r->ub, &r->full))) return rc;
+	if (h.blockSize[3] != 1 || h.blockSize[4] != 1) {
+		g_err = "blocks over several channels or time points interleave their frames: there is no in-order stream to read"; return LFM_ERR_UNSUPPORTED;
+	}
+	r->h = h;
+	r->src = src;
+	r->L = make_layout(h);
+	r->desc = make_desc(h, current_way());
+	r->pair = r->k != 0 && r->video;
+	r->st.predictor = r->k;
+	const Layout& L = r->L;
+	uint64_t nf = 1;
+	for (int d = 2; d < 5; d++) nf *= (uint64_t)(r->ub[d] - r->lb[d] + 1);
+	r->frames = nf;
+	r->box_fpx = (uint64_t)(r->ub[0] - r->lb[0] + 1) * (r->ub[1] - r->lb[1] + 1);
+	// slabs from the box's first to its last; with pair frames the first batch starts early enough to hold the even frame its
+	// first frame needs
+	const uint64_t C = h.xyzct[3];
+	uint64_t s_begin = ((uint64_t)r->lb[4] * C + r->lb[3]) * L.nb[2] + r->lb[2] / h.blockSize[2];
+	const uint64_t s_end = ((uint64_t)r->ub[4] * C + r->ub[3]) * L.nb[2] + r->ub[2] / h.blockSize[2] + 1;
+	const uint64_t first = r->flat(0), last = r->flat(nf - 1);
+	if (r->pair && (first & 1) && slab_first_frame(h, L, s_begin) == first) s_begin--;
+	const std::vector<uint64_t> cut = batch_cuts(h, L, batch_slabs(h, L), r->pair, s_begin, s_end);
+	const uint64_t u_first = r->pair ? first & ~1ull : first;
+	for (size_t b = 0; b + 1 < cut.size(); b++) {
+		lfm_stack_reader::Batch bt;
+		bt.s0 = cut[b]; bt.s1 = cut[b + 1];
+		bt.f0 = slab_first_frame(h, L, bt.s0); bt.f1 = slab_first_frame(h, L, bt.s1);
+		bt.u0 = std::max(bt.f0, u_first); bt.u1 = std::min(bt.f1, last + 1);
+		bt.i0 = r->box_before(bt.f0); bt.i1 = r->box_before(bt.f1);
+		r->max_box_frames = std::max(r->max_box_frames, bt.i1 - bt.i0);
+		r->B.push_back(bt);
+	}
+	return LFM_OK;
+}
+
+// buffers, resources and the two threads; with `direct` (a full read into an aligned device buffer) no frame buffer is needed
+int reader_start(lfm_stack_reader* r, uint16_t* direct)
+{
+	r->direct = direct;
+	r->e = &Engine::for_device(g_set.first_device);
+	const int dev = r->e->device();
+	cudaSetDevice(dev);
+	std::unique_ptr<PipeRes> res(take_res(dev));
+	if (!res) { res.reset(new PipeRes); if (res->init(dev)) { g_err = "pinned staging memory or copy streams could not be allocated"; return LFM_ERR_CUDA; } }
+	const Layout& L = r->L;
+	const klb_image_header& h = r->h;
+	uint64_t max_nf = 0, max_pay = 0;
+	for (const auto& bt : r->B) {
+		max_nf = std::max(max_nf, bt.f1 - bt.f0);
+		const uint64_t id0 = bt.s0 * L.blocksPerSlab, id1 = bt.s1 * L.blocksPerSlab;
+		max_pay = std::max(max_pay, h.blockOffset[id1 - 1] - (id0 ? h.blockOffset[id0 - 1] : 0));
+	}
+	const size_t img_bytes = (size_t)max_nf * L.fpx * 2;
+	Engine& e = *r->e;
+	if (e.reserve(res->pay[0], max_pay + 16) || e.reserve(res->pay[1], max_pay + 16) ||
+	    (!direct && (e.reserve(res->img[0], img_bytes) || e.reserve(res->img[1], img_bytes))) || (r->k != 0 && e.reserve(res->sym, img_bytes))) {
+		give_res(res.release()); g_err = "batch buffers could not be allocated"; return LFM_ERR_CUDA;
+	}
+	r->res = res.release();
+	try {
+		r->fetch_th = std::thread([r]() { r->fetch_loop(); });
+		r->worker = std::thread([r]() { r->decode_loop(); });
+	} catch (const std::system_error&) {
+		r->fail(LFM_ERR_CREATE, "the reader threads could not be started");
+		if (r->fetch_th.joinable()) r->fetch_th.join();
+		g_err = r->err; return LFM_ERR_CREATE;
+	}
+	return LFM_OK;
+}
+
+// box frames [i, j) of batch b (decoded) -> dst: device memory, or host memory through the staging buffer and the download ring
+int reader_deliver(lfm_stack_reader* r, uint64_t b, uint64_t i, uint64_t j, uint8_t* dst, bool device)
+{
+	PipeRes& R = *r->res;
+	const auto& bt = r->B[b];
+	const Layout& L = r->L;
+	const uint16_t* fb = (const uint16_t*)R.img[b & 1].p - bt.f0 * L.fpx;
+	const size_t bytes = (size_t)(j - i) * r->box_fpx * 2;
+	const bool whole_frames = r->box_fpx == L.fpx;
+	if (!device && whole_frames && r->flat(j - 1) - r->flat(i) == j - 1 - i) {
+		// uncropped frames that follow each other in the frame buffer: straight to the caller
+		d2h_ring(R.down_pin, dst, fb + r->flat(i) * L.fpx, bytes, R.down_st);
+	} else {
+		if (!device && r->e->reserve(R.stage, (size_t)r->max_box_frames * r->box_fpx * 2)) return r->fail(LFM_ERR_CUDA, "staging buffer could not be allocated");
+		uint16_t* to = device ? (uint16_t*)dst : (uint16_t*)R.stage.p;
+		const uint64_t nz = r->ub[2] - r->lb[2] + 1;
+		for (uint64_t u = i; u < j;) {
+			// frames of one channel and time point: one sub-box
+			const uint64_t f = r->flat(u), zoff = u % nz, n = std::min(j - u, nz - zoff);
+			const uint32_t z = (uint32_t)(f % r->h.xyzct[2]), c = (uint32_t)((f / r->h.xyzct[2]) % r->h.xyzct[3]);
+			const uint32_t t = (uint32_t)(f / ((uint64_t)r->h.xyzct[2] * r->h.xyzct[3]));
+			const uint32_t lb[5] = { r->lb[0], r->lb[1], z, c, t }, ub[5] = { r->ub[0], r->ub[1], (uint32_t)(z + n - 1), c, t };
+			if (int rc = r->e->roi_gather(fb, r->desc, lb, ub, to + (u - i) * r->box_fpx, R.down_st)) return r->fail(rc, "k_roi_gather launch failed");
+			{ std::lock_guard<std::mutex> lk(r->mu); r->st.gpu_launches++; }
+			u += n;
+		}
+		if (!device) d2h_ring(R.down_pin, dst, R.stage.p, bytes, R.down_st);
+	}
+	if (cudaStreamSynchronize(R.down_st) != cudaSuccess) { cudaGetLastError(); return r->fail(LFM_ERR_CUDA, "frame delivery failed"); }
+	return LFM_OK;
+}
+
+int reader_read(lfm_stack_reader* r, void* dst, uint64_t n, uint64_t* got, bool device)
+{
+	if (got) *got = 0;
+	if (int c = r->failed()) { g_err = r->err; return c; }
+	if (n == 0) return LFM_OK;
+	int rc = LFM_OK;
+	if (!dst) r->fail(LFM_ERR_OPEN, "dst is NULL");
+	else if (device && (rc = check_device_ptr(dst, "d_dst"))) r->fail(rc, g_err);
+	if (int c = r->failed()) { g_err = r->err; return c; }
+	if (r->pos >= r->frames) return LFM_OK;
+	cudaSetDevice(r->res->dev);
+	const double t0 = now_ms();
+	const uint64_t end = r->pos + std::min(n, r->frames - r->pos);
+	const size_t frame_bytes = (size_t)r->box_fpx * 2;
+	uint64_t i = r->pos;
+	while (i < end) {
+		const auto& bt = r->B[r->cur];
+		{
+			std::unique_lock<std::mutex> lk(r->mu);
+			r->cv.wait(lk, [&] { return r->decoded > r->cur || r->rc; });
+			if (r->rc) break;
+		}
+		const uint64_t j = std::min(end, bt.i1);
+		if (j > i && reader_deliver(r, r->cur, i, j, (uint8_t*)dst + (i - r->pos) * frame_bytes, device)) break;
+		i = j;
+		if (i == bt.i1) {
+			// batch cur is handed out: its frame buffer takes batch cur + 2 (batches without box frames go by as well)
+			do r->cur++; while (r->cur < r->B.size() && r->B[r->cur].i1 == r->B[r->cur].i0);
+			{ std::lock_guard<std::mutex> lk(r->mu); r->delivered = r->cur; }
+			r->cv.notify_all();
+		}
+	}
+	if (!device) { std::lock_guard<std::mutex> lk(r->mu); r->st.ms_d2h += now_ms() - t0; }
+	if (int c = r->failed()) { g_err = r->err; return c; }
+	if (got) *got = i - r->pos;
+	r->pos = i;
+	return LFM_OK;
+}
+
+// stops the threads, frees r; the reader's statistics become the calling thread's
+int reader_close(lfm_stack_reader* r)
+{
+	{ std::lock_guard<std::mutex> lk(r->mu); r->closing = true; }
+	r->cv.notify_all();
+	if (r->fetch_th.joinable()) r->fetch_th.join();
+	if (r->worker.joinable()) r->worker.join();
+	const int rc = r->rc;
+	if (rc) g_err = r->err;
+	if (r->own_fd >= 0) close(r->own_fd);
+	r->st.ms_total = now_ms() - r->t_open;
+	g_stats = r->st;
+	if (r->res) give_res(r->res);
+	delete r;
+	return rc;
+}
+
+// Full reads of large single-GPU stacks take the reader (the pixels of both paths are identical): host memory, or a device buffer
+bool takes_reader(const klb_image_header& h, const klb_ROI* roi, const DeviceSink* dsink)
+{
+	if (validate(h, false) || h.Nb == 0 || h.blockSize[3] != 1 || h.blockSize[4] != 1) return false;   // the other path reports these
+	if (roi) for (int d = 0; d < 5; d++) if (roi->xyzctLB[d] != 0 || roi->xyzctUB[d] != h.xyzct[d] - 1) return false;
+	const int ndev = current_ndev();
+	if (ndev <= 0) return false;
+	const Layout L = make_layout(h);
+	if (!dsink && std::min<uint64_t>((uint64_t)ndev, L.nSlabs) != 1) return false;                       // sharded over several GPUs
+	return slabs_per_batch(h, L) != 0;
+}
+
+// open a reader over the whole stack, read it into `out` (host) or the sink, close.  The batches decode straight into a 16-byte
+// aligned device buffer; anything else receives the frames as a reader's Read hands them out.
+int read_with_reader(const klb_image_header& h, const PayloadSource& src, uint16_t* out, const DeviceSink* dsink)
+{
+	memset(&g_stats, 0, sizeof(g_stats));
+	std::unique_ptr<lfm_stack_reader> up;
+	int rc = reader_init(up, h, src, nullptr, nullptr);
+	if (rc) return rc;
+	if (dsink) {
+		// the caller's buffer is checked before any kernel runs: nothing is written to it unless the whole stack fits
+		const uint64_t bytes = up->frames * up->box_fpx * 2;
+		if (dsink->out_bytes) *dsink->out_bytes = bytes;
+		if ((rc = check_device_ptr(dsink->d_out, "d_out"))) return rc;
+		if (dsink->capacity < bytes) { g_err = "d_out is smaller than the box (" + std::to_string(bytes) + " bytes)"; return LFM_ERR_CREATE; }
+		out = (uint16_t*)dsink->d_out;
+	}
+	const bool direct = dsink && ((uintptr_t)out & 15) == 0;
+	if ((rc = reader_start(up.get(), direct ? out : nullptr))) return rc;
+	lfm_stack_reader* r = up.release();
+	if (direct) {
+		std::unique_lock<std::mutex> lk(r->mu);
+		r->cv.wait(lk, [&] { return r->decoded == r->B.size() || r->rc; });
+	} else {
+		uint64_t got = 0;
+		try { rc = reader_read(r, out, r->frames, &got, dsink != nullptr); }
+		catch (const std::exception&) { rc = r->fail(LFM_ERR_CREATE, "out of host memory"); }   // the reader is closed all the same
+	}
+	const int rc2 = reader_close(r);
+	return rc ? rc : rc2;
+}
+
+// Pixels go to the host buffer `out`, or with a DeviceSink to its device buffer (then `out` is ignored): full reads into a
+// 16-byte aligned buffer decode straight into it; ROI reads, and full reads into any other buffer, decode into the engine's
+// frame buffers and k_roi_gather copies the box out.
+int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16_t* out, const klb_ROI* roi, const DeviceSink* dsink = nullptr)
+{
+	memset(&g_stats, 0, sizeof(g_stats));
+	int k = 0, video = 0;
+	int rc = check_stack(h, psrc.size, &k, &video);
+	if (rc) return rc;
+	const int ndev = current_ndev();
+	const Layout L = make_layout(h);
+	const StackDesc desc = make_desc(h, current_way());
 	const double t_start = now_ms();
 	g_stats.predictor = k;
 
 	// which slabs / blocks are needed
 	uint32_t lb[5], ub[5];
 	bool full = true;
-	for (int d = 0; d < 5; d++) {
-		lb[d] = roi ? roi->xyzctLB[d] : 0; ub[d] = roi ? roi->xyzctUB[d] : h.xyzct[d] - 1;
-		if (ub[d] >= h.xyzct[d] || lb[d] > ub[d]) return LFM_ERR_OPEN;
-		if (lb[d] != 0 || ub[d] != h.xyzct[d] - 1) full = false;
-	}
+	if ((rc = check_box(h, roi ? roi->xyzctLB : nullptr, roi ? roi->xyzctUB : nullptr, lb, ub, &full))) return rc;
 	if (dsink) {
 		// the caller's buffer is checked before any kernel runs: nothing is written to it unless the whole box fits
 		uint64_t bytes = 2;
@@ -1146,10 +1455,6 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 	// aligned as the engine's are: a caller's buffer that is not 16-byte aligned only receives k_roi_gather's copy of the box
 	// (the whole stack for a full read), which handles any alignment.
 	const bool sink_aligned = dsink && ((uintptr_t)dsink->d_out & 15) == 0;
-	if (full && D == 1 && desc.codec == 1 && (!dsink || sink_aligned)) {
-		const uint64_t per = slabs_per_batch(h, L);
-		if (per) return decompress_pipelined(h, L, desc, k, video, psrc, out, dsink != nullptr, per);
-	}
 	const bool direct = dsink && full && sink_aligned;   // decode into the caller's device buffer, no copy at the end
 	const std::vector<uint64_t> cut = shard_cuts(h, L, D, k != 0 && video);
 
@@ -1165,19 +1470,10 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 		for (uint64_t s : my) { uint64_t a, b; slab_frames(h, L, s, s + 1, a, b); f0 = std::min(f0, a); f1 = std::max(f1, b); }
 		if (k != 0 && video && (f0 & 1)) { rcs[d] = LFM_ERR_UNSUPPORTED; return; }   // odd block depth + video across shards
 		const uint64_t nf = f1 - f0 + 1;
-		// block list.  Full read: every block.  ROI without predictor: the blocks that intersect it.  ROI with a predictor: every
-		// operand of the prediction rules lies up and/or left of the pixel (lfm_predict.cuh), so a pixel only depends on the
-		// pixels with x' <= x and y' <= y of its frame (and of the previous frame, video) -> the blocks that start at or before
-		// the ROI's lower right corner; what lies right of / below it keeps zero symbols and decodes to values nobody reads.
+		// block list.  Full read: every block.  ROI: block_needed.
 		std::vector<uint64_t> ids, beg, end;
 		for (uint64_t s : my) for (uint64_t b = 0; b < L.blocksPerSlab; b++) {
-			if (!full) {
-				uint64_t bx = b % L.nb[0], by = b / L.nb[0];
-				uint64_t x0 = bx * h.blockSize[0], x1 = std::min<uint64_t>(h.xyzct[0], x0 + h.blockSize[0]) - 1;
-				uint64_t y0 = by * h.blockSize[1], y1 = std::min<uint64_t>(h.xyzct[1], y0 + h.blockSize[1]) - 1;
-				if (x0 > ub[0] || y0 > ub[1]) continue;
-				if (k == 0 && (x1 < lb[0] || y1 < lb[1])) continue;
-			}
+			if (!full && !block_needed(h, L, b, lb, ub, k)) continue;
 			uint64_t id = s * L.blocksPerSlab + b;
 			ids.push_back(id); beg.push_back(id ? h.blockOffset[id - 1] : 0); end.push_back(h.blockOffset[id]);
 			if (end.back() < beg.back()) { rcs[d] = LFM_ERR_BZIP; return; }
@@ -1199,7 +1495,7 @@ int decompress_core(const klb_image_header& h, const PayloadSource& psrc, uint16
 		    (k != 0 && !direct && e.reserve(e.user[UB_IMG], nf * L.fpx * 2))) { rcs[d] = LFM_ERR_CUDA; return; }
 		struct { void* p; } dpay{ e.user[UB_PAY].p }, dsym{ e.user[UB_SYM].p }, dimg{ e.user[UB_IMG].p };
 		double t0 = now_ms();
-		if ((rcs[d] = psrc.to_device(e, dpay.p, ranges, st))) { if (rcs[d] == LFM_ERR_BZIP) std::cerr << "ERROR: lfm_b200: file is truncated" << std::endl; return; }
+		if ((rcs[d] = psrc.to_device((uint8_t*)e.pinned(kStageBufs * kStageChunk, 0), dpay.p, ranges, st))) { if (rcs[d] == LFM_ERR_BZIP) std::cerr << "ERROR: lfm_b200: file is truncated" << std::endl; return; }
 		if (!full) cudaMemsetAsync(dsym.p, 0, nf * L.fpx * 2, st);
 		h2d[d] = now_ms() - t0;
 		// a direct read covers the whole stack (f0 == 0): the caller's buffer is the frame buffer
@@ -1393,7 +1689,7 @@ try {
 
 int klb_imageIO::readImageFromMemory(const char* fileBytes, size_t fileSize, char* imgOut, const klb_ROI* ROI)
 try {
-	LFM_API_LOCK();
+	DeviceGuard g;
 	if (fileSize < 320) return LFM_ERR_BZIP;
 	header.unpackFixed((const uint8_t*)fileBytes);
 	size_t nb = 0;
@@ -1401,6 +1697,8 @@ try {
 	header.resizeBlockOffset(nb);
 	memcpy(header.blockOffset, fileBytes + 320, header.Nb * 8);
 	PayloadSource ps; ps.base = (const uint8_t*)fileBytes + 320 + header.Nb * 8; ps.size = fileSize - 320 - header.Nb * 8;
+	if (takes_reader(header, ROI, nullptr)) return read_with_reader(header, ps, (uint16_t*)imgOut, nullptr);
+	LFM_API_LOCK();
 	return decompress_core(header, ps, (uint16_t*)imgOut, ROI);
 } LFM_CATCH
 
@@ -1408,7 +1706,7 @@ try {
 static int read_from_file(const std::string& filename, klb_image_header& header, uint16_t* out, const klb_ROI* roi,
                           const DeviceSink* dsink = nullptr)
 try {
-	LFM_API_LOCK();
+	DeviceGuard g;
 	if (filename.empty()) { std::cerr << "ERROR: Filename has not been defined. We cannot read image" << std::endl; return LFM_ERR_OPEN; }
 	if (header.Nb == 0) {
 		int err = header.readHeader(filename.c_str());
@@ -1420,7 +1718,12 @@ try {
 	struct stat sb;
 	PayloadSource ps; ps.fd = fd; ps.file_off = header.getSizeInBytes();
 	ps.size = (fstat(fd, &sb) == 0 && (uint64_t)sb.st_size > ps.file_off) ? (uint64_t)sb.st_size - ps.file_off : 0;
-	const int rc = decompress_core(header, ps, out, roi, dsink);
+	int rc;
+	try {
+		// a reader's worker thread takes the API lock itself: the full reads it serves run without holding it
+		if (takes_reader(header, roi, dsink)) rc = read_with_reader(header, ps, out, dsink);
+		else { LFM_API_LOCK(); rc = decompress_core(header, ps, out, roi, dsink); }
+	} catch (...) { close(fd); throw; }
 	close(fd);
 	return rc;
 } LFM_CATCH
@@ -1517,6 +1820,65 @@ try {
 	if (lb) for (int d = 0; d < 5; d++) { roi.xyzctLB[d] = lb[d]; roi.xyzctUB[d] = ub[d]; }
 	DeviceSink sink; sink.d_out = d_out; sink.capacity = capacity; sink.out_bytes = out_bytes;
 	return read_from_file(std::string(filename), h, nullptr, lb ? &roi : nullptr, &sink);
+} LFM_CATCH
+
+int lfmStackReaderOpen(lfm_stack_reader** r, const char* filename, const uint32_t lb[5], const uint32_t ub[5], uint64_t* frames, uint64_t* frame_bytes)
+try {
+	g_err.clear();
+	if (frames) *frames = 0;
+	if (frame_bytes) *frame_bytes = 0;
+	if (!r) return LFM_ERR_OPEN;
+	*r = nullptr;
+	// the checks of readLFMroiDevice, in its order
+	if (!filename || !*filename || (lb == nullptr) != (ub == nullptr)) return LFM_ERR_OPEN;
+	if (access(filename, R_OK) != 0) { g_err = std::string("cannot open ") + filename; return LFM_ERR_OPEN; }
+	DeviceGuard g;
+	klb_image_header h;
+	int rc = h.readHeader(filename);
+	if (rc > 0) return rc;
+	if (h.Nb == 0) { std::cerr << "ERROR: Image to read has not blocks" << std::endl; return LFM_ERR_BZIP; }
+	const int fd = open(filename, O_RDONLY);
+	if (fd < 0) { g_err = std::string("cannot open ") + filename; return LFM_ERR_OPEN; }
+	struct stat sb;
+	PayloadSource ps; ps.fd = fd; ps.file_off = h.getSizeInBytes();
+	ps.size = (fstat(fd, &sb) == 0 && (uint64_t)sb.st_size > ps.file_off) ? (uint64_t)sb.st_size - ps.file_off : 0;
+	std::unique_ptr<lfm_stack_reader> up;
+	try { rc = reader_init(up, h, ps, lb, ub); } catch (...) { close(fd); throw; }
+	if (!rc) rc = reader_start(up.get(), nullptr);
+	if (rc) { close(fd); return rc; }
+	up->own_fd = fd;
+	if (frames) *frames = up->frames;
+	if (frame_bytes) *frame_bytes = up->box_fpx * 2;
+	*r = up.release();
+	return LFM_OK;
+} LFM_CATCH
+
+int lfmStackReaderRead(lfm_stack_reader* r, void* dst, uint64_t n, uint64_t* got)
+try {
+	g_err.clear();
+	if (got) *got = 0;
+	if (!r) return LFM_ERR_OPEN;
+	DeviceGuard g;
+	try { return reader_read(r, dst, n, got, false); }
+	catch (const std::exception&) { g_err = "out of host memory"; return r->fail(LFM_ERR_CREATE, g_err); }   // fails the reader, as every other error
+} LFM_CATCH
+
+int lfmStackReaderReadDevice(lfm_stack_reader* r, void* d_dst, uint64_t n, uint64_t* got)
+try {
+	g_err.clear();
+	if (got) *got = 0;
+	if (!r) return LFM_ERR_OPEN;
+	DeviceGuard g;
+	try { return reader_read(r, d_dst, n, got, true); }
+	catch (const std::exception&) { g_err = "out of host memory"; return r->fail(LFM_ERR_CREATE, g_err); }   // fails the reader, as every other error
+} LFM_CATCH
+
+int lfmStackReaderClose(lfm_stack_reader* r)
+try {
+	g_err.clear();
+	if (!r) return LFM_ERR_OPEN;
+	DeviceGuard g;
+	return reader_close(r);
 } LFM_CATCH
 
 int readLFMheaderEx(const char* filename, uint8_t* headerVersion, uint8_t* Nnum)
