@@ -11,7 +11,6 @@
 // unresolved set, with the same tile pass.  Exactly periodic blocks keep their ties; rotation 0 is placed last in
 // its group (what bzip2 does for the periods met in practice, SURVEY.md Appendix D.3).
 #include "lfm_radix.cuh"
-#include <cstdlib>
 
 namespace lfm {
 
@@ -26,7 +25,7 @@ extern __shared__ __align__(16) uint8_t bwt_smem[];
 template <int NT>
 __global__ void __launch_bounds__(NT, NT == 1024 ? 1 : 4)
 k_bwt(const uint8_t* __restrict__ txt_all, uint32_t cap, EncJob* __restrict__ jobs, uint32_t njobs,
-      uint8_t* __restrict__ bwt_all, uint32_t* __restrict__ scratch_all, int text_in_smem, int prefix_forced)
+      uint8_t* __restrict__ bwt_all, uint32_t* __restrict__ scratch_all, int text_in_smem)
 {
 	constexpr int BWT_NT = NT;                       // shadows the namespace constant inside this kernel
 	uint32_t* wcnt = reinterpret_cast<uint32_t*>(bwt_smem);
@@ -69,7 +68,8 @@ k_bwt(const uint8_t* __restrict__ txt_all, uint32_t cap, EncJob* __restrict__ jo
 		// ---- phase 1: LSD passes over the rotation prefix (last byte first).  Prefix length: every byte costs a full pass, every
 		// byte less leaves more ties to the doubling phase; measured on light-field residuals (uint16, high bytes mostly 0): 6 bytes
 		// win on 18 KB blocks (c2 stage 0.61 -> 0.51 ms; 5: 0.66, 4: 0.82), 8 bytes on 147 KB blocks (12.1 ms; 6: 12.6, 4: 30.8)
-		const int prefix = prefix_forced ? prefix_forced : (n <= 49152u ? 6 : 8);
+		int prefix = n <= 49152u ? 6 : 8;
+		asm volatile("" : "+r"(prefix));                  // opaque to the optimiser: loops specialised on 6 / 8 spill more in k_bwt<1024>
 		uint32_t* src = nullptr; uint32_t* dst = scr + (size_t)S_SA0 * cap;
 		for (int p = prefix - 1; p >= 0; p--) {
 			if (tid < 256) run[tid] = base[tid];
@@ -189,24 +189,21 @@ size_t bwt_scratch_elems_per_cta(uint32_t cap) { return (size_t)S_COUNT * cap; }
 // resident CTAs per SM of the variant launch_bwt picks for this slot size: 4 (256 threads) when four texts fit shared memory
 int bwt_ctas_per_sm(uint32_t cap, int text_in_smem)
 {
-	static const int forced = getenv("LFM_B200_BWT_NT") ? atoi(getenv("LFM_B200_BWT_NT")) : 0;
-	if (forced == 1024) return 1;
 	return (text_in_smem && bwt_smem_bytes_nt(cap, 1, 256) + 1024 <= (size_t)227 * 1024 / 4) ? 4 : 1;
 }
 
 void launch_bwt(const uint8_t* txt, uint32_t cap, EncJob* jobs, uint32_t njobs, uint8_t* bwt, uint32_t* scratch,
                 int grid, int text_in_smem, cudaStream_t st)
 {
-	static const int prefix = getenv("LFM_B200_BWT_PREFIX") ? std::min(8, std::max(2, atoi(getenv("LFM_B200_BWT_PREFIX")))) : 0;      // 0: by block size
 	if (bwt_ctas_per_sm(cap, text_in_smem) == 4) {
 		const size_t smem = bwt_smem_bytes_nt(cap, text_in_smem, 256);
 		cudaFuncSetAttribute(k_bwt<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-		k_bwt<256><<<grid, 256, smem, st>>>(txt, cap, jobs, njobs, bwt, scratch, text_in_smem, prefix);
+		k_bwt<256><<<grid, 256, smem, st>>>(txt, cap, jobs, njobs, bwt, scratch, text_in_smem);
 		return;
 	}
 	const size_t smem = bwt_smem_bytes_nt(cap, text_in_smem, 1024);
 	cudaFuncSetAttribute(k_bwt<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-	k_bwt<1024><<<grid, 1024, smem, st>>>(txt, cap, jobs, njobs, bwt, scratch, text_in_smem, prefix);
+	k_bwt<1024><<<grid, 1024, smem, st>>>(txt, cap, jobs, njobs, bwt, scratch, text_in_smem);
 }
 
 }  // namespace lfm

@@ -1011,8 +1011,6 @@ constexpr uint32_t IB_MAXS_SMALL = 3072;
 // resident CTAs per SM of the variant launch_inv_bwt picks: 4 (256 threads) for slots of up to 48 KB
 int inv_bwt_ctas_per_sm(uint32_t cap)
 {
-	static const int forced = getenv("LFM_B200_IBWT_NT") ? atoi(getenv("LFM_B200_IBWT_NT")) : 0;
-	if (forced == 1024) return 1;
 	return cap <= 48 * 1024 ? 4 : 1;
 }
 void launch_inv_bwt(const uint8_t* bwt, uint32_t cap, DecJob* jobs, uint32_t njobs, uint32_t* tt_scratch, uint8_t* txt,

@@ -620,7 +620,7 @@ __device__ __forceinline__ void or_bits(uint32_t* out, uint32_t bitpos, uint32_t
 
 __global__ void __launch_bounds__(HP_NT)
 k_huff_pack(const uint16_t* __restrict__ mtfv_all, uint32_t mcap, EncJob* __restrict__ jobs, uint32_t njobs,
-            uint8_t* __restrict__ sel_all, uint32_t selcap, uint8_t* __restrict__ out_all, uint32_t ocap, int level, int spread)
+            uint8_t* __restrict__ sel_all, uint32_t selcap, uint8_t* __restrict__ out_all, uint32_t ocap, int level)
 {
 	__shared__ uint32_t freq[kMaxAlpha + 6];
 	__shared__ uint32_t rfreq[kGroups][kMaxAlpha + 2];
@@ -745,15 +745,11 @@ k_huff_pack(const uint16_t* __restrict__ mtfv_all, uint32_t mcap, EncJob* __rest
 		for (;;) {
 			__syncthreads();
 			if (tid == 0) s_redo = 0;
-			// small grids (latency matters, issue slots are plentiful): one warp per table, no divergence between the tables;
-			// large grids (throughput matters): the tables side by side in the lanes of one warp
-			{
-				const int tb = spread ? (int)wid : (int)lane;                        // the table this lane builds
-				const bool mine = spread ? ((int)wid < ng && lane == 0) : (wid == 0 && (int)lane < ng);
-				if (mine && ((redo >> tb) & 1u)) {
-					if (!(n_mtf < (1u << 17) - 1024u) || !hp_build_tree32(reinterpret_cast<uint32_t*>(hheap[tb]), hparent[tb], hlw[tb], alpha))
-						hp_build_tree(hheap[tb], hparent[tb], hlw[tb], alpha);
-				}
+			// the tables side by side in the lanes of one warp (one warp per table, one active lane each, was measured slower: the
+			// SM becomes issue bound, c2 2.2 ms against 1.0 ms on B200)
+			if (wid == 0 && (int)lane < ng && ((redo >> lane) & 1u)) {
+				if (!(n_mtf < (1u << 17) - 1024u) || !hp_build_tree32(reinterpret_cast<uint32_t*>(hheap[lane]), hparent[lane], hlw[lane], alpha))
+					hp_build_tree(hheap[lane], hparent[lane], hlw[lane], alpha);
 			}
 			__syncthreads();
 			if ((int)wid < ng && ((redo >> wid) & 1u)) {
@@ -1029,10 +1025,7 @@ void launch_huff_pack(const uint16_t* mtfv, uint32_t mcap, EncJob* jobs, uint32_
 {
 	const size_t smem = sizeof(uint64_t) * kGroups * HP_HEAP;
 	cudaFuncSetAttribute(k_huff_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-	// small grids (latency matters, issue slots are plentiful): one warp per table; large grids: the tables in the lanes of one warp
-	static const int forced = getenv("LFM_B200_HP_SPREAD") ? atoi(getenv("LFM_B200_HP_SPREAD")) : -1;
-	const int spread = forced >= 0 ? forced : 0;       // measured on B200: one-lane warps make the SM issue bound (c2: 2.2 ms against 1.0 ms)
-	k_huff_pack<<<njobs, HP_NT, smem, st>>>(mtfv, mcap, jobs, njobs, sel, selcap, out, ocap, level, spread);
+	k_huff_pack<<<njobs, HP_NT, smem, st>>>(mtfv, mcap, jobs, njobs, sel, selcap, out, ocap, level);
 }
 
 }  // namespace lfm

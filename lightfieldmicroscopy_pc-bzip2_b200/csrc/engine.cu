@@ -166,24 +166,7 @@ Engine::Engine(int device) : device_(device)
 	if (cudaGetDeviceProperties(&p, device_) == cudaSuccess) sm_count_ = p.multiProcessorCount;
 	cudaStream_t st; cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
 	stream_ = st;
-	for (int i = 0; i < 5 + kMaxGroups; i++) { cudaEvent_t e; cudaEventCreateWithFlags(&e, i < 4 ? cudaEventDefault : cudaEventDisableTiming); ev_[i] = e; }
-}
-
-void* Engine::aux_stream(int i)
-{
-	while ((int)aux_.size() <= i) { cudaStream_t s2; cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking); aux_.push_back(s2); }
-	return aux_[i];
-}
-
-// Groups a batch of nj KLB blocks is cut into, each running its kernel pipeline on a forked stream so that the stages of
-// different groups overlap.  Measured on B200 (profiles/r1_07): compress +5 % on one 2048^2 frame (484 blocks, 3 groups),
-// +13 % on 968 blocks of 147 KB (4 groups), nothing on decode -- k_bwt's 1024-thread CTAs own a whole SM, so little can
-// run beside them -- and the per-stage event times stop being separable.  Off unless LFM_B200_GROUPS=n asks for it.
-int Engine::groups_for(uint32_t nj) const
-{
-	static const int forced = getenv("LFM_B200_GROUPS") ? atoi(getenv("LFM_B200_GROUPS")) : 0;
-	if (forced <= 1) return 1;
-	return std::min<int>(std::min<int>(forced, kMaxGroups), (int)std::max<uint32_t>(1, nj / (uint32_t)sm_count_));
+	for (auto& ev : ev_) { cudaEvent_t e; cudaEventCreate(&e); ev = e; }
 }
 
 void* Engine::pooled_event(size_t i)
@@ -295,13 +278,11 @@ int Engine::select_mode(const uint16_t* d_frame0, const StackDesc& s, float entr
 	const uint64_t fpx = (uint64_t)W * H;
 	const uint32_t chunk_px = 450000;                                          // klb_imageIO.cpp:2032
 	const uint32_t nchunks = (uint32_t)((fpx + chunk_px - 1) / chunk_px);
-	const uint32_t sstride = round16((uint64_t)chunk_px * 2 + 2);
 	int rc;
 	if ((rc = reserve(sel_cand_, 7 * fpx * 2))) return rc;
-	if ((rc = reserve(sel_sorted_, (size_t)8 * nchunks * sstride))) return rc;
+	if ((rc = reserve(sel_tabs_, select_table_bytes(8, chunk_px, nchunks)))) return rc;
 	if ((rc = reserve(sel_hist_, (size_t)8 * nchunks * 65536 * 4))) return rc;
-	const size_t e_words = ((size_t)8 * nchunks + 63) & ~(size_t)63;                 // entropies, then the sort's per-part digit counts
-	if ((rc = reserve(sel_e_, (e_words + select_scratch_words(8, nchunks)) * 4))) return rc;
+	if ((rc = reserve(sel_e_, (size_t)8 * nchunks * 4))) return rc;
 	const uint16_t* cands[8];
 	cands[0] = d_frame0;
 	for (int k = 1; k < 8; k++) {
@@ -309,7 +290,7 @@ int Engine::select_mode(const uint16_t* d_frame0, const StackDesc& s, float entr
 		launch_predict_fwd(d_frame0, c, W, H, s.Nnum, s.way, k, 0, 0, 1, st);
 		cands[k] = c;
 	}
-	launch_select(cands, 8, fpx, chunk_px, nchunks, (uint8_t*)sel_sorted_.p, sstride, (uint32_t*)sel_hist_.p, (float*)sel_e_.p, (uint32_t*)sel_e_.p + e_words, st);
+	launch_select(cands, 8, fpx, chunk_px, nchunks, (uint16_t*)sel_tabs_.p, (uint32_t*)sel_hist_.p, (float*)sel_e_.p, st);
 	std::vector<float> e((size_t)8 * nchunks);
 	cudaMemcpyAsync(e.data(), sel_e_.p, e.size() * 4, cudaMemcpyDeviceToHost, st);
 	cudaStreamSynchronize(st);
@@ -459,8 +440,7 @@ int Engine::compress_blocks(const uint16_t* d_sym, const StackDesc& s, uint64_t 
 	if ((rc = reserve(mtfv_, BS * (size_t)z.mcap * 2))) return rc;
 	if ((rc = reserve(sel_, BS * (size_t)z.selcap * 2))) return rc;
 	if ((rc = reserve(out_, BS * (size_t)z.ocap + 16))) return rc;
-	const int Gres = groups_for((uint32_t)B);                                  // forked groups need a scratch region each
-	if ((rc = reserve(scratch_, (size_t)Gres * grid * bwt_scratch_elems_per_cta(z.cap) * 4))) return rc;
+	if ((rc = reserve(scratch_, (size_t)grid * bwt_scratch_elems_per_cta(z.cap) * 4))) return rc;
 	if ((rc = reserve(pay, pcap + 16))) return rc;
 	if ((rc = reserve(sizes_, count * 4))) return rc;
 	if ((rc = reserve(offs_, B * 8 + sizeof(Totals)))) return rc;
@@ -468,38 +448,24 @@ int Engine::compress_blocks(const uint16_t* d_sym, const StackDesc& s, uint64_t 
 	cudaMemsetAsync(tot, 0, sizeof(Totals), st);
 
 	std::vector<cudaEvent_t> evs;
+	auto mark = [&]() { if (stt) { cudaEvent_t e = (cudaEvent_t)pooled_event(evs.size()); cudaEventRecord(e, st); evs.push_back(e); } };
 	uint64_t launches = 0;
 	for (uint64_t b0 = 0; b0 < count; b0 += B) {
 		const uint32_t nj = (uint32_t)std::min<uint64_t>(B, count - b0);
 		const uint32_t ns = nj * z.nsub;                                       // job records of this batch
-		// optional (groups_for): the batch cut into G groups whose four-kernel pipelines run on forked streams
-		const int G = groups_for(nj);
-		if (G > 1) cudaEventRecord((cudaEvent_t)ev_[4], st);
-		for (int gi = 0; gi < G; gi++) {
-			const uint32_t j0 = (uint32_t)((uint64_t)nj * gi / G), j1 = (uint32_t)((uint64_t)nj * (gi + 1) / G);
-			const uint32_t gj = j1 - j0, gs = gj * z.nsub;
-			const size_t r0 = (size_t)j0 * z.nsub;                                // first job record of the group
-			cudaStream_t sg = G > 1 ? (cudaStream_t)aux_stream(gi) : st;
-			if (G > 1) cudaStreamWaitEvent(sg, (cudaEvent_t)ev_[4], 0);
-			auto markg = [&]() { if (stt) { cudaEvent_t e = (cudaEvent_t)pooled_event(evs.size()); cudaEventRecord(e, sg); evs.push_back(e); } };
-			EncJob* gjobs = (EncJob*)jobs_.p + r0;
-			uint8_t* gtxt = (uint8_t*)txt_.p + r0 * z.cap; uint8_t* gbwt = (uint8_t*)bwt_.p + r0 * z.cap; uint8_t* grank = (uint8_t*)rank_.p + r0 * z.cap;
-			uint16_t* gmtfv = (uint16_t*)mtfv_.p + r0 * z.mcap;
-			markg();
-			launch_rle1(d_sym, g, first + b0 + j0, gj, gtxt, gbwt, z.cap, z.nsub, (uint32_t)blockBytes, z.nblock_max, gjobs, sg);
-			markg();
-			launch_bwt(gtxt, z.cap, gjobs, gs, gbwt, (uint32_t*)scratch_.p + (size_t)gi * grid * bwt_scratch_elems_per_cta(z.cap),
-			           (int)std::min<uint32_t>(gs, (uint32_t)grid), z.text_in_smem, sg);
-			markg();
-			launch_mtf(gbwt, grank, z.cap, gjobs, gs, gmtfv, z.mcap, sg);
-			markg();
-			launch_huff_pack(gmtfv, z.mcap, gjobs, gs, (uint8_t*)sel_.p + r0 * (size_t)z.selcap * 2, z.selcap, (uint8_t*)out_.p + r0 * z.ocap, z.ocap, z.level, sg);
-			markg();
-			if (G > 1) { cudaEvent_t je = (cudaEvent_t)ev_[5 + gi]; cudaEventRecord(je, sg); cudaStreamWaitEvent(st, je, 0); }
-		}
-		k_offsets<<<1, 1024, 0, st>>>((EncJob*)jobs_.p, nj, z.nsub, tot, (uint64_t*)offs_.p, (uint32_t*)sizes_.p + b0, pcap);
-		k_compact<<<nj, 256, 0, st>>>((uint8_t*)out_.p, z.ocap, (EncJob*)jobs_.p, z.nsub, (uint64_t*)offs_.p, (uint32_t*)sizes_.p + b0, (uint8_t*)pay.p, pcap);
-		launches += 4 * G + 2;
+		EncJob* jobs = (EncJob*)jobs_.p;
+		mark();
+		launch_rle1(d_sym, g, first + b0, nj, (uint8_t*)txt_.p, (uint8_t*)bwt_.p, z.cap, z.nsub, (uint32_t)blockBytes, z.nblock_max, jobs, st);
+		mark();
+		launch_bwt((uint8_t*)txt_.p, z.cap, jobs, ns, (uint8_t*)bwt_.p, (uint32_t*)scratch_.p, (int)std::min<uint32_t>(ns, (uint32_t)grid), z.text_in_smem, st);
+		mark();
+		launch_mtf((uint8_t*)bwt_.p, (uint8_t*)rank_.p, z.cap, jobs, ns, (uint16_t*)mtfv_.p, z.mcap, st);
+		mark();
+		launch_huff_pack((uint16_t*)mtfv_.p, z.mcap, jobs, ns, (uint8_t*)sel_.p, z.selcap, (uint8_t*)out_.p, z.ocap, z.level, st);
+		mark();
+		k_offsets<<<1, 1024, 0, st>>>(jobs, nj, z.nsub, tot, (uint64_t*)offs_.p, (uint32_t*)sizes_.p + b0, pcap);
+		k_compact<<<nj, 256, 0, st>>>((uint8_t*)out_.p, z.ocap, jobs, z.nsub, (uint64_t*)offs_.p, (uint32_t*)sizes_.p + b0, (uint8_t*)pay.p, pcap);
+		launches += 6;
 		last_njobs_ = ns;
 	}
 	last_cap_ = z.cap; last_mcap_ = z.mcap;
@@ -794,7 +760,7 @@ int Engine::decompress_blocks(const uint8_t* d_payload, const uint64_t* begin, c
 	if ((rc = reserve(bwt_, BS * z.cap))) return rc;
 	if ((rc = reserve(txt_, BS * z.cap))) return rc;
 	if ((rc = reserve(mtfv_, BS * (size_t)z.mcap * 2))) return rc;
-	if ((rc = reserve(tt_, (size_t)groups_for((uint32_t)B) * inv_bwt_scratch_elems(grid, z.cap) * 4))) return rc;
+	if ((rc = reserve(tt_, inv_bwt_scratch_elems(grid, z.cap) * 4))) return rc;
 	if ((rc = reserve(dbegin_, count * 8))) return rc;
 	if ((rc = reserve(dend_, count * 8))) return rc;
 	if ((rc = reserve(dids_, count * 8))) return rc;
@@ -804,36 +770,24 @@ int Engine::decompress_blocks(const uint8_t* d_payload, const uint64_t* begin, c
 	cudaMemcpyAsync(dend_.p, end, count * 8, cudaMemcpyHostToDevice, st);
 	cudaMemcpyAsync(dids_.p, block_ids, count * 8, cudaMemcpyHostToDevice, st);
 	std::vector<cudaEvent_t> evs;
+	auto mark = [&]() { if (stt) { cudaEvent_t e = (cudaEvent_t)pooled_event(evs.size()); cudaEventRecord(e, st); evs.push_back(e); } };
 	uint64_t launches = 0;
 	for (uint64_t b0 = 0; b0 < count; b0 += B) {
 		const uint32_t nj = (uint32_t)std::min<uint64_t>(B, count - b0);
-		const int G = groups_for(nj);                                          // see compress_blocks
-		if (G > 1) cudaEventRecord((cudaEvent_t)ev_[4], st);
-		for (int gi = 0; gi < G; gi++) {
-			const uint32_t j0 = (uint32_t)((uint64_t)nj * gi / G), j1 = (uint32_t)((uint64_t)nj * (gi + 1) / G);
-			const uint32_t gj = j1 - j0, gs = gj * z.nsub;
-			const size_t r0 = (size_t)j0 * z.nsub;
-			cudaStream_t sg = G > 1 ? (cudaStream_t)aux_stream(gi) : st;
-			if (G > 1) cudaStreamWaitEvent(sg, (cudaEvent_t)ev_[4], 0);
-			auto markg = [&]() { if (stt) { cudaEvent_t e = (cudaEvent_t)pooled_event(evs.size()); cudaEventRecord(e, sg); evs.push_back(e); } };
-			DecJob* gjobs = (DecJob*)djobs_.p + r0;
-			uint8_t* gtxt = (uint8_t*)txt_.p + r0 * z.cap; uint8_t* gbwt = (uint8_t*)bwt_.p + r0 * z.cap;
-			uint16_t* gmtfv = (uint16_t*)mtfv_.p + r0 * z.mcap;
-			markg();
-			cudaEvent_t mid = nullptr;
-			if (stt) { mid = (cudaEvent_t)pooled_event(evs.size()); evs.push_back(mid); }      // recorded between k_huff_decode and k_imtf
-			if (launch_decode(d_payload, (uint64_t*)dbegin_.p + b0 + j0, (uint64_t*)dend_.p + b0 + j0, gj, z.nsub, gjobs, gmtfv, z.mcap,
-			                  gtxt, gbwt, z.cap, z.selcap, sg, mid)) { err_ = "decoder launch failed"; return LFM_ERR_UNSUPPORTED; }
-			markg();
-			const int ggrid = (int)std::min<uint32_t>(gs, (uint32_t)grid);
-			launch_inv_bwt(gbwt, z.cap, gjobs, gs, (uint32_t*)tt_.p + (size_t)gi * inv_bwt_scratch_elems(grid, z.cap), gtxt, ggrid, sg);
-			markg();
-			launch_unrle(gtxt, gbwt, z.cap, z.nsub, (uint32_t)blockBytes, gjobs, gj, d_sym, g, (uint64_t*)dids_.p + b0 + j0, sg);
-			k_dec_status<<<(gs + 255) / 256, 256, 0, sg>>>(gjobs, gs, flag);
-			markg();
-			if (G > 1) { cudaEvent_t je = (cudaEvent_t)ev_[5 + gi]; cudaEventRecord(je, sg); cudaStreamWaitEvent(st, je, 0); }
-		}
-		launches += 5 * G;
+		const uint32_t ns = nj * z.nsub;                                       // job records of this batch
+		DecJob* jobs = (DecJob*)djobs_.p;
+		mark();
+		cudaEvent_t mid = nullptr;
+		if (stt) { mid = (cudaEvent_t)pooled_event(evs.size()); evs.push_back(mid); }      // recorded between k_huff_decode and k_imtf
+		if (launch_decode(d_payload, (uint64_t*)dbegin_.p + b0, (uint64_t*)dend_.p + b0, nj, z.nsub, jobs, (uint16_t*)mtfv_.p, z.mcap,
+		                  (uint8_t*)txt_.p, (uint8_t*)bwt_.p, z.cap, z.selcap, st, mid)) { err_ = "decoder launch failed"; return LFM_ERR_UNSUPPORTED; }
+		mark();
+		launch_inv_bwt((uint8_t*)bwt_.p, z.cap, jobs, ns, (uint32_t*)tt_.p, (uint8_t*)txt_.p, (int)std::min<uint32_t>(ns, (uint32_t)grid), st);
+		mark();
+		launch_unrle((uint8_t*)txt_.p, (uint8_t*)bwt_.p, z.cap, z.nsub, (uint32_t)blockBytes, jobs, nj, d_sym, g, (uint64_t*)dids_.p + b0, st);
+		k_dec_status<<<(ns + 255) / 256, 256, 0, st>>>(jobs, ns, flag);
+		mark();
+		launches += 5;
 	}
 	uint32_t hflag = 0;
 	cudaMemcpyAsync(&hflag, flag, 4, cudaMemcpyDeviceToHost, st);

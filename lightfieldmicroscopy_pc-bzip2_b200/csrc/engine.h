@@ -125,16 +125,12 @@ private:
 	// workspace
 	Buf jobs_, txt_, bwt_, rank_, mtfv_, sel_, out_, scratch_, payload_, sizes_, offs_;
 	Buf djobs_, dbegin_, dend_, dids_, tt_;
-	Buf sel_sorted_, sel_hist_, sel_e_, sel_cand_;
+	Buf sel_tabs_, sel_hist_, sel_e_, sel_cand_;
 	Buf sz_tiles_, sz_bits_, sz_blocks_, sz_out_, sz_in_;      // bz2_compress: tile records, record-end bitmap, block records, stream, staging
 	Buf dz_in_, dz_cand_, dz_out_;                              // bz2_decompress: padded input, candidate / block records, output
 	uint32_t last_cap_ = 0, last_mcap_ = 0, last_njobs_ = 0;
 	void* pin_[2] = { nullptr, nullptr }; size_t pin_cap_[2] = { 0, 0 };
-	static constexpr int kMaxGroups = 4;   // forked streams a small batch is spread over
-	void* ev_[16] = { nullptr };          // 0-3 predictor timing, 4 fork, 5.. join of every group
-	std::vector<void*> aux_;               // forked streams
-	void* aux_stream(int i);
-	int groups_for(uint32_t nj) const;
+	void* ev_[4] = { nullptr };          // predictor / inverse predictor timing
 	std::vector<void*> ev_pool_;     // stage-timing events, created once and reused (event creation costs host time per call)
 	void* pooled_event(size_t i);
 };

@@ -14,8 +14,8 @@ void launch_roi_gather(const uint16_t* frames, const uint32_t xyzct[5], const ui
                        int sm_count, cudaStream_t st);
 // lfm_select.cu
 void launch_select(const uint16_t* const cand_ptrs[8], int ncand, uint64_t fpx, uint32_t chunk_px, uint32_t nchunks,
-                   uint8_t* sorted, uint32_t sstride, uint32_t* hist, float* e_out, uint32_t* scratch, cudaStream_t st);
-size_t select_scratch_words(int ncand, uint32_t nchunks);
+                   uint16_t* tabs, uint32_t* hist, float* e_out, cudaStream_t st);
+size_t select_table_bytes(int ncand, uint32_t chunk_px, uint32_t nchunks);
 // bz_encode.cu
 void launch_rle1(const uint16_t* sym, const Geom& g, uint64_t first_block, uint32_t njobs, uint8_t* txt, uint8_t* raw_scratch,
                  uint32_t cap, uint32_t nsub, uint32_t max_raw_bytes, uint32_t nblock_max, EncJob* jobs, cudaStream_t st);

@@ -292,11 +292,7 @@ constexpr int kStageBufs = 4;
 // pageable <-> device copies of at least 2 MB are staged: big ones in 8 MB chunks, a single frame in 2 MB chunks so that the
 // host copy of chunk i+1 overlaps the DMA of chunk i
 constexpr size_t kStageMin = (size_t)2 << 20;
-inline size_t stage_chunk(size_t bytes)
-{
-	static const size_t small = (size_t)std::min(8 << 10, std::max(256, env_int("LFM_B200_STAGE_KB", 2 << 10))) << 10;     // test knob
-	return bytes >= ((size_t)64 << 20) ? kStageChunk : small;
-}
+inline size_t stage_chunk(size_t bytes) { return bytes >= ((size_t)64 << 20) ? kStageChunk : kStageMin; }
 
 // pageable source: through `ring` (kStageBufs * kStageChunk pinned bytes); pinned / registered / device memory, or no ring: one copy
 static void h2d_ring(uint8_t* ring, void* dst, const void* src, size_t bytes, cudaStream_t st)
@@ -691,7 +687,7 @@ int writer_append(lfm_stack_writer* w, const void* frames, uint64_t n, bool devi
 			int k = 0;
 			if ((rc = w->e->select_mode((const uint16_t*)R.img[0].p, w->desc, w->st.entropy, &k))) { w->fail(rc, w->e->last_error()); break; }
 			w->st.ms_select = now_ms() - t0;
-			w->st.selected = 1; w->st.gpu_launches += 7 + 5;       // 7 candidate predictions + count, starts, sort, histogram, entropy
+			w->st.selected = 1; w->st.gpu_launches += 7 + 5;       // 7 candidate predictions + the selection (memset, walk, link, entropy: counted as 5, as bench.py does)
 			if (k != 0 && w->video && w->desc.way != 0) {
 				std::cout << "ERROR: lfm_b200: video stacks are only invertible with predictor way 0 (tiles); refusing to write" << std::endl;
 				w->fail(LFM_ERR_UNSUPPORTED, "video stacks are only invertible with predictor way 0"); break;
@@ -855,7 +851,7 @@ int compress_core(const FrameSource& src, klb_image_header& h, std::vector<Shard
 		rc = e.select_mode(f0, desc, g_stats.entropy, &k);
 		if (rc) { g_err = e.last_error(); return rc; }
 		g_stats.ms_select = now_ms() - t0;
-		g_stats.selected = 1; g_stats.gpu_launches += 7 + 5;       // 7 candidate predictions + count, starts, sort, histogram, entropy
+		g_stats.selected = 1; g_stats.gpu_launches += 7 + 5;       // 7 candidate predictions + the selection (memset, walk, link, entropy: counted as 5, as bench.py does)
 	} else {
 		k = hv_in & 0x77 & 0x7F;                       // `hv & 0x7F - 8` parses as hv & 0x77 (src/klb_imageIO.cpp:2380)
 		if (k > 7) { std::cout << "ERROR: The predictors hava not selected!" << std::endl; return LFM_ERR_UNSUPPORTED; }
@@ -1581,11 +1577,10 @@ static int stream_payload_to_fd(std::vector<ShardOut>& shards, int fd, uint64_t 
 		// destination: a shared mapping of this shard's byte range when the file allows it.  write() / pwrite() of one file serialise
 		// on its inode lock (ranks and threads that write disjoint ranges of ONE .lfm file queue up: measured 0.39 -> 1.0 ms per
 		// 4 MB payload with two ranks); stores through a mapping do not, and the copy is split over the pool.
-		static const int mmap_on = env_int("LFM_B200_MMAP_WRITE", 1);
 		const uint64_t fbeg = file_off + off[d], fend = fbeg + bytes;
 		const uint64_t page = (uint64_t)sysconf(_SC_PAGESIZE), mbase = fbeg & ~(page - 1);
 		uint8_t* map = nullptr;
-		if (mmap_on && bytes >= ((uint64_t)256 << 10)) {
+		if (bytes >= ((uint64_t)256 << 10)) {
 			struct stat sb;
 			if (fstat(fd, &sb) == 0 && ((uint64_t)sb.st_size >= fend || posix_fallocate(fd, sb.st_size, (off_t)(fend - (uint64_t)sb.st_size)) == 0)) {
 				void* m = mmap(nullptr, (size_t)(fend - mbase), PROT_READ | PROT_WRITE, MAP_SHARED, fd, (off_t)mbase);

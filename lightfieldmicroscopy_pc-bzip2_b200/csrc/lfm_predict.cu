@@ -10,7 +10,6 @@
 //     of interior tiles), which makes every image column one long chain. Rows then only depend on earlier rows, plus
 //     short left-to-right chains inside the first tile column / the first image row, which one thread walks.
 #include <algorithm>
-#include <cstdlib>
 #include <cooperative_groups.h>
 #include "lfm_device.cuh"
 #include "lfm_predict.cuh"
@@ -209,7 +208,7 @@ constexpr int PF2_NT = PF_NT / 2;
 template <int WAY, int K>
 __global__ void __launch_bounds__(PF2_NT)
 k_predict_fwd2(const uint16_t* __restrict__ img, uint16_t* __restrict__ sym, int W, int H, int T, int video,
-               uint32_t z0, int band, int hw, const __grid_constant__ CUtensorMap tmap, int use_tma)
+               uint32_t z0, int band, int hw, const __grid_constant__ CUtensorMap tmap)
 {
 	extern __shared__ __align__(128) uint8_t pf_smem[];
 	__shared__ __align__(8) uint64_t tile_bar;
@@ -222,30 +221,14 @@ k_predict_fwd2(const uint16_t* __restrict__ img, uint16_t* __restrict__ sym, int
 	const uint16_t* cur = img + (uint64_t)z * fpx;
 	uint16_t* out = sym + (uint64_t)z * fpx;
 	const int ys = y0 - (T + 1), xs = x0 - hw;                   // image coordinates of smem element (0, 0); may be negative
-	const int yc = max(0, ys);
-	const int nrows = y1 - yc;
-	if (use_tma) {
-		// the box of PF_PITCH columns x (band + T + 1) rows at image coordinates (xs, ys) of frame blockIdx.z of this launch
-		if (tid == 0) mbar_init(&tile_bar, 1);
-		__syncthreads();
-		if (tid == 0) {
-			mbar_expect_tx(&tile_bar, (uint32_t)((band + T + 1) * PF_PITCH * 2));
-			tma_load_3d(sm, &tmap, &tile_bar, xs, ys, (int)blockIdx.z);
-		}
-		mbar_wait(&tile_bar, 0);
-	} else {
-		const int cv = tid & 31, rr = tid >> 5;                    // 16-byte column cv (of 32) of rows rr, rr+4, ...
-		const int xv = xs + cv * 8;
-		if (xv >= 0 && xv < W) {
-			const uint32_t gstep = (uint32_t)(W >> 3);
-			const uint4* gp = reinterpret_cast<const uint4*>(cur + (size_t)yc * W + xv) + (uint32_t)rr * gstep;
-			uint32_t dsm = (uint32_t)__cvta_generic_to_shared(sm + (yc - ys) * PF_PITCH + cv * 8) + (uint32_t)rr * (PF_PITCH * 2);
-			for (int r = rr; r < nrows; r += 4, dsm += 4 * PF_PITCH * 2, gp += 4 * gstep)
-				asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(dsm), "l"(gp) : "memory");
-		}
-		asm volatile("cp.async.commit_group;" ::: "memory");
-		asm volatile("cp.async.wait_group 0;" ::: "memory");
+	// the box of PF_PITCH columns x (band + T + 1) rows at image coordinates (xs, ys) of frame blockIdx.z of this launch
+	if (tid == 0) mbar_init(&tile_bar, 1);
+	__syncthreads();
+	if (tid == 0) {
+		mbar_expect_tx(&tile_bar, (uint32_t)((band + T + 1) * PF_PITCH * 2));
+		tma_load_3d(sm, &tmap, &tile_bar, xs, ys, (int)blockIdx.z);
 	}
+	mbar_wait(&tile_bar, 0);
 	__syncthreads();
 	const int sc = 2 * tid;                                      // my first tile column
 	const int x = xs + sc;
@@ -742,7 +725,8 @@ static void launch_tiles_angle(const uint16_t* sym, uint16_t* out, int W, int H,
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Universal shared-memory inverse (any way, predictor, video): one CTA per FRAME walks the frame block by block --
+// Shared-memory inverse of predictor 2 of the ways tiles (incl. video) and angle where k_unpredict_cols2 does not apply (frames of
+// one row, rows wider than its shared memory): one CTA per FRAME walks the frame block by block --
 // a block = one tile row x up to 64 tiles -- in raster order.  Everything a block needs from earlier blocks (T+1 decoded
 // rows above, T+1 decoded columns to the left, the previous frame for odd video frames) is re-read from the output in
 // global memory (written by this CTA, or by the previous launch), so only the block and its halo live in shared memory.
@@ -752,7 +736,7 @@ static void launch_tiles_angle(const uint16_t* sym, uint16_t* out, int W, int H,
 // stacks and videos (hundreds of frames); a single frame is better served by the cluster kernel above.
 constexpr int US_TILES = 64;             // tiles per block
 
-template <int WAY, int K>
+template <int WAY>
 __global__ void __launch_bounds__(1024)
 k_unpredict_strips(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H, int T, int video,
                    uint32_t z_start, uint32_t z_step, int hw, int pitch)
@@ -826,7 +810,7 @@ k_unpredict_strips(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H
 								const int yy = v + dy;
 								return (int)(yy >= 0 ? c[dy * pitch + dx] : prv[(yy + halo) * pitch + hw + xb + dx]);
 							};
-							int p = predict0(px, T, WAY, K, tx, ty, u, v);
+							int p = predict0(px, T, WAY, 2, tx, ty, u, v);
 							if (zflag) { const int P = (int)pfr[v * pitch + hw + xb]; p = (x0 + xb == 0 && y0 + v == 0) ? P : ((p + P) >> 1); }
 							*c = (uint16_t)(unsymbolize16(*c) + p);
 						}
@@ -850,21 +834,18 @@ k_unpredict_strips(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H
 	}
 }
 
+// returns 0 ok, 1 launch error, 2 not applicable
 template <int WAY>
 static int launch_unpredict_strips(const uint16_t* sym, uint16_t* out, int W, int H, int T, int k, int video,
                                    uint32_t z_start, uint32_t z_step, uint32_t count, cudaStream_t st)
 {
+	if (k != 2) return 2;
 	const int hw = (T + 1 + 7) & ~7, pitch = hw + ((US_TILES * T + 7) & ~7);
 	const size_t smem = (size_t)(3 * T + 1) * pitch * 2;
 	if (smem > (size_t)UG_MAX_SMEM) return 2;                   // Nnum too large for this path
 	const unsigned nt = (unsigned)std::min(1024, ((2 * T - 1) * T + 31) & ~31);
-	#define LFM_US(KK) do { cudaFuncSetAttribute(k_unpredict_strips<WAY, KK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-		k_unpredict_strips<WAY, KK><<<count, nt, smem, st>>>(sym, out, W, H, T, video, z_start, z_step, hw, pitch); } while (0)
-	switch (k) {
-	case 1: LFM_US(1); break; case 2: LFM_US(2); break; case 3: LFM_US(3); break; case 4: LFM_US(4); break;
-	case 5: LFM_US(5); break; case 6: LFM_US(6); break; default: LFM_US(7); break;
-	}
-	#undef LFM_US
+	cudaFuncSetAttribute(k_unpredict_strips<WAY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+	k_unpredict_strips<WAY><<<count, nt, smem, st>>>(sym, out, W, H, T, video, z_start, z_step, hw, pitch);
 	return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 
@@ -981,8 +962,7 @@ k_unpredict_cols2(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H,
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Band-pipelined inverse (way "tiles" incl. video; any way whose rule only looks at the operands listed below; not
-// predictor 2 of the ways tiles / angle, whose U crosses the tile border).
+// Band-pipelined inverse (way "tiles" incl. video; not predictor 2, whose U crosses the tile border).
 //
 // A CTA owns a BAND of R tile rows of one frame; thread (j, u, v) owns in-tile position (u, v) of band row j and walks
 // along its tile row: at wavefront step w it decodes tile  tx = w - (u + v + j + 1).  Every operand of the rule function
@@ -1029,7 +1009,7 @@ __device__ __forceinline__ void ub_st_relaxed_gpu(uint32_t* p, uint32_t v)
 }
 __device__ __forceinline__ void ub_fence_gpu() { asm volatile("fence.acq_rel.gpu;" ::: "memory"); }
 
-template <int WAY, int K, int ZF>
+template <int K, int ZF>
 __global__ void __launch_bounds__(1024, 1)   // at most 64 registers: two CTAs of <= 512 threads (or four of 256) share an SM
 k_unpredict_bands(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H, int T,
                   uint32_t z_start, uint32_t z_step, uint32_t count, int R, int ncomp, uint32_t* flags)
@@ -1172,7 +1152,7 @@ k_unpredict_bands(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H,
 					const uint16_t* base = back == 1 ? P1 : P2;
 					return (int)base[(fy ? -TT : 0) + nx + ny * T];
 				};
-				int pr = tx == 0 ? predict0(px, T, WAY, K, 0, tyc, u, v) : predict0(px, T, WAY, K, 1, tyc, u, v);
+				int pr = tx == 0 ? predict0(px, T, 0, K, 0, tyc, u, v) : predict0(px, T, 0, K, 1, tyc, u, v);
 				if (ZF) pr = (tx == 0 && ty == 0 && u == 0 && v == 0) ? (int)(q >> 16) : ((pr + (int)(q >> 16)) >> 1);
 				const uint16_t val = (uint16_t)(unsymbolize16((uint16_t)q) + pr);
 				C[0] = val;
@@ -1271,7 +1251,7 @@ k_unscan_rows(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H, int
 
 constexpr int SC_COLS_NT = 128;
 constexpr int SC_COLS_B = 12;                                             // rows fetched ahead of the running sum
-// thread = (VEC adjacent columns, v): the chain over ty.  VEC = 4 / 2 need W to be a multiple of 4 / 2 (64- / 32-bit accesses).
+// thread = (VEC adjacent columns, v): the chain over ty.  VEC = 2 needs W to be a multiple of 2 (32-bit accesses).
 template <bool SRC_OUT, int VEC>
 __global__ void __launch_bounds__(SC_COLS_NT)
 k_unscan_cols(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H, int T, uint32_t z_start, uint32_t z_step,
@@ -1285,40 +1265,28 @@ k_unscan_cols(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H, int
 	const uint64_t fbase = (uint64_t)z * W * H;
 	const uint16_t* src = (SRC_OUT ? (const uint16_t*)out : sym) + fbase;
 	uint16_t* o = out + fbase;
-	constexpr int NW = VEC == 4 ? 2 : 1;                                    // 32-bit words per thread and row
-	uint32_t acc[NW];
-	#pragma unroll
-	for (int w = 0; w < NW; w++) acc[w] = 0;
+	uint32_t acc = 0;
 	for (int yb = v; yb < H; yb += T * SC_COLS_B) {
-		uint32_t val[SC_COLS_B][NW];
+		uint32_t val[SC_COLS_B];
 		#pragma unroll
 		for (int j = 0; j < SC_COLS_B; j++) {                               // independent loads first: the stores below may alias them
 			const int y = yb + j * T;
-			#pragma unroll
-			for (int w = 0; w < NW; w++) val[j][w] = 0;
+			val[j] = 0;
 			if (y < H) {
 				const size_t at = (size_t)y * W + x;
 				if (VEC == 1) {
 					uint32_t sv = src[at];
 					if (!SRC_OUT) { sv = (uint32_t)unsymbolize16((uint16_t)sv) & 0xffffu; if (y < T && head_rule && (head_rule == 2 || x < T)) sv = o[at]; }
-					val[j][0] = sv;
+					val[j] = sv;
 				} else {
-					uint32_t wv[NW];
-					if (VEC == 4) { const uint2 q = *reinterpret_cast<const uint2*>(src + at); wv[0] = q.x; wv[NW - 1] = q.y; }
-					else wv[0] = *reinterpret_cast<const uint32_t*>(src + at);
-					if (!SRC_OUT) {
-						#pragma unroll
-						for (int w = 0; w < NW; w++) {
-							wv[w] = unsymbolize16x2(wv[w]);
-							if (y < T && head_rule) {                           // heads that are already decoded (per half)
-								const uint32_t ov = *reinterpret_cast<const uint32_t*>(o + at + 2 * w);
-								const bool h0 = head_rule == 2 || x + 2 * w < T, h1 = head_rule == 2 || x + 2 * w + 1 < T;
-								wv[w] = (h0 ? (ov & 0xffffu) : (wv[w] & 0xffffu)) | (h1 ? (ov & 0xffff0000u) : (wv[w] & 0xffff0000u));
-							}
-						}
+					uint32_t wv = *reinterpret_cast<const uint32_t*>(src + at);
+					if (!SRC_OUT) wv = unsymbolize16x2(wv);
+					if (!SRC_OUT && y < T && head_rule) {                   // heads that are already decoded (per half)
+						const uint32_t ov = *reinterpret_cast<const uint32_t*>(o + at);
+						const bool h0 = head_rule == 2 || x < T, h1 = head_rule == 2 || x + 1 < T;
+						wv = (h0 ? (ov & 0xffffu) : (wv & 0xffffu)) | (h1 ? (ov & 0xffff0000u) : (wv & 0xffff0000u));
 					}
-					#pragma unroll
-					for (int w = 0; w < NW; w++) val[j][w] = wv[w];
+					val[j] = wv;
 				}
 			}
 		}
@@ -1327,13 +1295,8 @@ k_unscan_cols(const uint16_t* __restrict__ sym, uint16_t* out, int W, int H, int
 			const int y = yb + j * T;
 			if (y < H) {
 				const size_t at = (size_t)y * W + x;
-				if (VEC == 1) { acc[0] = (acc[0] + val[j][0]) & 0xffffu; o[at] = (uint16_t)acc[0]; }
-				else {
-					#pragma unroll
-					for (int w = 0; w < NW; w++) acc[w] = __vadd2(acc[w], val[j][w]);
-					if (VEC == 4) *reinterpret_cast<uint2*>(o + at) = make_uint2(acc[0], acc[NW - 1]);
-					else *reinterpret_cast<uint32_t*>(o + at) = acc[0];
-				}
+				if (VEC == 1) { acc = (acc + val[j]) & 0xffffu; o[at] = (uint16_t)acc; }
+				else { acc = __vadd2(acc, val[j]); *reinterpret_cast<uint32_t*>(o + at) = acc; }
 			}
 		}
 	}
@@ -1411,8 +1374,7 @@ static int launch_unpredict_space_scans(const uint16_t* sym, uint16_t* out, int 
 	const int pitch = ((W + 7) & ~7) + 16;                               // +8 words: the rows of a CTA start in different banks (the chain threads of one step touch R rows)
 	// rows per CTA: R * T chain threads; small CTAs (R = 8, 128 threads) so that seven of them share an SM and the load, chain and
 	// store phases of different CTAs overlap (R = 16 / 256 threads: 4 per SM, ncu 45 % of the warp slots, DRAM latency exposed)
-	static const int r_forced = getenv("LFM_B200_SCAN_R") ? atoi(getenv("LFM_B200_SCAN_R")) : 0;
-	int R = std::min(r_forced > 0 ? r_forced : 8, (int)((48 * 1024) / ((size_t)pitch * 2)));
+	int R = std::min(8, (int)((48 * 1024) / ((size_t)pitch * 2)));
 	if (R < 1) return 2;                                                   // rows wider than 24 K pixels: the wavefront kernels
 	while (R > 1 && (uint64_t)((H + R - 1) / R) * count < 592) R >>= 1;     // enough CTAs for a single frame
 	const int rnt = R * T > 128 ? 256 : R * T > 64 ? 128 : 64;
@@ -1434,12 +1396,10 @@ static int launch_unpredict_space_scans(const uint16_t* sym, uint16_t* out, int 
 		const int vc = x_limit >= W ? vec : 1;                              // the restricted pass stops at a column that need not be even
 		const int nthr = (xl + vc - 1) / vc;
 		const dim3 grid((unsigned)((nthr + SC_COLS_NT - 1) / SC_COLS_NT), (unsigned)std::min(T, H), n);
-		static const int seg_on = getenv("LFM_B200_SCAN_SEG") ? atoi(getenv("LFM_B200_SCAN_SEG")) : 1;
-		if (vc == 4 && seg_on) {
+		if (vc == 4) {
 			const dim3 g2((unsigned)((W / 4 + 31) / 32), (unsigned)std::min(T, H), n);
 			k_unscan_cols_seg<<<g2, dim3(32, SC_SEG), 0, st>>>(sym, out, W, H, T, zs, z_step, head);
 		}
-		else if (vc == 4) k_unscan_cols<false, 4><<<grid, SC_COLS_NT, 0, st>>>(sym, out, W, H, T, zs, z_step, x_limit, head);
 		else if (vc == 2) k_unscan_cols<false, 2><<<grid, SC_COLS_NT, 0, st>>>(sym, out, W, H, T, zs, z_step, x_limit, head);
 		else k_unscan_cols<false, 1><<<grid, SC_COLS_NT, 0, st>>>(sym, out, W, H, T, zs, z_step, x_limit, head);
 	};
@@ -1477,7 +1437,6 @@ static uint32_t* ub_flags(size_t n)
 }
 
 // returns 0 ok, 1 launch error, 2 shape not supported by this path
-template <int WAY>
 static int launch_unpredict_bands(const uint16_t* sym, uint16_t* out, int W, int H, int T, int k, int zflag,
                                   uint32_t z_start, uint32_t z_step, uint32_t count, cudaStream_t st)
 {
@@ -1485,9 +1444,8 @@ static int launch_unpredict_bands(const uint16_t* sym, uint16_t* out, int W, int
 	int R = 0;
 	while ((((R + 1) * TT + 31) & ~31) + UB_HELPERS <= 1024) R++;
 	if (R == 0) return 2;
-	static const int r_max = getenv("LFM_B200_BANDS_R") ? atoi(getenv("LFM_B200_BANDS_R")) : 1024;
 	const int tilesY = (H + T - 1) / T;
-	R = std::max(1, std::min(std::min(R, r_max), tilesY));
+	R = std::max(1, std::min(R, tilesY));
 	const int ncomp = (R * TT + 31) & ~31;
 	const int nbands = (tilesY + R - 1) / R;
 	const uint64_t nctas = (uint64_t)nbands * count;
@@ -1496,12 +1454,11 @@ static int launch_unpredict_bands(const uint16_t* sym, uint16_t* out, int W, int
 	if (!flags) return 2;
 	cudaMemsetAsync(flags, 0, ((size_t)nctas + 1) * 4, st);
 	const size_t smem = (size_t)4 * ((R + 1) * TT + T + 2) * 2;
-	#define LFM_UB(KK) do { if (zflag) k_unpredict_bands<WAY, KK, 1><<<(unsigned)nctas, ncomp + UB_HELPERS, smem, st>>>(sym, out, W, H, T, z_start, z_step, count, R, ncomp, flags); \
-		else k_unpredict_bands<WAY, KK, 0><<<(unsigned)nctas, ncomp + UB_HELPERS, smem, st>>>(sym, out, W, H, T, z_start, z_step, count, R, ncomp, flags); } while (0)
+	#define LFM_UB(KK) do { if (zflag) k_unpredict_bands<KK, 1><<<(unsigned)nctas, ncomp + UB_HELPERS, smem, st>>>(sym, out, W, H, T, z_start, z_step, count, R, ncomp, flags); \
+		else k_unpredict_bands<KK, 0><<<(unsigned)nctas, ncomp + UB_HELPERS, smem, st>>>(sym, out, W, H, T, z_start, z_step, count, R, ncomp, flags); } while (0)
 	switch (k) {
 	case 1: LFM_UB(1); break; case 3: LFM_UB(3); break; case 4: LFM_UB(4); break;
 	case 5: LFM_UB(5); break; case 6: LFM_UB(6); break; case 7: LFM_UB(7); break;
-	case 2: if (WAY == 2) { LFM_UB(2); break; } return 2;
 	default: return 2;
 	}
 	#undef LFM_UB
@@ -1538,26 +1495,26 @@ static void launch_predict_fwd_wk(const uint16_t* img, uint16_t* sym, int W, int
 	const size_t smem = (size_t)(band + T + 1) * PF_PITCH * 2;
 	if (pairs) cudaFuncSetAttribute(k_predict_fwd2<WAY, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 	else if (tile) cudaFuncSetAttribute(k_predict_fwd<WAY, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-	static const int tma_on = getenv("LFM_B200_TMA") ? atoi(getenv("LFM_B200_TMA")) : 1;
 	for (uint32_t zb = 0; zb < nz; zb += 65535) {            // gridDim.z limit
 		const uint32_t cz = std::min<uint32_t>(65535, nz - zb);
 		dim3 grid((unsigned)colchunks, (unsigned)((H + band - 1) / band), cz);
-		if (pairs) {
-			// tensor map of the cz frames of this launch: uint16 [cz][H][W], box = one tile + halo
-			CUtensorMap tmap; memset(&tmap, 0, sizeof(tmap));
-			int use_tma = 0;
-			if (tma_on && tensor_map_encoder()) {
-				const cuuint64_t gdim[3] = { (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)cz };
-				const cuuint64_t gstr[2] = { (cuuint64_t)W * 2, (cuuint64_t)W * H * 2 };
-				const cuuint32_t box[3] = { (cuuint32_t)PF_PITCH, (cuuint32_t)(band + T + 1), 1u };
-				const cuuint32_t estr[3] = { 1u, 1u, 1u };
-				void* base = const_cast<uint16_t*>(img + (uint64_t)(z0 + zb) * W * H);
-				use_tma = tensor_map_encoder()(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 3, base, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-				                               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-			}
-			k_predict_fwd2<WAY, K><<<grid, PF2_NT, smem, st>>>(img, sym, W, H, T, video, z0 + zb, band, hw, tmap, use_tma);
+		// tensor map of the cz frames of this launch: uint16 [cz][H][W], box = one tile + halo
+		CUtensorMap tmap; memset(&tmap, 0, sizeof(tmap));
+		bool tma = false;
+		if (pairs && tensor_map_encoder()) {
+			const cuuint64_t gdim[3] = { (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)cz };
+			const cuuint64_t gstr[2] = { (cuuint64_t)W * 2, (cuuint64_t)W * H * 2 };
+			const cuuint32_t box[3] = { (cuuint32_t)PF_PITCH, (cuuint32_t)(band + T + 1), 1u };
+			const cuuint32_t estr[3] = { 1u, 1u, 1u };
+			void* base = const_cast<uint16_t*>(img + (uint64_t)(z0 + zb) * W * H);
+			tma = tensor_map_encoder()(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 3, base, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+			                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 		}
-		else if (tile) k_predict_fwd<WAY, K><<<grid, PF_NT, smem, st>>>(img, sym, W, H, T, video, z0 + zb, band, hw);
+		if (tma) k_predict_fwd2<WAY, K><<<grid, PF2_NT, smem, st>>>(img, sym, W, H, T, video, z0 + zb, band, hw, tmap);
+		else if (tile) {                                         // no tensor map (no driver entry point, or the encode failed): the same tile, staged with cp.async
+			if (pairs) cudaFuncSetAttribute(k_predict_fwd<WAY, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+			k_predict_fwd<WAY, K><<<grid, PF_NT, smem, st>>>(img, sym, W, H, T, video, z0 + zb, band, hw);
+		}
 		else k_predict_fwd_rows<WAY, K><<<grid, PF_NT, 0, st>>>(img, sym, W, H, T, video, z0 + zb, band);   // huge Nnum
 	}
 }
@@ -1599,12 +1556,6 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 {
 	(void)sm_count;
 	if (count == 0) return 0;
-	static const int bands_all = getenv("LFM_B200_BANDS") ? atoi(getenv("LFM_B200_BANDS")) : 1;
-	if (bands_all >= 2 && !video && ((way == 1 && k != 2) || way == 2)) {      // measurement switch: every way through the band pipeline
-		const int rcb = way == 1 ? launch_unpredict_bands<1>(sym, out, W, H, T, k, 0, z_start, z_step, count, st)
-		                         : launch_unpredict_bands<2>(sym, out, W, H, T, k, 0, z_start, z_step, count, st);
-		if (rcb != 2) return rcb ? failed_launch("k_unpredict_bands", failed) : 0;
-	}
 	const int tilesX = (W + T - 1) / T, tilesY = (H + T - 1) / T;
 	const unsigned wpb = UF_NT / 32;
 	// sub-images per CTA for the way "space" (neighbours in u share 32-byte sectors): as many as shared memory / 1024 threads allow
@@ -1613,8 +1564,7 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 	int G = std::min(4, T);
 	while (G > 1 && ((size_t)G * plane_b + 16 > (size_t)UG_MAX_SMEM || G * nxr > 1024)) G--;
 	const bool grid_ok = nxr <= 1024 && plane_b + 16 <= (size_t)UG_MAX_SMEM;
-	static const int scans_on = getenv("LFM_B200_SCANS") ? atoi(getenv("LFM_B200_SCANS")) : 1;
-	if (!video && way == 2 && scans_on) {                    // linear rules: strided prefix sums
+	if (!video && way == 2) {                    // linear rules: strided prefix sums
 		const int rcs = launch_unpredict_space_scans(sym, out, W, H, T, k, z_start, z_step, count, st);
 		if (rcs != 2) return rcs ? failed_launch("k_unscan_rows / k_unscan_cols", failed) : 0;
 	}
@@ -1652,24 +1602,19 @@ int launch_unpredict(const uint16_t* sym, uint16_t* out, int W, int H, int T, in
 		return cudaGetLastError() == cudaSuccess ? 0 : failed_launch("k_unpredict_seed / k_unpredict_angle", failed);
 	}
 	// way tiles (image stacks and video), every predictor but 2: the band pipeline
-	static const int bands_on = getenv("LFM_B200_BANDS") ? atoi(getenv("LFM_B200_BANDS")) : 1;
 	// (a single frame is a chain of tilesY / R bands, each ~R + UB_D + 10 steps behind the one above: one or two frames are
 	// served faster by the cluster wavefront below, which puts 8 SMs on every frame)
-	static const int bands_min = getenv("LFM_B200_BANDS_MIN") ? atoi(getenv("LFM_B200_BANDS_MIN")) : 3;
-	if (bands_on && way == 0 && k != 2 && (int)count >= bands_min) {
-		const int rcb = launch_unpredict_bands<0>(sym, out, W, H, T, k, (video && (z_start & 1u)) ? 1 : 0, z_start, z_step, count, st);
+	if (way == 0 && k != 2 && count >= 3) {
+		const int rcb = launch_unpredict_bands(sym, out, W, H, T, k, (video && (z_start & 1u)) ? 1 : 0, z_start, z_step, count, st);
 		if (rcb != 2) return rcb ? failed_launch("k_unpredict_bands", failed) : 0;
 	}
-	// remaining cases (way tiles, video, predictor 2 of tiles/angle): many frames -> one CTA per frame in shared memory;
-	// few frames -> the cluster wavefront below (all SMs on one frame)
-	// predictor 2 of the ways tiles / angle: below the first tile row every image column is an independent chain
-	static const int cols_on = getenv("LFM_B200_COLS") ? atoi(getenv("LFM_B200_COLS")) : 1;
-	const bool cols = cols_on && k == 2 && way != 2 && T <= 32 && H > 1 && (size_t)W * 4 <= (size_t)UG_MAX_SMEM;
-	static const int strips_min = getenv("LFM_B200_STRIPS_MIN") ? atoi(getenv("LFM_B200_STRIPS_MIN")) : 128;
-	if ((int)count >= strips_min && !cols) {
+	// predictor 2 of the ways tiles / angle: below the first tile row every image column is an independent chain.  Where the
+	// column kernel does not apply: many frames -> one CTA per frame in shared memory; few frames, and what the band pipeline
+	// declines -> the cluster wavefront below (all SMs on one frame)
+	const bool cols = k == 2 && way != 2 && T <= 32 && H > 1 && (size_t)W * 4 <= (size_t)UG_MAX_SMEM;
+	if (count >= 128 && !cols) {                             // (ways tiles and angle here: way space has returned above)
 		const int rcs = way == 0 ? launch_unpredict_strips<0>(sym, out, W, H, T, k, video, z_start, z_step, count, st)
-		              : way == 1 ? launch_unpredict_strips<1>(sym, out, W, H, T, k, video, z_start, z_step, count, st)
-		                         : launch_unpredict_strips<2>(sym, out, W, H, T, k, video, z_start, z_step, count, st);
+		                         : launch_unpredict_strips<1>(sym, out, W, H, T, k, video, z_start, z_step, count, st);
 		if (rcs != 2) return rcs ? failed_launch("k_unpredict_strips", failed) : 0;
 	}
 	const uint64_t steps = (k == 2 && way != 2) ? (uint64_t)H : (uint64_t)(tilesX + tilesY + 2 * T);

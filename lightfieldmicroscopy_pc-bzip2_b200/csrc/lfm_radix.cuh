@@ -1,5 +1,5 @@
 // lfm_radix.cuh -- CTA-wide stable 8-bit counting-sort pass and group-splitting helpers shared by the
-// BWT (bz_bwt.cu), the inverse BWT (bz_decode.cu) and the order-1 context sort of the mode selection (lfm_select.cu).
+// BWT (bz_bwt.cu) and the inverse BWT (bz_decode.cu).
 #pragma once
 #include "lfm_device.cuh"
 
@@ -7,7 +7,6 @@ namespace lfm {
 
 constexpr int BWT_NT = 1024;
 constexpr int BWT_R  = 12;                // elements per thread per radix tile (4-byte payloads)
-constexpr int BWT_NW = BWT_NT / 32;
 constexpr int BWT_WS = 257;               // row stride (words) of the per-warp digit counters: conflict-free rows AND columns;
                                           // column 256 is the dummy digit of the lanes past the end of the data
 constexpr int SPLIT_R = 4;                // elements per thread per tile in split_groups
@@ -17,7 +16,7 @@ struct Trip { uint32_t g, r, v; };
 
 // One stable 8-bit counting-sort pass over m elements, tile by tile (tile = BWT_NT * R elements).
 // run[256] (shared) must hold the exclusive bucket starts on entry; it is advanced as tiles are placed.
-// wcnt: BWT_NW x BWT_WS shared words; every warp owns (and zeroes) its own row.
+// wcnt: NT / 32 x BWT_WS shared words; every warp owns (and zeroes) its own row.
 //   1. all loads of the tile are issued first (independent global loads in flight together);
 //   2. ranking inside the warp: R match.any instructions back to back, then R shared-memory atomics by the group
 //      leaders (issued back to back: the counter update is ordered by the memory pipe, not by a register dependency),
@@ -105,9 +104,8 @@ __device__ __forceinline__ void radix_scatter(uint32_t m, uint32_t* run, uint32_
 
 // per-warp private histograms (match.any aggregated) of an 8-bit digit over m elements,
 // reduced and exclusive-scanned into run[256]
-// (SCAN = false: run[] receives the plain digit counts)
-template <bool SCAN, int NT = BWT_NT, class DigitOfIndex>
-__device__ __forceinline__ void digit_hist(uint32_t m, uint32_t* run, uint32_t* wcnt, uint32_t* red, DigitOfIndex dig)
+template <int NT = BWT_NT, class DigitOfIndex>
+__device__ __forceinline__ void digit_starts(uint32_t m, uint32_t* run, uint32_t* wcnt, uint32_t* red, DigitOfIndex dig)
 {
 	const uint32_t lane = lane_id(), w = warp_id();
 	const uint32_t lt = (1u << lane) - 1u;
@@ -133,12 +131,7 @@ __device__ __forceinline__ void digit_hist(uint32_t m, uint32_t* run, uint32_t* 
 		run[threadIdx.x] = s;
 	}
 	__syncthreads();
-	if (SCAN) scan256_excl<NT>(run, red);
-}
-template <int NT = BWT_NT, class DigitOfIndex>
-__device__ __forceinline__ void digit_starts(uint32_t m, uint32_t* run, uint32_t* wcnt, uint32_t* red, DigitOfIndex dig)
-{
-	digit_hist<true, NT>(m, run, wcnt, red, dig);
+	scan256_excl<NT>(run, red);
 }
 
 // Walk cnt sorted entries; entry j is a group head when its 64-bit key differs from the key of entry j-1.

@@ -8,102 +8,11 @@
 //   3. E = sum over bins 0..65534 of -P ln P, P = (float)cnt / (float)n   (bin 65535 is never summed)
 // The integer part is exact; the per-bin terms are fp32 like the reference, summed in a fixed order in fp64
 // (the reference's fp32 thrust::reduce order is unspecified, SURVEY.md Appendix C).
-#include "lfm_radix.cuh"
-#include <cstdlib>
+#include "lfm_device.cuh"
 
 namespace lfm {
 
 struct CandPtrs { const uint16_t* p[8]; };
-
-// The stable sort of one (candidate, chunk) is spread over SEL_P CTAs (80 sorts would leave half of the 148 SMs idle and
-// walk 74 tiles each): part p owns a contiguous range of whole tiles of the pair list;
-//   k_select_count    digit histogram of every part
-//   k_select_starts   bucket start of every (part, digit): all smaller digits, then the same digit of the earlier parts
-//   k_select_sort     the counting-sort pass of the part from those starts (stable across parts: ranges are contiguous)
-constexpr int SEL_P = 8;
-__device__ __forceinline__ void sel_part_range(uint32_t m, uint32_t part, uint32_t& r0, uint32_t& r1)
-{
-	constexpr uint32_t TILE = BWT_NT * BWT_R;
-	const uint32_t tiles = (m + TILE - 1) / TILE, per = (tiles + SEL_P - 1) / SEL_P;
-	r0 = min(m, part * per * TILE); r1 = min(m, (part + 1) * per * TILE);
-}
-
-__global__ void __launch_bounds__(BWT_NT, 1)
-k_select_count(CandPtrs cands, uint64_t fpx, uint32_t chunk_px, uint32_t nchunks, uint32_t* __restrict__ counts)
-{
-	__shared__ uint32_t wcnt[BWT_NW * BWT_WS];
-	__shared__ uint32_t run[256];
-	__shared__ uint32_t red[64];
-	const uint32_t part = blockIdx.x, chunk = blockIdx.y, cand = blockIdx.z;
-	const uint64_t px0 = (uint64_t)chunk * chunk_px;
-	const uint32_t n = (uint32_t)(min((uint64_t)chunk_px, fpx - px0) * 2);
-	const uint8_t* b = reinterpret_cast<const uint8_t*>(cands.p[cand] + px0);
-	uint32_t r0, r1; sel_part_range(n + 1, part, r0, r1);
-	digit_hist<false>(r1 - r0, run, wcnt, red, [&](uint32_t e) { return r0 + e < n ? (uint32_t)b[r0 + e] : 0u; });
-	if (threadIdx.x < 256) counts[(((size_t)cand * nchunks + chunk) * SEL_P + part) * 256 + threadIdx.x] = run[threadIdx.x];
-}
-
-__global__ void __launch_bounds__(256)
-k_select_starts(uint32_t* __restrict__ counts /* in: counts, out: starts */)
-{
-	__shared__ uint32_t red[64];
-	uint32_t* c = counts + (size_t)blockIdx.x * SEL_P * 256;          // [SEL_P][256] of one (candidate, chunk)
-	const uint32_t d = threadIdx.x;
-	uint32_t v[SEL_P], tot = 0;
-	#pragma unroll
-	for (int p = 0; p < SEL_P; p++) { v[p] = c[p * 256 + d]; tot += v[p]; }
-	uint32_t all; const uint32_t incl = block_scan_add<256>(tot, red, &all);
-	uint32_t acc = incl - tot;                                       // elements with a smaller digit
-	#pragma unroll
-	for (int p = 0; p < SEL_P; p++) { c[p * 256 + d] = acc; acc += v[p]; }
-}
-
-__global__ void __launch_bounds__(BWT_NT, 1)
-k_select_sort(CandPtrs cands, uint64_t fpx, uint32_t chunk_px, uint32_t nchunks, uint8_t* __restrict__ sorted_all,
-              uint32_t sstride, const uint32_t* __restrict__ starts)
-{
-	__shared__ uint32_t wcnt[BWT_NW * BWT_WS];
-	__shared__ uint32_t run[256];
-	const uint32_t part = blockIdx.x, chunk = blockIdx.y, cand = blockIdx.z;
-	const uint64_t px0 = (uint64_t)chunk * chunk_px;
-	const uint32_t n = (uint32_t)(min((uint64_t)chunk_px, fpx - px0) * 2);
-	const uint8_t* b = reinterpret_cast<const uint8_t*>(cands.p[cand] + px0);
-	uint8_t* dst = sorted_all + ((size_t)cand * nchunks + chunk) * sstride;
-	uint32_t r0, r1; sel_part_range(n + 1, part, r0, r1);
-	if (threadIdx.x < 256) run[threadIdx.x] = starts[(((size_t)cand * nchunks + chunk) * SEL_P + part) * 256 + threadIdx.x];
-	auto pair_of = [&](uint32_t e0) -> uint32_t {
-		const uint32_t e = r0 + e0;
-		if (e < n) return ((uint32_t)b[e] << 8) | (e ? (uint32_t)b[e - 1] : 0u);
-		return (uint32_t)b[n - 1];                      // key 0
-	};
-	radix_scatter<BWT_R, uint32_t>(r1 - r0, run, wcnt, pair_of,
-		[&](uint32_t p) { return p >> 8; },
-		[&](uint32_t pos, uint32_t p) { dst[pos] = (uint8_t)p; });
-}
-
-constexpr int SH_NT = 256;
-__global__ void __launch_bounds__(SH_NT)
-k_select_hist(const uint8_t* __restrict__ sorted_all, uint32_t sstride, uint64_t fpx, uint32_t chunk_px,
-              uint32_t nchunks, uint32_t* __restrict__ hist_all)
-{
-	const uint32_t cc = blockIdx.y;                       // cand * nchunks + chunk
-	const uint32_t chunk = cc % nchunks;
-	const uint64_t px0 = (uint64_t)chunk * chunk_px;
-	const uint32_t n = (uint32_t)(min((uint64_t)chunk_px, fpx - px0) * 2);
-	const uint8_t* S = sorted_all + (size_t)cc * sstride;
-	uint32_t* hist = hist_all + (size_t)cc * 65536;
-	const uint32_t lane = lane_id();
-	for (uint32_t x0 = blockIdx.x * SH_NT; x0 < n; x0 += gridDim.x * SH_NT) {
-		uint32_t x = x0 + threadIdx.x;
-		bool act = x < n;
-		uint32_t amask = __ballot_sync(0xffffffffu, act);
-		if (act) {
-			uint32_t key = ((uint32_t)S[x] << 8) | S[x + 1];
-			uint32_t peers = __match_any_sync(amask, key);
-			if (lane == (uint32_t)(__ffs(peers) - 1)) atomicAdd(&hist[key], (uint32_t)__popc(peers));
-		}
-	}
-}
 
 constexpr int SE_NT = 1024;
 __global__ void __launch_bounds__(SE_NT)
@@ -148,12 +57,12 @@ constexpr int SN_PARTS = 8;                       // CTAs per (candidate, chunk)
 constexpr uint32_t SN_HOT = 32;                   // pairs whose first byte is below this are counted in shared memory
 constexpr uint16_t SN_NONE = 0xFFFFu;
 // ncu of the first version (one match.any for the key, one to aggregate equal pairs before the global atomic): MIO bound, 24 % of
-// the issue slots.  Now ONE match.any (the key peers; eight ballots were measured slower), and the pairs whose first byte is small -- high bytes and small
+// the issue slots.  Now ONE match.any (the key peers; eight ballots were measured slower: 0.78 against 0.70 ms), and the pairs whose first byte is small -- high bytes and small
 // residuals: most of them, and the ones that would contend for the same global counter -- go to a 32 x 256 shared-memory
 // histogram that the CTA adds to the global one once, after ~55 segments; the others are spread over 57 K counters.
 __global__ void __launch_bounds__(32 * SN_WARPS)
 k_select_next(CandPtrs cands, uint64_t fpx, uint32_t chunk_px, uint32_t nchunks, uint16_t* __restrict__ tabs_all, uint32_t tstride,
-              uint32_t* __restrict__ hist_all, int use_match)
+              uint32_t* __restrict__ hist_all)
 {
 	extern __shared__ __align__(16) uint8_t sn_smem[];
 	uint32_t* hot = reinterpret_cast<uint32_t*>(sn_smem);                            // [SN_HOT][256]
@@ -192,15 +101,7 @@ k_select_next(CandPtrs cands, uint64_t fpx, uint32_t chunk_px, uint32_t nchunks,
 			const uint32_t am = __ballot_sync(0xffffffffu, act);
 			uint32_t key = 0, val = 0;
 			if (act) { key = sb[(int)(j - j0)]; val = sb[(int)(j - j0) - 1]; }         // position n holds key 0 (staged as 0), b[-1] = 0
-			uint32_t peers = am;                                                     // lanes with the same key
-			if (use_match) peers = __match_any_sync(0xffffffffu, act ? key : 256u) & am;
-			else {
-				#pragma unroll
-				for (int bit = 0; bit < 8; bit++) {
-					const uint32_t bm = __ballot_sync(0xffffffffu, (key >> bit) & 1u);
-					peers &= ((key >> bit) & 1u) ? bm : ~bm;
-				}
-			}
+			const uint32_t peers = __match_any_sync(0xffffffffu, act ? key : 256u) & am;   // lanes with the same key
 			const uint32_t higher = peers & ~lt_incl;
 			const uint32_t partner = (act && higher) ? (uint32_t)__ffs((int)higher) - 1u : lane;
 			uint32_t pv = __shfl_sync(0xffffffffu, val, partner);
@@ -279,30 +180,20 @@ k_select_link(const uint16_t* __restrict__ tabs_all, uint32_t tstride, uint64_t 
 	}
 }
 
-// sorted: ncand*nchunks*sstride bytes; hist: ncand*nchunks*65536 uint32 (zeroed here); e_out: ncand*nchunks floats;
-// scratch: select_scratch_words() uint32
-size_t select_scratch_words(int ncand, uint32_t nchunks) { return (size_t)ncand * nchunks * SEL_P * 256; }
+// tabs: select_table_bytes(); hist: ncand*nchunks*65536 uint32 (zeroed here); e_out: ncand*nchunks floats
+static uint32_t select_segments(uint32_t chunk_px) { return (chunk_px * 2 + 1 + SN_SEG - 1) / SN_SEG; }
+size_t select_table_bytes(int ncand, uint32_t chunk_px, uint32_t nchunks) { return (size_t)ncand * nchunks * select_segments(chunk_px) * 1024; }
 void launch_select(const uint16_t* const cand_ptrs[8], int ncand, uint64_t fpx, uint32_t chunk_px, uint32_t nchunks,
-                   uint8_t* sorted, uint32_t sstride, uint32_t* hist, float* e_out, uint32_t* scratch, cudaStream_t st)
+                   uint16_t* tabs, uint32_t* hist, float* e_out, cudaStream_t st)
 {
 	CandPtrs cp;
 	for (int i = 0; i < 8; i++) cp.p[i] = cand_ptrs[i < ncand ? i : 0];
 	cudaMemsetAsync(hist, 0, (size_t)ncand * nchunks * 65536 * sizeof(uint32_t), st);
-	static const int sorted_path = getenv("LFM_B200_SELECT_SORT") ? atoi(getenv("LFM_B200_SELECT_SORT")) : 0;
-	const uint32_t max_seg = (chunk_px * 2 + 1 + SN_SEG - 1) / SN_SEG;
-	if (!sorted_path && (size_t)max_seg * 1024 <= (size_t)sstride) {                   // the segment tables live in the (unused) sort buffer
-		const uint32_t tstride = sstride / 2;                                           // uint16 elements per (candidate, chunk)
-		static const int use_match = getenv("LFM_B200_SELECT_MATCH") ? atoi(getenv("LFM_B200_SELECT_MATCH")) : 1;      // 0: eight ballots instead of one match.any (measured 0.78 against 0.70 ms)
-		const size_t sn_smem = (size_t)SN_HOT * 256 * 4 + (size_t)SN_WARPS * 256 * 2 + (size_t)SN_WARPS * (16 + SN_SEG);
-		cudaFuncSetAttribute(k_select_next, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sn_smem);
-		k_select_next<<<dim3(SN_PARTS, nchunks, ncand), 32 * SN_WARPS, sn_smem, st>>>(cp, fpx, chunk_px, nchunks, reinterpret_cast<uint16_t*>(sorted), tstride, hist, use_match);
-		k_select_link<<<ncand * nchunks, 256 * SL_Q, 0, st>>>(reinterpret_cast<const uint16_t*>(sorted), tstride, fpx, chunk_px, nchunks, hist);
-	} else {
-		k_select_count<<<dim3(SEL_P, nchunks, ncand), BWT_NT, 0, st>>>(cp, fpx, chunk_px, nchunks, scratch);
-		k_select_starts<<<ncand * nchunks, 256, 0, st>>>(scratch);
-		k_select_sort<<<dim3(SEL_P, nchunks, ncand), BWT_NT, 0, st>>>(cp, fpx, chunk_px, nchunks, sorted, sstride, scratch);
-		k_select_hist<<<dim3(32, ncand * nchunks), SH_NT, 0, st>>>(sorted, sstride, fpx, chunk_px, nchunks, hist);
-	}
+	const uint32_t tstride = select_segments(chunk_px) * 512;                          // uint16 elements per (candidate, chunk)
+	const size_t sn_smem = (size_t)SN_HOT * 256 * 4 + (size_t)SN_WARPS * 256 * 2 + (size_t)SN_WARPS * (16 + SN_SEG);
+	cudaFuncSetAttribute(k_select_next, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sn_smem);
+	k_select_next<<<dim3(SN_PARTS, nchunks, ncand), 32 * SN_WARPS, sn_smem, st>>>(cp, fpx, chunk_px, nchunks, tabs, tstride, hist);
+	k_select_link<<<ncand * nchunks, 256 * SL_Q, 0, st>>>(tabs, tstride, fpx, chunk_px, nchunks, hist);
 	k_select_entropy<<<ncand * nchunks, SE_NT, 0, st>>>(hist, fpx, chunk_px, nchunks, e_out);
 }
 

@@ -14,10 +14,11 @@ libbz2 must reject are rejected, and each forged stream has the property its row
 blocks (raw pixels, header_version 8) are re-encoded by the forge; they read back through oracle.read.
 
 On the GPU every row goes through bz2_decompress (k_huff_decode<*, true>, k_unrle_flat) and every KLB row through read_stack
-on the host and into device memory (k_huff_decode<*, false>, k_unrle).  The switches LFM_B200_DEC_LB, LFM_B200_IBWT_NT and
-LFM_B200_GROUPS are read once per process, so each group of rows runs in a fresh child process with every inherited
-LFM_B200_* variable removed, at most once per test session.  One torch.profiler capture per row must list the kernel
-variant the row is for, and not the one a fall-back row exists to avoid.
+on the host and into device memory (k_huff_decode<*, false>, k_unrle).  The dispatcher picks 9- or 10-bit Huffman tables by
+launch size; LFM_B200_DEC_LB forces one width, so that every stream runs through both.  It is read once per process, so
+each group of rows runs in a fresh child process with every inherited LFM_B200_* variable removed, at most once per test
+session.  One torch.profiler capture per row must list the kernel variant the row is for, and not the one a fall-back row
+exists to avoid.
 """
 import bz2
 import heapq
@@ -603,7 +604,7 @@ BY_NAME["concatenated_levels"] = ROWS[-1]
 class KlbRow:
     def __init__(self, name, img, bs, opts, small=False, many=False):
         self.name, self.img, self.bs, self.opts = name, img, bs, opts   # bs: (x, y, z) block size
-        self.small = small                  # slots of <= 48 KB: k_inv_bwt<256> unless LFM_B200_IBWT_NT=1024
+        self.small = small                  # slots of <= 48 KB: k_inv_bwt<256>
         self.many = many                    # more blocks than 10-bit tables keep resident: k_huff_decode<9, false>
 
 
@@ -737,10 +738,7 @@ GROUPS = {
     "default": {},
     "dec_lb9": {"LFM_B200_DEC_LB": "9"},
     "dec_lb10": {"LFM_B200_DEC_LB": "10"},
-    "ibwt_nt1024": {"LFM_B200_IBWT_NT": "1024"},
-    "groups4": {"LFM_B200_GROUPS": "4"},
 }
-STANDALONE_GROUPS = ("default", "dec_lb9", "dec_lb10", "ibwt_nt1024")
 
 
 def expected_kernels(group, row):
@@ -753,9 +751,8 @@ def expected_kernels(group, row):
         if not row.reject:
             must += ["k_inv_bwt<1024>", "k_unrle_flat"]
         return must, ["k_huff_decode<%d, true>" % (19 - lb), "k_huff_decode<10, false>", "k_huff_decode<9, false>"]
-    # LFM_B200_GROUPS=4 splits the 2400 blocks into launches of 600, which 10-bit tables keep resident
-    lb = 9 if forced == "9" or (forced != "10" and row.many and group != "groups4") else 10
-    nt = 256 if row.small and env.get("LFM_B200_IBWT_NT") != "1024" else 1024
+    lb = 9 if forced == "9" or (forced != "10" and row.many) else 10
+    nt = 256 if row.small else 1024
     return (["k_huff_decode<%d, false>" % lb, "k_inv_bwt<%d>" % nt, "k_unrle<", "k_imtf"],
             ["k_huff_decode<%d, false>" % (19 - lb), "k_inv_bwt<%d>" % (1280 - nt), "true>"])
 
@@ -855,9 +852,8 @@ def _child(args, env_extra, timeout):
     return json.loads(lines[-1][len("RESULT "):])
 
 
-def _names(group):
-    klb = [r.name for r in KLB_ROWS] + ["write_stack_const300_hv8"]
-    return klb if group == "groups4" else [r.name for r in ROWS] + klb
+def _names():
+    return [r.name for r in ROWS] + [r.name for r in KLB_ROWS] + ["write_stack_const300_hv8"]
 
 
 @pytest.fixture(scope="session")
@@ -877,14 +873,14 @@ def row_cache(tmp_path_factory):
 
 def _group_results(row_cache, group):
     if group not in _results:
-        _results[group] = _child([row_cache] + _names(group), GROUPS[group], timeout=1200)
+        _results[group] = _child([row_cache] + _names(), GROUPS[group], timeout=1200)
     res = _results[group]
     if isinstance(res, str):
         pytest.fail(res)
     return res
 
 
-GPU_CASES = [(g, n) for g in GROUPS for n in _names(g)]
+GPU_CASES = [(g, n) for g in GROUPS for n in _names()]
 
 
 @pytest.mark.gpu

@@ -1,8 +1,8 @@
 """Every forward and inverse predictor kernel that launch_predict_fwd / launch_unpredict (csrc/lfm_predict.cu) can choose,
 run at a shape that chooses it and checked against the oracle's plain C statement of the prediction rules.
 
-A row of ROWS names a stack (frames x H x W, Nnum), a way, its predictors, image and / or video mode, the byte offsets of
-the device buffers (views into a larger tensor) and the run-time switches it needs.  For each row, through
+A row of ROWS names a stack (frames x H x W, Nnum), a way, its predictors, image and / or video mode and the byte offsets of
+the device buffers (views into a larger tensor).  For each row, through
 lfmDebugPredictDevice:
   * forward: the GPU's symbols equal oracle.predict_frame for every frame (odd video frames: prev = the frame before);
   * inverse: from the ORACLE's symbols, into a buffer filled with a sentinel, the GPU gives the stack back exactly, and so
@@ -13,9 +13,8 @@ lfmDebugPredictDevice:
 Stacks of more than 65535 frames repeat a few distinct frames with a period that does not divide 65536, so every frame is
 checked while the oracle only predicts one period; a kernel that reads the wrong frame index still fails.
 
-The switches are read once per process, on first use.  So every group of rows with the same switches runs in a fresh
-child process, from which every inherited LFM_B200_* variable is removed: a setting left behind by an earlier test in the
-same process cannot change which kernel a row reaches.
+The rows run in a fresh child process, from which every inherited LFM_B200_* variable is removed, with decode buffers
+poisoned (LFM_B200_DEBUG_POISON) so that a wrong wavefront order cannot hide behind stale data.
 """
 import ctypes as C
 import json
@@ -35,10 +34,9 @@ SENTINEL = -21555                # 0xABCD
 
 
 class Row:
-    def __init__(self, name, way, ks, shape, T, video=(0,), off=(0, 0), env=None, fwd=(), not_fwd=(), inv=(), not_inv=()):
+    def __init__(self, name, way, ks, shape, T, video=(0,), off=(0, 0), fwd=(), not_fwd=(), inv=(), not_inv=()):
         self.name, self.way, self.ks, self.shape, self.T, self.video = name, way, tuple(ks), shape, T, tuple(video)
         self.off = off                  # byte offsets of the source and the destination view of each call
-        self.env = dict(env or {})
         # fwd / inv: kernels that must run in the capture of EVERY (predictor, video mode) of the row -- an entry (pattern, ks)
         # only for those predictors; not_fwd / not_inv: kernels that must run in none of them
         self.fwd, self.not_fwd, self.inv, self.not_inv = fwd, not_fwd, inv, not_inv
@@ -47,14 +45,10 @@ class Row:
         """(pattern, predictors it is expected for)"""
         return [(p, self.ks) if isinstance(p, str) else (p[0], tuple(p[1])) for p in pats]
 
-    @property
-    def group(self):
-        return ",".join("%s=%s" % kv for kv in sorted(self.env.items())) or "default"
-
 
 K7, K_NOT2, K_SCAN, K_NOSCAN = range(1, 8), (1, 3, 4, 5, 6, 7), (1, 2, 4), (3, 5, 6, 7)
 FWD2, FWD, FWD_ROWS = "k_predict_fwd2<", "k_predict_fwd<", "k_predict_fwd_rows<"
-SEG, COLS4, COLS2, COLS1, UROWS = "k_unscan_cols_seg", "k_unscan_cols<false, 4>", "k_unscan_cols<false, 2>", "k_unscan_cols<false, 1>", "k_unscan_rows<"
+SEG, COLS2, COLS1, UROWS = "k_unscan_cols_seg", "k_unscan_cols<false, 2>", "k_unscan_cols<false, 1>", "k_unscan_rows<"
 GRID2, GRID1, SPACE, ANGLE, TANGLE = "k_unpredict_grid<2,", "k_unpredict_grid<1,", "k_unpredict_space(", "k_unpredict_angle(", "k_unpredict_tiles_angle<"
 BANDS, CLUSTER, ROW0, UCOLS2, STRIPS = "k_unpredict_bands<", "k_unpredict(", "k_unpredict_row0<", "k_unpredict_cols2<", "k_unpredict_strips<"
 
@@ -93,11 +87,11 @@ ROWS = [
     Row("w1_space", 2, K7, (4, 30, 1), 5),
     # ---- way space inverse: prefix-sum passes (predictors 1, 2, 4)
     # (predictor 1 has no full-width column pass: only the first tile column, always one pixel wide)
-    Row("scan_cols_seg", 2, K_SCAN, (2, 60, 64), 11, inv=((SEG, (2, 4)), UROWS), not_inv=(COLS4, COLS2)),
-    Row("scan_cols2_w66", 2, K_SCAN, (2, 60, 66), 11, inv=((COLS2, (2, 4)), UROWS), not_inv=(SEG, COLS4)),
-    Row("scan_cols2_off4", 2, K_SCAN, (2, 60, 64), 11, off=(4, 4), inv=((COLS2, (2, 4)), UROWS), not_inv=(SEG, COLS4)),
-    Row("scan_cols1_w67", 2, K_SCAN, (2, 60, 67), 11, inv=(COLS1, UROWS), not_inv=(SEG, COLS4, COLS2)),
-    Row("scan_cols1_off2", 2, K_SCAN, (2, 60, 64), 11, off=(2, 2), inv=(COLS1, UROWS), not_inv=(SEG, COLS4, COLS2)),
+    Row("scan_cols_seg", 2, K_SCAN, (2, 60, 64), 11, inv=((SEG, (2, 4)), UROWS), not_inv=(COLS2,)),
+    Row("scan_cols2_w66", 2, K_SCAN, (2, 60, 66), 11, inv=((COLS2, (2, 4)), UROWS), not_inv=(SEG,)),
+    Row("scan_cols2_off4", 2, K_SCAN, (2, 60, 64), 11, off=(4, 4), inv=((COLS2, (2, 4)), UROWS), not_inv=(SEG,)),
+    Row("scan_cols1_w67", 2, K_SCAN, (2, 60, 67), 11, inv=(COLS1, UROWS), not_inv=(SEG, COLS2)),
+    Row("scan_cols1_off2", 2, K_SCAN, (2, 60, 64), 11, off=(2, 2), inv=(COLS1, UROWS), not_inv=(SEG, COLS2)),
     Row("scan_rows_r1_short_frame", 2, K_SCAN, (1, 30, 64), 11, inv=(UROWS,)),
     Row("scan_rows_r8", 2, K_SCAN, (80, 64, 64), 11, inv=(UROWS, (SEG, (2, 4)))),
     Row("scan_l2_groups", 2, (4,), (9, 2048, 2048), 15, inv=(UROWS, SEG)),
@@ -107,7 +101,9 @@ ROWS = [
     Row("grid2_g2", 2, K_NOSCAN, (1, 1024, 1024), 5, inv=(GRID2,), not_inv=(SPACE,)),
     Row("grid2_g1", 2, K_NOSCAN, (1, 1024, 1024), 4, inv=(GRID2,), not_inv=(SPACE,)),
     Row("space_1024_nnum3", 2, K7, (1, 1024, 1024), 3, inv=((SPACE, K_NOSCAN), (UROWS, K_SCAN)), not_inv=(GRID2,)),
-    Row("space_w24600", 2, K_SCAN, (1, 40, 24600), 15, inv=(SPACE,), not_inv=(GRID2, UROWS, SEG, COLS4, COLS2, COLS1)),
+    # rows too wide for the row pass: the grid for at most 1024 tile columns, else the fall-back
+    Row("grid2_scan_k_w24600", 2, K_SCAN, (1, 50, 24600), 25, inv=(GRID2,), not_inv=(UROWS, SEG, SPACE)),
+    Row("space_w24600", 2, K_SCAN, (1, 40, 24600), 15, inv=(SPACE,), not_inv=(GRID2, UROWS, SEG, COLS2, COLS1)),
     # ---- way angle inverse
     Row("angle_tiles_nnum28", 1, K_NOT2, (2, 100, 168), 28, inv=(GRID1, TANGLE), not_inv=(ANGLE,)),
     Row("angle_tiles_nnum28_odd_w", 1, K_NOT2, (2, 90, 150), 28, inv=(GRID1, TANGLE), not_inv=(ANGLE,)),
@@ -116,12 +112,20 @@ ROWS = [
     # ---- way tiles inverse
     Row("bands_nnum30_odd", 0, K_NOT2, (7, 70, 100), 30, video=(0, 1), inv=(BANDS,), not_inv=(CLUSTER,)),
     Row("bands_nnum30_even", 0, K_NOT2, (8, 70, 100), 30, video=(0, 1), inv=(BANDS,), not_inv=(CLUSTER,)),
+    Row("bands_r1", 0, K_NOT2, (7, 13, 100), 13, video=(0, 1), inv=(BANDS,), not_inv=(CLUSTER,)),     # one tile row: bands of R = 1
     Row("cluster_nnum31", 0, K_NOT2, (4, 70, 100), 31, inv=(CLUSTER,), not_inv=(BANDS,)),
     Row("cols2_tiles", 0, (2,), (5, 60, 100), 13, video=(0, 1), inv=(ROW0, UCOLS2), not_inv=(CLUSTER, STRIPS)),
     Row("cols2_angle", 1, (2,), (5, 60, 100), 13, inv=(ROW0, UCOLS2), not_inv=(CLUSTER, STRIPS)),
     Row("strips_h1_tiles", 0, (2,), (130, 1, 200), 13, inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
     Row("strips_h1_angle", 1, (2,), (130, 1, 200), 13, inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
     Row("strips_h1_video", 0, (2,), (260, 1, 200), 13, video=(1,), inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
+    # rows wider than k_unpredict_cols2's shared memory (W > 51200)
+    Row("strips_tiles_w51208", 0, (2,), (256, 2, 51208), 13, video=(0, 1), inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
+    Row("strips_tiles_w51211", 0, (2,), (256, 2, 51211), 13, video=(0, 1), inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
+    Row("strips_tiles_w51208_off2", 0, (2,), (256, 2, 51208), 13, video=(0, 1), off=(2, 2), inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
+    Row("strips_angle_w51208", 1, (2,), (128, 2, 51208), 13, inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
+    Row("strips_angle_w51211", 1, (2,), (128, 2, 51211), 13, inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
+    Row("strips_angle_w51208_off2", 1, (2,), (128, 2, 51208), 13, off=(2, 2), inv=(STRIPS,), not_inv=(CLUSTER, UCOLS2)),
     Row("cluster_1_frame_csz1", 0, K_NOT2, (1, 40, 50), 13, video=(0, 1), inv=(CLUSTER,), not_inv=(BANDS,)),
     Row("cluster_2_frames_csz8", 0, K_NOT2, (2, 1024, 1024), 13, video=(0, 1), inv=(CLUSTER,), not_inv=(BANDS,)),
     Row("cluster_rows_k2_nnum33", 0, (2,), (3, 100, 136), 33, video=(0, 1), inv=(CLUSTER,), not_inv=(UCOLS2, STRIPS)),
@@ -131,19 +135,7 @@ ROWS = [
     Row("frames65537_angle", 1, K7, (65537, 16, 16), 5, fwd=(FWD2,), inv=((GRID1, K_NOT2), (TANGLE, K_NOT2), (UCOLS2, (2,)))),
     Row("frames65537_space", 2, K7, (65537, 16, 16), 5, fwd=(FWD2,), inv=((UROWS, K_SCAN), (GRID2, K_NOSCAN))),
     Row("frames131074_video", 0, K7, (131074, 8, 16), 5, video=(1,), fwd=(FWD2,), inv=((BANDS, K_NOT2), (UCOLS2, (2,)))),
-    # ---- rows that need a switch (child process of their own)
-    Row("tma_off_cp_async", 0, K7, (3, 40, 64), 11, video=(0, 1), env={"LFM_B200_TMA": "0"}, fwd=(FWD2,)),
-    Row("tma_off_cp_async_space", 2, K7, (3, 40, 64), 11, env={"LFM_B200_TMA": "0"}, fwd=(FWD2,)),
-    Row("scan_seg_off_cols4", 2, K_SCAN, (2, 60, 64), 11, env={"LFM_B200_SCAN_SEG": "0"}, inv=((COLS4, (2, 4)), UROWS), not_inv=(SEG,)),
-    Row("scans_off_grid", 2, K_SCAN, (2, 60, 64), 11, env={"LFM_B200_SCANS": "0"}, inv=(GRID2,), not_inv=(UROWS, SEG)),
-    Row("bands_r1", 0, K_NOT2, (7, 70, 100), 13, video=(0, 1), env={"LFM_B200_BANDS_R": "1"}, inv=(BANDS,), not_inv=(CLUSTER,)),
 ]
-_STRIPS_ENV = {"LFM_B200_BANDS": "0", "LFM_B200_COLS": "0", "LFM_B200_STRIPS_MIN": "1"}
-for _shape, _off, _tag in (((6, 40, 64), (0, 0), "w64"), ((6, 40, 67), (0, 0), "w67"), ((6, 40, 64), (2, 2), "w64_off2")):
-    ROWS.append(Row("strips_all_tiles_" + _tag, 0, K7, _shape, 13, video=(0, 1), off=_off, env=_STRIPS_ENV,
-                    inv=(STRIPS,), not_inv=(BANDS, UCOLS2, CLUSTER)))
-    ROWS.append(Row("strips_all_angle_k2_" + _tag, 1, (2,), _shape, 13, off=_off, env=_STRIPS_ENV,
-                    inv=(STRIPS,), not_inv=(UCOLS2, CLUSTER)))
 BY_NAME = {r.name: r for r in ROWS}
 assert len(BY_NAME) == len(ROWS)
 
@@ -215,7 +207,7 @@ def test_oracle_round_trip(oracle, name):
 def test_rows_cover_every_switch_and_kernel():
     """the table names every kernel of the dispatcher at least once (a kernel name typo would make a row vacuous)"""
     named = {p for r in ROWS for p, _ in r.expected(r.fwd + r.inv)}
-    for p in (FWD2, FWD, FWD_ROWS, SEG, COLS4, COLS2, COLS1, UROWS, GRID2, GRID1, SPACE, ANGLE, TANGLE, BANDS, CLUSTER, ROW0,
+    for p in (FWD2, FWD, FWD_ROWS, SEG, COLS2, COLS1, UROWS, GRID2, GRID1, SPACE, ANGLE, TANGLE, BANDS, CLUSTER, ROW0,
               UCOLS2, STRIPS):
         assert p in named, p
 
@@ -350,9 +342,8 @@ def child_main(argv):
 _results = {}        # key -> the child's result, or the text of its failure: each child runs at most once per session
 
 
-def _child(args, env_extra, timeout):
+def _child(args, timeout):
     env = {k: v for k, v in os.environ.items() if not k.startswith("LFM_B200_")}
-    env.update(env_extra)
     env["LFM_B200_DEBUG_POISON"] = "1"
     cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [os.path.abspath(__file__)] + list(args)
     try:
@@ -365,26 +356,25 @@ def _child(args, env_extra, timeout):
     return json.loads(lines[-1][len("RESULT "):])
 
 
-def _cached_child(key, args, env_extra, timeout):
-    """the child's result; a child that failed is not started again, every later test of its group reports that failure"""
+def _cached_child(key, args, timeout):
+    """the child's result; a child that failed is not started again, every later test that needs it reports that failure"""
     if key not in _results:
-        _results[key] = _child(args, env_extra, timeout)
+        _results[key] = _child(args, timeout)
     res = _results[key]
     if isinstance(res, str):
         pytest.fail(res)
     return res
 
 
-def _group_results(group):
-    rows = [r for r in ROWS if r.group == group]
-    return _cached_child(group, ["rows"] + [r.name for r in rows], rows[0].env, timeout=1200)
+def _row_results():
+    return _cached_child("rows", ["rows"] + [r.name for r in ROWS], timeout=1200)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", [r.name for r in ROWS])
 def test_dispatch_row(name):
     row = BY_NAME[name]
-    res = _group_results(row.group)[name]
+    res = _row_results()[name]
     assert not res["errors"], "\n".join(res["errors"])
     for what, caps, want, avoid in (("forward", res["fwd_kernels"], row.fwd, row.not_fwd), ("inverse", res["inv_kernels"], row.inv, row.not_inv)):
         assert sorted(caps) == sorted("%d,%d" % kv for kv in combos(row)), (what, sorted(caps))
@@ -397,8 +387,8 @@ def test_dispatch_row(name):
                 assert not _ran(names, p), "%s k,video=%s: %s ran, the row is there for its fall-back; kernels: %s" % (what, combo, p, names)
 
 
-def _select(sort):
-    return _cached_child("select_sort" if sort else "select", ["select"], {"LFM_B200_SELECT_SORT": "1" if sort else "0"}, timeout=600)
+def _select():
+    return _cached_child("select", ["select"], timeout=600)
 
 
 def _f32(bits):
@@ -413,7 +403,7 @@ def test_mode_selection_against_oracle(oracle, name):
     predictor wins, as std::map overwrite does in the reference)"""
     make, T, ways = SELECT_FRAMES[name]
     f = make()
-    got_all = _select(False)
+    got_all = _select()
     for way in ways:
         got = got_all["%s/way%d" % (name, way)]
         want_k, want = oracle.select(f, T, way)
@@ -425,16 +415,6 @@ def test_mode_selection_against_oracle(oracle, name):
         others = [want[k] - want[want_k] for k in range(8) if k != want_k]
         if all(d == 0 or d > tol[want_k] for d in others):          # a clear margin, or exact ties only
             assert got["predictor"] == want_k, (name, way, got["predictor"], want_k, want)
-
-
-@pytest.mark.gpu
-def test_mode_selection_sorted_path_bit_identical():
-    """LFM_B200_SELECT_SORT=1 (stable sort instead of the next-occurrence walk) builds the same integer histograms and runs the
-    same entropy kernel: bit-identical entropies and the same predictor"""
-    a, b = _select(False), _select(True)
-    assert a.keys() == b.keys()
-    for key in a:
-        assert a[key] == b[key], (key, a[key], b[key])
 
 
 # ------------------------------------------------------------------------------------------------ whole files
